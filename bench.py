@@ -52,6 +52,19 @@ WORKLOADS = {
 FP64_PEAK_TFLOPS = 37.1  # measured on this pool's B200: DMMA m8n8k4 saturation (profiles/r01_fp64_peaks_and_box_probe.log)
 TAYLOR_T = 20            # canonical term count of SURVEY.md section 8d (C1)
 TDB_RHS = 80             # right-hand sides per interval of K7 with eight extrapolation columns and one macro step (BASELINE.md section 3); the kernels size the columns per interval: tdb_rhs_per_interval
+DUMP_MAX_ENTRIES = 1 << 20  # per array of --dump-outputs: five float64 arrays stay under 64 MB at every workload
+
+
+def dump_outputs(directory, arrays):
+    """--dump-outputs: writes each output as <directory>/<name>.npy (float64, flattened).  An array of more than
+    DUMP_MAX_ENTRIES entries is stored as its entries at a fixed sample of positions (seed 0, sorted), so that two builds
+    run with the same arguments can be compared entry for entry."""
+    os.makedirs(directory, exist_ok=True)
+    for name, a in arrays.items():
+        a = np.ascontiguousarray(a, dtype=np.float64).reshape(-1)
+        if a.size > DUMP_MAX_ENTRIES:
+            a = a[np.sort(np.random.default_rng(0).choice(a.size, DUMP_MAX_ENTRIES, replace=False))]
+        np.save(os.path.join(directory, f"{name}.npy"), a)
 
 
 def canonical_flops_per_interval(n, m, T=TAYLOR_T, s=0):
@@ -361,6 +374,9 @@ def run_workload(args, workload, steps, warmup, *, rank, world, local_rank, full
     ev.kernel_timing(False)
     launches = ev.launch_count - l0
     dev_ms = float(np.sum(step_ms))
+    if args.dump_outputs and full and rank == 0:  # what the last timed step left in HBM, before anything overwrites it
+        dump_outputs(args.dump_outputs, {"objective": dJ.cpu().numpy(), "gradient": dgrad.cpu().numpy(), "constraint": dg.cpu().numpy(),
+                                         "jacobian": djac.cpu().numpy(), "hessian": dhess.cpu().numpy()})
     # outputs of iterate 0 for the parity guards below
     with torch.cuda.stream(stream):
         step_dev(0)
@@ -592,7 +608,14 @@ def main():
     ap.add_argument("--no-extra", action="store_true", help="skip the embedded c3/c4/c5 runs of the default workload")
     ap.add_argument("--no-e2e", action="store_true", help="device-resident loop only (profiling: the ncu launch list of one step)")
     ap.add_argument("--scalar-reduce", default="peer", choices=["peer", "nccl"], help="knot shards: objective/violation reduction")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the outputs of the last timed step of the headline workload (rank 0: objective, gradient, constraint, "
+                         "jacobian, hessian values) as DIR/<name>.npy, float64; arrays above 2^20 entries as a fixed seeded sample")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of the CUDA evaluator (--impl ours)")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
 
     rank = int(os.environ.get("RANK", "0"))
