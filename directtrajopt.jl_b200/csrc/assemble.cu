@@ -478,12 +478,12 @@ __global__ void violation_kernel(long long n_cons, const double* __restrict__ g,
     double m = 0.0;
     for (long long r = (long long)blockIdx.x * blockDim.x + threadIdx.x; r < n_cons; r += (long long)gridDim.x * blockDim.x) {
         const double v = g[(long long)b * n_cons + r];
-        m = fmax(m, row_is_eq[r] ? fabs(v) : fmax(v, 0.0));
+        m = nan_max(m, row_is_eq[r] ? fabs(v) : nan_max(0.0, v));
     }
 #pragma unroll
-    for (int o = 16; o > 0; o >>= 1) m = fmax(m, __shfl_xor_sync(0xffffffffu, m, o));
-    // non-negative doubles order like their bit patterns
-    if ((threadIdx.x & 31) == 0 && m > 0.0) atomicMax((unsigned long long*)(viol + b), (unsigned long long)__double_as_longlong(m));
+    for (int o = 16; o > 0; o >>= 1) m = nan_max(m, __shfl_xor_sync(0xffffffffu, m, o));
+    // non-negative doubles order like their bit patterns, and every NaN above +inf
+    if ((threadIdx.x & 31) == 0) atomicMax((unsigned long long*)(viol + b), (unsigned long long)__double_as_longlong(m));
 }
 
 __global__ void jac_product_kernel(long long nnz, long long n_rows, long long n_cols, const double* __restrict__ jac,
@@ -669,16 +669,29 @@ void launch_constraint_pattern_probe(const DProb& P, const double* Z, double* de
     }
 }
 
+// warps per CTA of the Hessian assembler and its dynamic shared memory: every knot group stages its z x z diagonal tile
+// (and the cross tile when some integrator couples neighbouring knots)
+static size_t hessian_assemble_plan(const DProb& P, int& W) {
+    const size_t per_group = sizeof(double) * (size_t)P.z * P.z * (P.any_cross ? 2 : 1);
+    const int GS = P.z <= 16 ? 8 : (P.z <= 24 ? 16 : 32), GPW = 32 / GS;
+    W = 8;
+    while (W > 1 && W * GPW * per_group > 64 * 1024) W >>= 1;
+    const size_t tab_bytes = (sizeof(unsigned int) * ((size_t)P.z * P.z + (size_t)P.z * (P.z + 1) / 2) + 15) / 16 * 16;
+    return W * GPW * per_group + (GS < 32 ? tab_bytes : 0);
+}
+
+size_t hessian_assemble_smem_bytes(const DProb& P) {
+    int W;
+    return hessian_assemble_plan(P, W);
+}
+
 void launch_hessian_assemble(const DProb& P, const double* Z, double sigma, const double* mu, double* hess, cudaStream_t st,
                              long long* launches) {
     const int nKc = std::min(P.kc1, P.nOwn) - P.kc0;
     if (nKc <= 0) return;
-    const size_t per_group = sizeof(double) * (size_t)P.z * P.z * (P.any_cross ? 2 : 1);
     const int GS = P.z <= 16 ? 8 : (P.z <= 24 ? 16 : 32), GPW = 32 / GS;
-    int W = 8;
-    while (W > 1 && W * GPW * per_group > 64 * 1024) W >>= 1;
-    const size_t tab_bytes = (sizeof(unsigned int) * ((size_t)P.z * P.z + (size_t)P.z * (P.z + 1) / 2) + 15) / 16 * 16;
-    const size_t smem = W * GPW * per_group + (GS < 32 ? tab_bytes : 0);
+    int W;
+    const size_t smem = hessian_assemble_plan(P, W);
     static PerDeviceOnce configured;
     if (smem > 48 * 1024 && configured.first()) {
         cudaFuncSetAttribute(hessian_assemble_kernel<32>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);

@@ -1,4 +1,6 @@
-// K1 (generic variant): BilinearIntegrator interval kernel for any state dimension.
+// K1 (generic variant): BilinearIntegrator interval kernel for state dimensions up to 96 whose block fits shared memory.
+// A block holds the generator and every jet column of its interval (generic_smem_bytes): with the Hessian on a B200
+// (227 KB per block) that is n <= 83 at one drive and n <= 76 at four; dto_create rejects larger shapes.
 //
 // One warp per (problem, interval).  Replaces `expv` + ForwardDiff through it
 // (/root/reference/src/integrators/bilinear_integrator.jl:81,98-161): the warp propagates, through a
@@ -238,7 +240,7 @@ __global__ void __launch_bounds__(32) bilinear_generic_kernel(DProb P, int ii, c
 
 }  // namespace
 
-static size_t generic_smem_bytes(int n, int m, bool want_jac, bool want_hess) {
+size_t generic_smem_bytes(int n, int m, bool want_jac, bool want_hess) {
     int n2 = m * (m + 1) / 2;
     int nfwd = want_hess ? 1 + m + n2 : (want_jac ? 1 + m : 1);
     int ncol = nfwd + (want_jac ? n : 0) + (want_hess ? 1 + m : 0);

@@ -287,6 +287,15 @@ extern "C" int dto_create(const dto_problem_desc* d, dto_handle** out) {
     }
     if (cudaStreamCreateWithFlags(&h->stream, cudaStreamNonBlocking) != cudaSuccess)
         return fail_create(h, DTO_ERR_CUDA, "cudaStreamCreate failed");
+    // the kernels whose shared memory grows with the shape are checked against it here, so that a shape no kernel can
+    // launch is rejected at construction instead of failing at its first evaluation
+    int smem_optin = 0;
+    if (cudaDeviceGetAttribute(&smem_optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, h->device) != cudaSuccess)
+        return fail_create(h, DTO_ERR_CUDA, "cudaDeviceGetAttribute(MaxSharedMemoryPerBlockOptin) failed");
+    auto smem_msg = [&](const std::string& what, size_t need) {
+        return what + " needs " + std::to_string(need) + " bytes of shared memory per block, above the device's limit of " +
+               std::to_string(smem_optin) + " bytes";
+    };
 
     const int N = d->N, z = d->z;
     h->eval_hessian = d->eval_hessian;
@@ -384,6 +393,13 @@ extern "C" int dto_create(const dto_problem_desc* d, dto_handle** out) {
             }
             if (pin_generic) I.variant = DTO_VAR_GENERIC;
             if (s.x_dim > 96) return fail_create(h, DTO_ERR_UNSUPPORTED, "bilinear integrator: state dimension > 96 not supported");
+            if (I.variant == DTO_VAR_GENERIC) {  // one block per interval holds the generator and every jet column
+                const size_t need = generic_smem_bytes(s.x_dim, s.u_dim, true, d->eval_hessian);
+                if (need > (size_t)smem_optin)
+                    return fail_create(h, DTO_ERR_UNSUPPORTED, smem_msg("bilinear integrator: the generic kernel at state dimension " +
+                                                                        std::to_string(s.x_dim) + " with " + std::to_string(s.u_dim) +
+                                                                        " drives" + (d->eval_hessian ? " and the Hessian" : ""), need));
+            }
         } else if (s.kind == DTO_INT_DERIVATIVE) {
             if (s.u_dim != s.x_dim || s.u_off < 0 || s.u_off + s.u_dim > z) return fail_create(h, DTO_ERR_INVALID, "derivative integrator: derivative component must match the variable's dimension");
         } else if (s.kind == DTO_INT_TDBILINEAR) {
@@ -460,7 +476,9 @@ extern "C" int dto_create(const dto_problem_desc* d, dto_handle** out) {
                 const char* pin = getenv("DTO_B200_KERNEL");
                 I.variant = (I.Asw != nullptr && tdb_dmma_supported(I) && !(pin && strcmp(pin, "generic") == 0)) ? DTO_VAR_DMMA : DTO_VAR_GENERIC;
             }
-            if (!tdb_fits(I)) return fail_create(h, DTO_ERR_UNSUPPORTED, "tdbilinear integrator: too many drives/carriers or state too large for shared memory");
+            if (!tdb_fits(I, (size_t)smem_optin))
+                return fail_create(h, DTO_ERR_UNSUPPORTED, "tdbilinear integrator: more than 4 drives or 4 carriers, or a state too large for the device's " +
+                                                           std::to_string(smem_optin) + " bytes of shared memory per block");
             if (s.x_dim > 96) return fail_create(h, DTO_ERR_UNSUPPORTED, "tdbilinear integrator: state dimension > 96 not supported");
         } else {
             return fail_create(h, DTO_ERR_UNSUPPORTED, "unknown integrator kind");
@@ -561,6 +579,10 @@ extern "C" int dto_create(const dto_problem_desc* d, dto_handle** out) {
 
     P.hess_tab = nullptr;
     if (d->eval_hessian) {  // stream-out gather table of the Hessian assembler (assemble.cu), knots with cross rows
+        const size_t need = hessian_assemble_smem_bytes(P);
+        if (need > (size_t)smem_optin)
+            return fail_create(h, DTO_ERR_UNSUPPORTED, smem_msg("Hessian assembly of a knot of " + std::to_string(P.z) + " variables" +
+                                                                (P.any_cross ? " coupled to its neighbour" : ""), need));
         const int zz = P.z;
         std::vector<unsigned int> tab((size_t)zz * zz + (size_t)zz * (zz + 1) / 2);
         size_t e = 0;

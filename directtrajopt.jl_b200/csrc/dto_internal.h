@@ -166,6 +166,9 @@ __device__ inline int tdb_item_steps(const DInt& I, const double* zk, const doub
     return s;
 }
 
+// max that keeps a NaN operand (fmax drops it): a residual poisoned with NaN must not reduce to a feasible violation
+__host__ __device__ inline double nan_max(double a, double b) { return (b > a || b != b) ? b : a; }
+
 // Jacobian position helpers (local numbering) --------------------------------------------------
 // column of local knot kl (0-based), component l: [I1 prev | I1 own | I2 prev | I2 own | ... | constraints]
 __host__ __device__ inline long long jac_own_off(const DProb& P, int kl, int doff, int d) {
@@ -241,6 +244,7 @@ struct EvalFlags {
 void launch_hpp_contract(const DProb& P, int ii, const double* mu, cudaStream_t st, long long* launches);
 void launch_bilinear_generic(const DProb& P, int ii, const double* Z, const double* mu, double* g, double* jac, EvalFlags f,
                              cudaStream_t st, long long* launches);
+size_t generic_smem_bytes(int n, int m, bool want_jac, bool want_hess);  // dynamic shared memory of one generic K1 block
 bool launch_bilinear_dmma(const DProb& P, int ii, const double* Z, const double* mu, double* g, double* jac, EvalFlags f,
                           cudaStream_t st, long long* launches);
 bool bilinear_dmma_supported(int n, int m);
@@ -264,7 +268,7 @@ bool tdb_available();
 bool tdb_dmma_supported(const DInt& I);
 bool launch_tdb_dmma(const DProb& P, int ii, const double* Z, const double* mu, double* g, double* jac, EvalFlags f, cudaStream_t st,
                      long long* launches);
-bool tdb_fits(const DInt& I);
+bool tdb_fits(const DInt& I, size_t smem_limit);
 void launch_tdb(const DProb& P, int ii, const double* Z, const double* mu, double* g, double* jac, EvalFlags f, cudaStream_t st,
                 long long* launches);
 void launch_analytic(const DProb& P, const double* Z, double* g, double* jac, EvalFlags f, cudaStream_t st, long long* launches);
@@ -272,6 +276,7 @@ void launch_constraints(const DProb& P, const double* Z, double* g, double* jac,
 bool launch_knot_objective_pairs(const DProb& P, const double* Z, cudaStream_t st, long long* launches);
 void launch_hessian_assemble(const DProb& P, const double* Z, double sigma, const double* mu, double* hess, cudaStream_t st,
                              long long* launches);
+size_t hessian_assemble_smem_bytes(const DProb& P);  // dynamic shared memory of one assembler block (depends on z, any_cross)
 void launch_objective(const DProb& P, const double* Z, double* J, double* grad, double* partials, cudaStream_t st,
                       long long* launches);
 void launch_violation(const DProb& P, const double* g, const int* row_is_eq, double* viol, cudaStream_t st, long long* launches);

@@ -113,7 +113,7 @@ __device__ void exchange_scalars(XWin* own, XWin* const* __restrict__ peers, int
         double sum = 0.0, mx = 0.0;
         for (int r = 0; r < world; ++r) {  // rank order on every rank: identical bits everywhere
             sum += ((volatile double*)own->scal[par][r])[0];
-            mx = fmax(mx, ((volatile double*)own->scal[par][r])[1]);
+            mx = nan_max(mx, ((volatile double*)own->scal[par][r])[1]);
         }
         *J = sum;
         *viol = mx;
@@ -126,7 +126,7 @@ __global__ void scalar_exchange_kernel(XWin* own, XWin* const* __restrict__ peer
 }
 
 // The shard's constraint violation (max(|g_eq|, max(0, g_ineq)) over its rows) AND the exchange in one launch: every CTA
-// reduces its rows into scratch[0] (non-negative doubles order like their bit patterns); the CTA that arrives last at
+// reduces its rows into scratch[0] (non-negative doubles order like their bit patterns, NaN above +inf); the CTA that arrives last at
 // scratch[1] owns the complete maximum, exchanges {J, viol} with the peers and leaves the scratch words zeroed for the next call.
 __global__ void __launch_bounds__(256) shard_scalars_kernel(XWin* own, XWin* const* __restrict__ peers, int rank, int world,
                                                             unsigned long long seq, long long n_cons, const double* __restrict__ g,
@@ -137,15 +137,15 @@ __global__ void __launch_bounds__(256) shard_scalars_kernel(XWin* own, XWin* con
     double m = 0.0;
     for (long long r = (long long)blockIdx.x * blockDim.x + threadIdx.x; r < n_cons; r += (long long)gridDim.x * blockDim.x) {
         const double v = g[r];
-        m = fmax(m, row_is_eq[r] ? fabs(v) : fmax(v, 0.0));
+        m = nan_max(m, row_is_eq[r] ? fabs(v) : nan_max(0.0, v));
     }
 #pragma unroll
-    for (int o = 16; o > 0; o >>= 1) m = fmax(m, __shfl_xor_sync(0xffffffffu, m, o));
+    for (int o = 16; o > 0; o >>= 1) m = nan_max(m, __shfl_xor_sync(0xffffffffu, m, o));
     if ((threadIdx.x & 31) == 0) red[threadIdx.x >> 5] = m;
     __syncthreads();
     if (threadIdx.x == 0) {
-        for (int w = 1; w < (int)(blockDim.x >> 5); ++w) m = fmax(m, red[w]);
-        if (m > 0.0) atomicMax(&scratch[0], (unsigned long long)__double_as_longlong(m));
+        for (int w = 1; w < (int)(blockDim.x >> 5); ++w) m = nan_max(m, red[w]);
+        atomicMax(&scratch[0], (unsigned long long)__double_as_longlong(m));
         __threadfence();
         is_last = atomicAdd(&scratch[1], 1ull) == (unsigned long long)gridDim.x - 1;
     }

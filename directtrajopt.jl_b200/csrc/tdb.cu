@@ -422,4 +422,6 @@ void launch_tdb(const DProb& P, int ii, const double* Z, const double* mu, doubl
     ++*launches;
 }
 
-bool tdb_fits(const DInt& I) { return I.m <= kMaxM && I.n_carrier <= kMaxC && tdb_smem_bytes(I, true, true) <= 227 * 1024; }
+bool tdb_fits(const DInt& I, size_t smem_limit) {
+    return I.m <= kMaxM && I.n_carrier <= kMaxC && tdb_smem_bytes(I, true, true) <= smem_limit;
+}

@@ -136,6 +136,14 @@ def test_violation_reduction():
     ev.violation_dev(dg.data_ptr(), dv.data_ptr())
     ev.synchronize()
     assert dv.item() == ref
+    # a residual the kernels poisoned with NaN is no feasible point: NaN in an equality row, then in an inequality row
+    for row in (int(np.flatnonzero(lo == 0)[3]), int(np.flatnonzero(lo < 0)[1])):
+        gn = g.copy()
+        gn[row] = np.nan
+        dg = torch.from_numpy(gn).cuda()
+        ev.violation_dev(dg.data_ptr(), dv.data_ptr())
+        ev.synchronize()
+        assert np.isnan(dv.item()), row
     ev.close()
 
 
@@ -201,5 +209,23 @@ def test_linked_shards_follow_a_changing_iterate():
             for sh in shards:
                 sh.synchronize()
             assert all(float(t.item()) == tot[0] for t in dJ2) and all(float(v.item()) == vw for v in dV2)
+    # one shard's residuals hold a NaN: every rank reports the violation as NaN, from its own rows and from the exchange
+    dGs[2][5] = float("nan")
+    dJ3 = [torch.tensor([float(sh.eval_objective(Zloc))], dtype=torch.float64, device="cuda") for sh, Zloc in zip(shards, locs)]
+    dV3 = [torch.full((1,), -1.0, dtype=torch.float64, device="cuda") for _ in shards]
+    torch.cuda.synchronize()
+    for sh, dG, dJ, dV in zip(shards, dGs, dJ3, dV3):
+        sh.shard_scalars_dev(dG.data_ptr(), dJ.data_ptr(), dV.data_ptr())
+    for sh in shards:
+        sh.synchronize()
+    assert all(np.isnan(float(v.item())) for v in dV3)
+    dV4 = [torch.tensor([np.nan if i == 2 else 0.5], dtype=torch.float64, device="cuda") for i in range(len(shards))]
+    dJ4 = [torch.zeros(1, dtype=torch.float64, device="cuda") for _ in shards]
+    torch.cuda.synchronize()
+    for sh, dJ, dV in zip(shards, dJ4, dV4):
+        sh.allreduce_scalars_dev(dJ.data_ptr(), dV.data_ptr())
+    for sh in shards:
+        sh.synchronize()
+    assert all(np.isnan(float(v.item())) for v in dV4)
     for e in shards + [whole]:
         e.close()
