@@ -17,6 +17,7 @@ from .components import (AbstractIntegrator, AbstractNonlinearConstraint, Abstra
                          GlobalObjective, GlobalKnotPointObjective, NonlinearGlobalConstraint, NonlinearGlobalKnotPointConstraint,
                          NormProduct, SplitSqDist, KnotHVP, ConstantLowRankHVP, CustomKnotHVP, knot_hvp)
 from .evaluator import DirectTrajOptProblem, Evaluator
+from .knot_program import KnotProgram
 from .trajectory import KnotPoint, NamedTrajectory
 from . import problem_templates
 

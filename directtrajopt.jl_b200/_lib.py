@@ -10,12 +10,13 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("DTO_B200_LIB") or os.path.join(HERE, "lib", "libdto_b200.so")
 
 DTO_OK, DTO_ERR_INVALID, DTO_ERR_UNSUPPORTED, DTO_ERR_CUDA, DTO_ERR_ALLOC = 0, -1, -2, -3, -4
-ABI_VERSION = 3
+ABI_VERSION = 4
 
 INT_BILINEAR, INT_DERIVATIVE, INT_TDBILINEAR = 1, 2, 3
 OBJ_QUADREG, OBJ_MINTIME, OBJ_KNOT, OBJ_NULL, OBJ_LINREG, OBJ_GLOBAL_KNOT = 1, 2, 3, 4, 5, 6
 G_FUNCS = {"norm_minus_c": 1, "normsq_minus_c": 2, "sqdist_minus_c": 3, "linear": 4, "norm_product": 5}
 L_FUNCS = {"normsq_plus_p": 1, "sqdist": 2, "linear": 3, "iso_infidelity": 4, "split_sqdist": 5}
+G_PROGRAM, L_PROGRAM = 100, 100  # knot programs (knot_program.py): the term's `program` indexes ProblemDesc.programs
 
 c_double_p = C.POINTER(C.c_double)
 c_int32_p = C.POINTER(C.c_int32)
@@ -37,7 +38,7 @@ class ObjectiveDesc(C.Structure):
     _fields_ = [
         ("kind", C.c_int32), ("fn", C.c_int32), ("weight", C.c_double), ("n_vars", C.c_int32), ("n_times", C.c_int32),
         ("var_offs", c_int32_p), ("times", c_int32_p), ("R", c_double_p), ("baseline", c_double_p), ("D", C.c_double),
-        ("n_params", C.c_int32), ("_pad", C.c_int32), ("params", c_double_p), ("Qs", c_double_p),
+        ("n_params", C.c_int32), ("program", C.c_int32), ("params", c_double_p), ("Qs", c_double_p),
         ("n_gvars", C.c_int32), ("_pad2", C.c_int32), ("gvar_offs", c_int32_p),
     ]
 
@@ -46,7 +47,14 @@ class ConstraintDesc(C.Structure):
     _fields_ = [
         ("fn", C.c_int32), ("equality", C.c_int32), ("n_vars", C.c_int32), ("n_times", C.c_int32),
         ("var_offs", c_int32_p), ("times", c_int32_p), ("g_dim", C.c_int32), ("n_params", C.c_int32), ("params", c_double_p),
-        ("n_gvars", C.c_int32), ("_pad", C.c_int32), ("gvar_offs", c_int32_p),
+        ("n_gvars", C.c_int32), ("program", C.c_int32), ("gvar_offs", c_int32_p),
+    ]
+
+
+class KnotProgramDesc(C.Structure):
+    _fields_ = [
+        ("n_ops", C.c_int32), ("n_out", C.c_int32), ("ops", c_int32_p), ("out", c_int32_p),
+        ("n_consts", C.c_int32), ("_pad", C.c_int32), ("consts", c_double_p),
     ]
 
 
@@ -57,7 +65,7 @@ class ProblemDesc(C.Structure):
         ("n_integrators", C.c_int32), ("n_objectives", C.c_int32), ("n_constraints", C.c_int32),
         ("integrators", C.POINTER(IntegratorDesc)), ("objectives", C.POINTER(ObjectiveDesc)),
         ("constraints", C.POINTER(ConstraintDesc)), ("Z0", c_double_p),
-        ("global_dim", C.c_int32), ("_pad", C.c_int32),
+        ("global_dim", C.c_int32), ("n_programs", C.c_int32), ("programs", C.POINTER(KnotProgramDesc)),
     ]
 
 

@@ -3,8 +3,9 @@ integrators (src/integrators/*.jl), objectives (src/objectives/{regularizers,min
 knot_point_objectives,_objectives}.jl) and NonlinearKnotPointConstraint
 (src/constraints/nonlinear/knot_point_constraint.jl).  Same names and argument meaning; the opaque
 Julia closures (G, g, l) are *lowered to data*: a bilinear generator to (G_drift, G_drives) by
-probing, knot functions to entries of the device catalogue (``KnotFunction``).  A component that
-cannot be lowered raises at construction -- never mid-solve, never a CPU fallback."""
+probing, knot functions to entries of the device catalogue (``KnotFunction``) or to traced device programs
+(``KnotProgram``, knot_program.py).  A component that cannot be lowered raises at construction -- never mid-solve,
+never a CPU fallback."""
 from __future__ import annotations
 
 import numpy as np
@@ -88,6 +89,28 @@ def NormProduct(n1, c1=1.0, c2=1.0):
 def IsoInfidelity(goal):
     """l(psi_iso) = 1 - |<goal|psi>|^2 for iso-vectors [re; im]"""
     return KnotFunction("iso_infidelity", goal)
+
+
+def _knot_function(fn, catalogue, who, n_vars, objective):
+    """Check the knot function of a term: a catalogue ``KnotFunction`` or a ``KnotProgram`` (traced here, where the
+    term's variable count is known).  A bare callable is refused: it has to be wrapped so that it is clear it will be
+    traced.  Returns the term's g_dim."""
+    from .knot_program import KnotProgram
+
+    if isinstance(fn, KnotProgram):
+        gd = fn.g_dim(n_vars)
+        if objective and gd != 1:
+            raise UnsupportedComponent(f"{who}: a KnotProgram objective must return one value, not {gd}")
+        return gd
+    if not isinstance(fn, KnotFunction) or fn.name not in catalogue:
+        kind = "objective" if objective else "constraint"
+        raise UnsupportedComponent(f"{who}: expected a KnotProgram or a KnotFunction from the device {kind} catalogue")
+    return fn.g_dim
+
+
+def _spec_fn(fn):
+    """What the CPU oracle receives as the term's function: the catalogue name, or the KnotProgram (a callable)."""
+    return fn.name if isinstance(fn, KnotFunction) else fn
 
 
 def _offsets(traj, names):
@@ -291,13 +314,12 @@ class MinimumTimeObjective(AbstractObjective):
 
 class KnotPointObjective(AbstractObjective):
     """``KnotPointObjective(l, names, traj; times, Qs)``: J = sum_i Q_i l([vars]_{times[i]}, params_i)
-    (knot_point_objectives.jl:65-157); ``l`` is a ``KnotFunction`` of the objective catalogue."""
+    (knot_point_objectives.jl:65-157); ``l`` is a ``KnotProgram`` or a ``KnotFunction`` of the objective catalogue."""
 
     def __init__(self, l, names, traj, times=None, Qs=None):
-        if not isinstance(l, KnotFunction) or l.name not in _lib.L_FUNCS:
-            raise UnsupportedComponent("KnotPointObjective: l must be a KnotFunction from the device objective catalogue")
         self.l = l
         self.var_names, self.var_offs = _offsets(traj, names)
+        _knot_function(l, _lib.L_FUNCS, "KnotPointObjective", len(self.var_offs), objective=True)
         self.times = list(range(1, traj.N + 1)) if times is None else [int(t) for t in times]
         self.Qs = np.ones(len(self.times)) if Qs is None else np.asarray(Qs, float)
         if self.Qs.shape != (len(self.times),):
@@ -306,7 +328,7 @@ class KnotPointObjective(AbstractObjective):
         self.knot_hvp = None  # optional KnotHVP carrier (knot_hvp.jl)
 
     def to_spec(self, traj):
-        return {"kind": "knot", "fn": self.l.name, "names": self.var_names, "times": self.times, "params": self.params, "Qs": self.Qs}
+        return {"kind": "knot", "fn": _spec_fn(self.l), "names": self.var_names, "times": self.times, "params": self.params, "Qs": self.Qs}
 
 
 def _global_offsets(traj, global_names):
@@ -326,11 +348,10 @@ class GlobalKnotPointObjective(AbstractObjective):
     ``global_names=None`` takes every global component of the trajectory."""
 
     def __init__(self, l, names, global_names, traj, times=None, Qs=None):
-        if not isinstance(l, KnotFunction) or l.name not in _lib.L_FUNCS:
-            raise UnsupportedComponent("GlobalKnotPointObjective: l must be a KnotFunction from the device objective catalogue")
         self.l = l
         self.var_names, self.var_offs = _offsets(traj, names) if names else ([], np.zeros(0, np.int32))
         self.global_names, self.gvar_offs = _global_offsets(traj, global_names)
+        _knot_function(l, _lib.L_FUNCS, "GlobalKnotPointObjective", len(self.var_offs) + len(self.gvar_offs), objective=True)
         self.times = list(range(1, traj.N + 1)) if times is None else [int(t) for t in times]
         self.Qs = np.ones(len(self.times)) if Qs is None else np.asarray(Qs, float)
         if self.Qs.shape != (len(self.times),):
@@ -339,7 +360,7 @@ class GlobalKnotPointObjective(AbstractObjective):
         self.knot_hvp = None
 
     def to_spec(self, traj):
-        return {"kind": "global_knot", "fn": self.l.name, "names": self.var_names, "global_names": self.global_names,
+        return {"kind": "global_knot", "fn": _spec_fn(self.l), "names": self.var_names, "global_names": self.global_names,
                 "times": self.times, "params": self.params, "Qs": self.Qs}
 
 
@@ -399,22 +420,20 @@ class AbstractNonlinearConstraint:
 
 class NonlinearKnotPointConstraint(AbstractNonlinearConstraint):
     """``NonlinearKnotPointConstraint(g, names, traj; times, equality)`` (knot_point_constraint.jl:27-107);
-    ``g`` is a ``KnotFunction`` of the constraint catalogue."""
+    ``g`` is a ``KnotProgram`` or a ``KnotFunction`` of the constraint catalogue."""
 
     def __init__(self, g, names, traj, times=None, equality=True):
-        if not isinstance(g, KnotFunction) or g.name not in _lib.G_FUNCS:
-            raise UnsupportedComponent("NonlinearKnotPointConstraint: g must be a KnotFunction from the device constraint catalogue")
         self.g = g
         self.var_names, self.var_offs = _offsets(traj, names)
+        self.g_dim = _knot_function(g, _lib.G_FUNCS, "NonlinearKnotPointConstraint", len(self.var_offs), objective=False)
         self.equality = bool(equality)
         self.times = list(range(1, traj.N + 1)) if times is None else [int(t) for t in times]
         self.params = g.param_table(len(self.times))
-        self.g_dim = g.g_dim
         self.var_dim = len(self.var_offs)
         self.dim = self.g_dim * len(self.times)
 
     def to_spec(self, traj):
-        return {"kind": "knot", "fn": self.g.name, "names": self.var_names, "times": self.times, "params": self.params,
+        return {"kind": "knot", "fn": _spec_fn(self.g), "names": self.var_names, "times": self.times, "params": self.params,
                 "equality": self.equality}
 
 
@@ -423,22 +442,21 @@ class NonlinearGlobalKnotPointConstraint(AbstractNonlinearConstraint):
     at every listed time (global_knot_point_constraint.jl:30-256)."""
 
     def __init__(self, g, names, global_names, traj, times=None, equality=True):
-        if not isinstance(g, KnotFunction) or g.name not in _lib.G_FUNCS:
-            raise UnsupportedComponent("NonlinearGlobalKnotPointConstraint: g must be a KnotFunction from the device constraint catalogue")
         self.g = g
         self.var_names, self.var_offs = _offsets(traj, names) if names else ([], np.zeros(0, np.int32))
         self.global_names, self.gvar_offs = _global_offsets(traj, global_names)
+        self.g_dim = _knot_function(g, _lib.G_FUNCS, "NonlinearGlobalKnotPointConstraint", len(self.var_offs) + len(self.gvar_offs),
+                                    objective=False)
         self.equality = bool(equality)
         self.times = list(range(1, traj.N + 1)) if times is None else [int(t) for t in times]
         self.params = g.param_table(len(self.times))
-        self.g_dim = g.g_dim
         self.var_dim = len(self.var_offs)
         self.global_dim = len(self.gvar_offs)
         self.combined_dim = self.var_dim + self.global_dim
         self.dim = self.g_dim * len(self.times)
 
     def to_spec(self, traj):
-        return {"kind": "global_knot", "fn": self.g.name, "names": self.var_names, "global_names": self.global_names,
+        return {"kind": "global_knot", "fn": _spec_fn(self.g), "names": self.var_names, "global_names": self.global_names,
                 "times": self.times, "params": self.params, "equality": self.equality}
 
 

@@ -1,6 +1,7 @@
 // K2/K3/K4/K5/K6: the HBM-bound kernels around the interval kernels.
 //   analytic_kernel      DerivativeIntegrator residual + dense Jacobian block          (derivative_integrator.jl:45-86)
 //   constraint_kernel    NonlinearKnotPointConstraint values + Jacobian (hyper-duals)   (knot_point_constraint.jl:235-268)
+//   knot_program_kernel  the same for a constraint given as a knot program, one thread per seed
 //   hessian_assemble     per-knot upper-triangle Hessian of the Lagrangian in COO order (evaluator.jl:560-647)
 //   objective_kernel     objective value + dense gradient, warp-shuffle reductions       (_objectives.jl:111-128)
 //   violation_kernel     max-norm constraint violation
@@ -63,14 +64,14 @@ __global__ void constraint_kernel(DProb P, int ci, const double* __restrict__ Z,
     const int nv = C.nv, gd = C.gd;
     if (g != nullptr) {
         double out[16];
-        knot_cfun<double>(C.fn, ValueVars{zk, gp, C.var_offs, C.nvk}, nv, p, out, gd);
+        knot_cfun<false, double>(C.fn, C.prog, ValueVars{zk, gp, C.var_offs, C.nvk}, nv, p, out, gd);
         double* gp = g + (long long)b * P.n_cons_local + C.row_off + (long long)j * gd;
         for (int a = 0; a < gd; ++a) gp[a] = out[a];
     }
     if (jac != nullptr || dense_probe != nullptr) {
         HDual out[16];
         for (int i = 0; i < nv; ++i) {
-            knot_cfun<HDual>(C.fn, SeededVars{zk, gp, C.var_offs, C.nvk, i, -1}, nv, p, out, gd);
+            knot_cfun<false, HDual>(C.fn, C.prog, SeededVars{zk, gp, C.var_offs, C.nvk, i, -1}, nv, p, out, gd);
             for (int a = 0; a < gd; ++a) {
                 const long long e = ((long long)j * gd + a) * nv + i;
                 if (dense_probe != nullptr) {
@@ -80,6 +81,43 @@ __global__ void constraint_kernel(DProb P, int ci, const double* __restrict__ Z,
                     if (pos >= 0) jac[(long long)b * P.nnz_jac_local + pos] = out[a].d1;
                 }
             }
+        }
+    }
+}
+
+// K5 for knot programs: one thread per (problem, owned time entry, seed).  Seed 0 evaluates the values, seed 1 + i the
+// Jacobian column of variable i.  A program of 100 operations costs a few thousand instructions per seed; the catalogue
+// kernel's loop over the nv seeds in one thread would leave most of the GPU idle.
+__global__ void knot_program_kernel(DProb P, int ci, const double* __restrict__ Z, double* __restrict__ g, double* __restrict__ jac,
+                                    double* __restrict__ dense_probe, int seed0, int seeds, long long total) {
+    const DCon& C = P.co[ci];
+    const long long t = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (t >= total) return;
+    const int seed = seed0 + (int)(t % seeds);
+    const long long r = t / seeds;
+    const int b = (int)(r / C.nt_own), j = (int)(r % C.nt_own);
+    const int kl = C.own_knot[j];
+    const double* zk = Z + (long long)b * P.n_vars_local + (long long)kl * P.z;
+    const double* gp = Z + (long long)b * P.n_vars_local + (long long)P.nK * P.z;  // global variables
+    const double* p = C.params + (long long)C.own_ti[j] * C.np;
+    const int nv = C.nv, gd = C.gd;
+    if (seed == 0) {
+        double out[16];
+        run_knot_program<double, ValueVars>(C.prog.code, C.prog.n_code, ValueVars{zk, gp, C.var_offs, C.nvk}, p, out);
+        double* gr = g + (long long)b * P.n_cons_local + C.row_off + (long long)j * gd;
+        for (int a = 0; a < gd; ++a) gr[a] = out[a];
+        return;
+    }
+    const int i = seed - 1;
+    HDual out[16];
+    run_knot_program<HDual, SeededVars>(C.prog.code, C.prog.n_code, SeededVars{zk, gp, C.var_offs, C.nvk, i, -1}, p, out);
+    for (int a = 0; a < gd; ++a) {
+        const long long e = ((long long)j * gd + a) * nv + i;
+        if (dense_probe != nullptr) {
+            if (b == 0) dense_probe[e] = out[a].d1;
+        } else {
+            const long long pos = C.jac_pos[e];
+            if (pos >= 0) jac[(long long)b * P.nnz_jac_local + pos] = out[a].d1;
         }
     }
 }
@@ -122,7 +160,7 @@ __device__ __forceinline__ double group_sum(double v, unsigned gmask) {
 // Narrow knots are register-limited at the compiler's own allocation (68 registers: 3 CTAs of 256 threads per SM, a third
 // of the warp slots, too few loads in flight for a latency-bound stream-out): capped to 5 (GS = 8) / 4 (GS = 16) CTAs per SM
 // (c5: 560 -> 477 us, 0.62 of the measured HBM copy rate).
-template <int GS>
+template <int GS, bool Prog>
 __global__ void __launch_bounds__(256, GS == 8 ? 5 : (GS == 16 ? 4 : 1))
 hessian_assemble_kernel(DProb P, const double* __restrict__ Z, double sigma, const double* __restrict__ mu, double* __restrict__ hess,
                         int warps_per_cta, long long total) {
@@ -231,7 +269,7 @@ hessian_assemble_kernel(DProb P, const double* __restrict__ Z, double sigma, con
                 const int a = e / nvk, c = e % nvk;
                 if (a > c) continue;
                 HDual out[16];
-                knot_cfun<HDual>(C.fn, SeededVars{zk, gpz, C.var_offs, nvk, a, c}, nv, p, out, gd);
+                knot_cfun<Prog, HDual>(C.fn, C.prog, SeededVars{zk, gpz, C.var_offs, nvk, a, c}, nv, p, out, gd);
                 double s = 0.0;
                 for (int q = 0; q < gd; ++q) s = fma(mup[q], out[q].d12, s);
                 sym_add(diag, z, C.var_offs[a], C.var_offs[c], s);
@@ -342,6 +380,7 @@ hessian_assemble_kernel(DProb P, const double* __restrict__ Z, double sigma, con
 // terminal cost on a 32- or 64-dimensional state is one knot with ~500-2000 hyper-dual evaluations, which would serialise
 // inside the per-knot warp of the assembler).  Depends on Z only: it runs beside the interval kernels on the second stream
 // and the assembler adds sigma times the pairs to the knot's tile.
+template <bool Prog>
 __global__ void knot_objective_pairs_kernel(DProb P, int oi, const double* __restrict__ Z, long long total) {
     const DObj& O = P.ob[oi];
     const long long t = (long long)blockIdx.x * blockDim.x + threadIdx.x;
@@ -361,7 +400,7 @@ __global__ void knot_objective_pairs_kernel(DProb P, int oi, const double* __res
     const double* zk = Z + (long long)b * P.n_vars_local + (long long)kl * z;
     const double* prm = O.params + (long long)O.own_ti[j] * O.np;
     const double* gp = Z + (long long)b * P.n_vars_local + (long long)P.nK * z;
-    const HDual res = knot_lfun<HDual>(O.fn, SeededVars{zk, gp, O.var_offs, nv, a, c}, O.nv, prm);
+    const HDual res = knot_lfun<Prog, HDual>(O.fn, O.prog, SeededVars{zk, gp, O.var_offs, nv, a, c}, O.nv, prm);
     P.knot_side[(long long)b * P.side_stride + O.side_off + (long long)j * npairs + pair] = O.weight * O.Qs[O.own_ti[j]] * res.d12;
 }
 
@@ -369,7 +408,7 @@ __global__ void knot_objective_pairs_kernel(DProb P, int oi, const double* __res
 // K6: objective value + gradient, one WARP per (problem, owned knot); partial sums reduced in a
 // second, deterministic pass.
 // ------------------------------------------------------------------------------------------------
-template <int GS>
+template <int GS, bool Prog>
 __global__ void objective_kernel(DProb P, const double* __restrict__ Z, double* __restrict__ grad, double* __restrict__ partials,
                                  int warps_per_cta, long long total) {
     extern __shared__ double sm[];
@@ -436,10 +475,10 @@ __global__ void objective_kernel(DProb P, const double* __restrict__ Z, double* 
                 const int nv = O.nv, nvk = O.nvk;
                 const double* p = O.params + (long long)O.own_ti[j] * O.np;
                 const double w = O.weight * O.Qs[O.own_ti[j]];
-                if (tid == 0) Jk += w * knot_lfun<double>(O.fn, ValueVars{zk, gp, O.var_offs, nvk}, nv, p);
+                if (tid == 0) Jk += w * knot_lfun<Prog, double>(O.fn, O.prog, ValueVars{zk, gp, O.var_offs, nvk}, nv, p);
                 if (grad != nullptr)
                     for (int a = tid; a < nvk; a += nt) {
-                        const HDual r = knot_lfun<HDual>(O.fn, SeededVars{zk, gp, O.var_offs, nvk, a, -1}, nv, p);
+                        const HDual r = knot_lfun<Prog, HDual>(O.fn, O.prog, SeededVars{zk, gp, O.var_offs, nvk, a, -1}, nv, p);
                         gz[O.var_offs[a]] += w * r.d1;
                     }
             }
@@ -532,6 +571,7 @@ __global__ void analytic_product_kernel(DProb P, const double* __restrict__ Z, c
     }
 }
 
+template <bool Prog>
 __global__ void constraint_product_kernel(DProb P, int ci, const double* __restrict__ Z, const double* __restrict__ w,
                                           double* __restrict__ y, int transpose) {
     const DCon& C = P.co[ci];
@@ -550,7 +590,7 @@ __global__ void constraint_product_kernel(DProb P, int ci, const double* __restr
     for (int a = 0; a < gd; ++a) acc[a] = 0.0;
     HDual out[16];
     for (int i = 0; i < nv; ++i) {
-        knot_cfun<HDual>(C.fn, SeededVars{zk, gp, C.var_offs, C.nvk, i, -1}, nv, p, out, gd);
+        knot_cfun<Prog, HDual>(C.fn, C.prog, SeededVars{zk, gp, C.var_offs, C.nvk, i, -1}, nv, p, out, gd);
         double col = 0.0;
         for (int a = 0; a < gd; ++a) {
             if (C.jac_pos[((long long)j * gd + a) * nv + i] < 0) continue;  // never stored by the reference: not part of J
@@ -616,6 +656,12 @@ __global__ void hpp_contract_kernel(DProb P, int ii, const double* __restrict__ 
     }
 }
 
+bool any_program_constraint(const DProb& P) {
+    for (int ci = 0; ci < P.n_con; ++ci)
+        if (P.co[ci].fn == DTO_G_PROGRAM) return true;
+    return false;
+}
+
 }  // namespace
 
 void launch_hpp_contract(const DProb& P, int ii, const double* mu, cudaStream_t st, long long* launches) {
@@ -646,10 +692,25 @@ void launch_analytic(const DProb& P, const double* Z, double* g, double* jac, Ev
     }
 }
 
+void launch_knot_program(const DProb& P, int ci, const double* Z, double* g, double* jac, double* dense_probe, cudaStream_t st,
+                         long long* launches) {
+    const DCon& C = P.co[ci];
+    const bool want_jac = jac != nullptr || dense_probe != nullptr;
+    const int seed0 = g != nullptr ? 0 : 1, seeds = (g != nullptr ? 1 : 0) + (want_jac ? C.nv : 0);
+    const long long tot = (long long)P.batch * C.nt_own * seeds;
+    if (tot == 0) return;
+    knot_program_kernel<<<(unsigned)((tot + 127) / 128), 128, 0, st>>>(P, ci, Z, g, jac, dense_probe, seed0, seeds, tot);
+    ++*launches;
+}
+
 void launch_constraints(const DProb& P, const double* Z, double* g, double* jac, EvalFlags f, cudaStream_t st, long long* launches) {
     for (int ci = 0; ci < P.n_con; ++ci) {
         const long long tot = (long long)P.batch * P.co[ci].nt_own;
         if (tot == 0) continue;
+        if (P.co[ci].fn == DTO_G_PROGRAM) {
+            launch_knot_program(P, ci, Z, f.want_g ? g : nullptr, f.want_jac ? jac : nullptr, nullptr, st, launches);
+            continue;
+        }
         constraint_kernel<<<(unsigned)((tot + 63) / 64), 64, 0, st>>>(P, ci, Z, f.want_g ? g : nullptr, f.want_jac ? jac : nullptr,
                                                                        nullptr);
         ++*launches;
@@ -661,7 +722,9 @@ void launch_constraint_pattern_probe(const DProb& P, const double* Z, double* de
     for (int ci = 0; ci < P.n_con; ++ci) {
         const DCon& C = P.co[ci];
         const long long tot = (long long)P.batch * C.nt_own;
-        if (tot) {
+        if (tot && C.fn == DTO_G_PROGRAM) {
+            launch_knot_program(P, ci, Z, nullptr, nullptr, dense + off, st, launches);
+        } else if (tot) {
             constraint_kernel<<<(unsigned)((tot + 63) / 64), 64, 0, st>>>(P, ci, Z, nullptr, nullptr, dense + off);
             ++*launches;
         }
@@ -694,15 +757,24 @@ void launch_hessian_assemble(const DProb& P, const double* Z, double sigma, cons
     const size_t smem = hessian_assemble_plan(P, W);
     static PerDeviceOnce configured;
     if (smem > 48 * 1024 && configured.first()) {
-        cudaFuncSetAttribute(hessian_assemble_kernel<32>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
-        cudaFuncSetAttribute(hessian_assemble_kernel<16>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
-        cudaFuncSetAttribute(hessian_assemble_kernel<8>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
+        cudaFuncSetAttribute(hessian_assemble_kernel<32, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
+        cudaFuncSetAttribute(hessian_assemble_kernel<16, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
+        cudaFuncSetAttribute(hessian_assemble_kernel<8, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
+        cudaFuncSetAttribute(hessian_assemble_kernel<32, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
+        cudaFuncSetAttribute(hessian_assemble_kernel<16, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
+        cudaFuncSetAttribute(hessian_assemble_kernel<8, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
     }
     const long long total = (long long)nKc * P.batch;
     const unsigned grid = (unsigned)((total + (long long)W * GPW - 1) / ((long long)W * GPW));
-    if (GS == 8) hessian_assemble_kernel<8><<<grid, W * 32, smem, st>>>(P, Z, sigma, mu, hess, W, total);
-    else if (GS == 16) hessian_assemble_kernel<16><<<grid, W * 32, smem, st>>>(P, Z, sigma, mu, hess, W, total);
-    else hessian_assemble_kernel<32><<<grid, W * 32, smem, st>>>(P, Z, sigma, mu, hess, W, total);
+    if (any_program_constraint(P)) {
+        if (GS == 8) hessian_assemble_kernel<8, true><<<grid, W * 32, smem, st>>>(P, Z, sigma, mu, hess, W, total);
+        else if (GS == 16) hessian_assemble_kernel<16, true><<<grid, W * 32, smem, st>>>(P, Z, sigma, mu, hess, W, total);
+        else hessian_assemble_kernel<32, true><<<grid, W * 32, smem, st>>>(P, Z, sigma, mu, hess, W, total);
+    } else {
+        if (GS == 8) hessian_assemble_kernel<8, false><<<grid, W * 32, smem, st>>>(P, Z, sigma, mu, hess, W, total);
+        else if (GS == 16) hessian_assemble_kernel<16, false><<<grid, W * 32, smem, st>>>(P, Z, sigma, mu, hess, W, total);
+        else hessian_assemble_kernel<32, false><<<grid, W * 32, smem, st>>>(P, Z, sigma, mu, hess, W, total);
+    }
     ++*launches;
 }
 
@@ -715,7 +787,8 @@ bool launch_knot_objective_pairs(const DProb& P, const double* Z, cudaStream_t s
         if ((O.kind != DTO_OBJ_KNOT && O.kind != DTO_OBJ_GLOBAL_KNOT) || O.nt_own == 0 || O.nvk == 0) continue;
         if (O.own_kmax < P.kc0 || O.own_kmin >= P.kc1) continue;  // no listed knot in the active range
         const long long tot = (long long)P.batch * O.nt_own * (O.nvk * (O.nvk + 1) / 2);
-        knot_objective_pairs_kernel<<<(unsigned)((tot + 127) / 128), 128, 0, st>>>(P, oi, Z, tot);
+        if (O.fn == DTO_L_PROGRAM) knot_objective_pairs_kernel<true><<<(unsigned)((tot + 127) / 128), 128, 0, st>>>(P, oi, Z, tot);
+        else knot_objective_pairs_kernel<false><<<(unsigned)((tot + 127) / 128), 128, 0, st>>>(P, oi, Z, tot);
         ++*launches;
         any = true;
     }
@@ -730,9 +803,17 @@ void launch_objective(const DProb& P, const double* Z, double* J, double* grad, 
     const size_t smem = sizeof(double) * (size_t)P.z * W * GPW;
     const long long total = (long long)P.nOwn * P.batch;
     const unsigned grid = (unsigned)((total + (long long)W * GPW - 1) / ((long long)W * GPW));
-    if (GS == 8) objective_kernel<8><<<grid, W * 32, smem, st>>>(P, Z, grad, J ? partials : nullptr, W, total);
-    else if (GS == 16) objective_kernel<16><<<grid, W * 32, smem, st>>>(P, Z, grad, J ? partials : nullptr, W, total);
-    else objective_kernel<32><<<grid, W * 32, smem, st>>>(P, Z, grad, J ? partials : nullptr, W, total);
+    bool prog = false;
+    for (int oi = 0; oi < P.n_obj; ++oi) prog |= P.ob[oi].fn == DTO_L_PROGRAM && (P.ob[oi].kind == DTO_OBJ_KNOT || P.ob[oi].kind == DTO_OBJ_GLOBAL_KNOT);
+    if (prog) {
+        if (GS == 8) objective_kernel<8, true><<<grid, W * 32, smem, st>>>(P, Z, grad, J ? partials : nullptr, W, total);
+        else if (GS == 16) objective_kernel<16, true><<<grid, W * 32, smem, st>>>(P, Z, grad, J ? partials : nullptr, W, total);
+        else objective_kernel<32, true><<<grid, W * 32, smem, st>>>(P, Z, grad, J ? partials : nullptr, W, total);
+    } else {
+        if (GS == 8) objective_kernel<8, false><<<grid, W * 32, smem, st>>>(P, Z, grad, J ? partials : nullptr, W, total);
+        else if (GS == 16) objective_kernel<16, false><<<grid, W * 32, smem, st>>>(P, Z, grad, J ? partials : nullptr, W, total);
+        else objective_kernel<32, false><<<grid, W * 32, smem, st>>>(P, Z, grad, J ? partials : nullptr, W, total);
+    }
     ++*launches;
     if (J) {
         // partials layout: [batch][nOwn] followed by [batch][nchunks] of scratch
@@ -780,7 +861,10 @@ void launch_analytic_product(const DProb& P, const double* Z, const double* w, d
     for (int ci = 0; ci < P.n_con; ++ci) {
         const long long tot = (long long)P.batch * P.co[ci].nt_own;
         if (tot == 0) continue;
-        constraint_product_kernel<<<(unsigned)((tot + 63) / 64), 64, 0, st>>>(P, ci, Z, w, y, transpose ? 1 : 0);
+        if (P.co[ci].fn == DTO_G_PROGRAM)
+            constraint_product_kernel<true><<<(unsigned)((tot + 63) / 64), 64, 0, st>>>(P, ci, Z, w, y, transpose ? 1 : 0);
+        else
+            constraint_product_kernel<false><<<(unsigned)((tot + 63) / 64), 64, 0, st>>>(P, ci, Z, w, y, transpose ? 1 : 0);
         ++*launches;
     }
 }

@@ -231,6 +231,175 @@ static int fail_create(dto_handle* h, int code, const std::string& msg) {
 
 extern "C" int dto_abi_version(void) { return DTO_B200_ABI_VERSION; }
 
+// ---- knot programs ------------------------------------------------------------------------------
+// Compile the SSA tape of a knot program (include/dto_b200.h) into the register-machine words the device interpreter
+// runs (knot_program.cuh): values no output depends on are dropped, the rest are emitted depth-first in post-order from
+// the outputs (operand a's subtree, then b's), each output is written out as soon as it is complete, and slots are
+// allocated by linear scan (a slot is freed at the last use of its value and handed to the next value, lowest first).
+// A leaf is loaded right before each use, so sum_i v_i^2 over 128 variables needs two live slots, not 128.
+// Returns DTO_OK and appends the words (constants packed after them), or an error code with the message in `msg`.
+static int compile_knot_program(const dto_problem_desc* d, int index, int n_vars, int n_params, int n_out, std::vector<int4>& words,
+                                 std::string& msg) {
+    if (index < 0 || index >= d->n_programs || !d->programs) {
+        msg = "knot program index " + std::to_string(index) + " outside 0.." + std::to_string(d->n_programs - 1);
+        return DTO_ERR_INVALID;
+    }
+    const dto_knot_program& K = d->programs[index];
+    const std::string who = "knot program " + std::to_string(index) + ": ";
+    if (K.n_ops < 1 || K.n_out < 1 || !K.ops || !K.out || K.n_consts < 0 || (K.n_consts > 0 && !K.consts)) {
+        msg = who + "empty tape, no outputs or missing arrays";
+        return DTO_ERR_INVALID;
+    }
+    if (K.n_ops > DTO_MAX_PROGRAM_OPS) {
+        msg = who + std::to_string(K.n_ops) + " operations, above the limit of " + std::to_string(DTO_MAX_PROGRAM_OPS) +
+              " (DTO_MAX_PROGRAM_OPS)";
+        return DTO_ERR_UNSUPPORTED;
+    }
+    if (K.n_out != n_out) {
+        msg = who + std::to_string(K.n_out) + " outputs where the term has " + std::to_string(n_out);
+        return DTO_ERR_INVALID;
+    }
+    const int n = K.n_ops;
+    auto op = [&](int i, int f) { return K.ops[3 * i + f]; };
+    for (int i = 0; i < n; ++i) {
+        const int o = op(i, 0), a = op(i, 1), b = op(i, 2);
+        bool ok;
+        switch (o) {
+            case DTO_OP_VAR: ok = a >= 0 && a < n_vars; break;
+            case DTO_OP_PARAM: ok = a >= 0 && a < n_params; break;
+            case DTO_OP_CONST: ok = a >= 0 && a < K.n_consts; break;
+            case DTO_OP_ADD: case DTO_OP_SUB: case DTO_OP_MUL: case DTO_OP_DIV: ok = a >= 0 && a < i && b >= 0 && b < i; break;
+            case DTO_OP_NEG: case DTO_OP_SQRT: case DTO_OP_EXP: case DTO_OP_LOG: case DTO_OP_SIN: case DTO_OP_COS: case DTO_OP_TANH:
+                ok = a >= 0 && a < i;
+                break;
+            case DTO_OP_POWC: ok = a >= 0 && a < i && b >= 0 && b < K.n_consts; break;
+            default:
+                msg = who + "unknown opcode " + std::to_string(o) + " at operation " + std::to_string(i);
+                return DTO_ERR_INVALID;
+        }
+        if (!ok) {
+            msg = who + "operand out of range at operation " + std::to_string(i) +
+                  " (a variable, parameter or constant index beyond the term's, or a reference to a later operation)";
+            return DTO_ERR_INVALID;
+        }
+    }
+    for (int k = 0; k < K.n_out; ++k)
+        if (K.out[k] < 0 || K.out[k] >= n) {
+            msg = who + "output " + std::to_string(k) + " references no operation";
+            return DTO_ERR_INVALID;
+        }
+    auto n_operands = [&](int i) {
+        const int o = op(i, 0);
+        return o <= DTO_OP_CONST ? 0 : (o <= DTO_OP_DIV ? 2 : 1);  // POWC's b is a constant index
+    };
+    // Leaves (variables, parameters, constants) cost one load and are never kept live: a leaf operand is loaded into a
+    // scratch slot right before each operation that reads it.  Only computed values occupy slots between operations --
+    // an infidelity |<goal|psi>|^2 reads every variable and parameter twice, and keeping those leaves live would need
+    // 4n slots.
+    auto leaf = [&](int i) { return op(i, 0) <= DTO_OP_CONST; };
+    // post-order emission of the computed values: entries >= 0 are operations, -1 - k writes output k
+    std::vector<int> order;
+    std::vector<char> seen(n, 0);
+    for (int k = 0; k < K.n_out; ++k) {
+        std::vector<std::pair<int, int>> stack;
+        if (!leaf(K.out[k])) stack.push_back({K.out[k], 0});
+        while (!stack.empty()) {
+            auto& top = stack.back();
+            const int i = top.first;
+            if (seen[i]) {
+                stack.pop_back();
+                continue;
+            }
+            if (top.second < n_operands(i)) {
+                const int c = op(i, 1 + top.second++);
+                if (!leaf(c) && !seen[c]) stack.push_back({c, 0});
+                continue;
+            }
+            seen[i] = 1;
+            order.push_back(i);
+            stack.pop_back();
+        }
+        order.push_back(-1 - k);
+    }
+    const int len = (int)order.size();
+    std::vector<int> last(n, -1);  // position of the last use of each computed value
+    for (int e = 0; e < len; ++e) {
+        const int i = order[e];
+        if (i < 0) last[K.out[-1 - i]] = e;
+        else
+            for (int q = 0; q < n_operands(i); ++q) last[op(i, 1 + q)] = e;
+    }
+    std::vector<int> slot(n, -1), free_slots;  // free slots in descending order: the lowest is handed out first
+    int n_slots = 0;
+    auto give_back = [&](int sl) {
+        free_slots.push_back(sl);
+        std::sort(free_slots.begin(), free_slots.end(), std::greater<int>());
+    };
+    auto take = [&]() {
+        if (free_slots.empty()) return n_slots++;
+        const int sl = free_slots.back();
+        free_slots.pop_back();
+        return sl;
+    };
+    auto load = [&](int v) {  // a leaf into a scratch slot
+        const int sl = take();
+        words.push_back(make_int4(op(v, 0), sl, op(v, 1), 0));
+        return sl;
+    };
+    const size_t base = words.size();
+    for (int e = 0; e < len && n_slots <= DTO_MAX_PROGRAM_SLOTS; ++e) {
+        const int i = order[e];
+        if (i < 0) {
+            const int v = K.out[-1 - i];
+            const int sl = leaf(v) ? load(v) : slot[v];
+            words.push_back(make_int4(DTO_OP_OUT, -1 - i, sl, 0));
+            if (leaf(v) || last[v] == e) give_back(sl);
+            continue;
+        }
+        const int o = op(i, 0), nop = n_operands(i);
+        int sl[2] = {op(i, 1), op(i, 2)};  // leaf operands of an operation are indices, POWC's b a constant index
+        for (int q = 0; q < nop; ++q) {
+            const int c = op(i, 1 + q);
+            if (!leaf(c)) sl[q] = slot[c];
+            else if (q == 1 && c == op(i, 1)) sl[1] = sl[0];  // x * x of a leaf: one load
+            else sl[q] = load(c);
+        }
+        for (int q = 0; q < nop; ++q) {  // operands whose last use this is free their slots (each slot once)
+            const int c = op(i, 1 + q);
+            if (q == 1 && c == op(i, 1)) continue;
+            if (leaf(c) || last[c] == e) give_back(sl[q]);
+        }
+        slot[i] = take();
+        words.push_back(make_int4(o, slot[i], sl[0], sl[1]));
+    }
+    if (n_slots > DTO_MAX_PROGRAM_SLOTS) {
+        words.resize(base);
+        msg = who + "needs more than " + std::to_string(DTO_MAX_PROGRAM_SLOTS) +
+              " live values at once, above the interpreter's limit (DTO_MAX_PROGRAM_SLOTS)";
+        return DTO_ERR_UNSUPPORTED;
+    }
+    // constants after the words, two per int4
+    const int cw = (K.n_consts + 1) / 2;
+    const size_t at = words.size();
+    words.resize(at + cw, make_int4(0, 0, 0, 0));
+    if (K.n_consts > 0) memcpy(&words[at], K.consts, sizeof(double) * K.n_consts);
+    return DTO_OK;
+}
+
+// compile and upload: the device view of program `index` for a term with n_vars variables, n_params parameters and
+// n_out outputs
+static int upload_knot_program(dto_handle* h, const dto_problem_desc* d, int index, int n_vars, int n_params, int n_out, DProgram& pg) {
+    std::vector<int4> words;
+    std::string msg;
+    const int rc = compile_knot_program(d, index, n_vars, n_params, n_out, words, msg);
+    if (rc != DTO_OK) return fail_create(h, rc, msg);
+    const int cw = (d->programs[index].n_consts + 1) / 2;
+    pg.n_code = (int)words.size() - cw;
+    pg.code = dev_upload(h, words.data(), words.size());
+    if (!pg.code) return fail_create(h, DTO_ERR_ALLOC, "device allocation failed (knot program)");
+    return DTO_OK;
+}
+
 extern "C" const char* dto_last_error(const dto_handle* h) { return h ? h->err.c_str() : g_create_error.c_str(); }
 
 extern "C" void dto_destroy(dto_handle* h) {
@@ -266,7 +435,11 @@ extern "C" void dto_destroy(dto_handle* h) {
 extern "C" int dto_create(const dto_problem_desc* d, dto_handle** out) {
     if (!d || !out) return fail_create(nullptr, DTO_ERR_INVALID, "null descriptor");
     *out = nullptr;
-    if (d->abi_version != DTO_B200_ABI_VERSION) return fail_create(nullptr, DTO_ERR_INVALID, "ABI version mismatch");
+    // version 3 descriptors (no knot programs) end before n_programs: those fields are read only at version 4
+    if (d->abi_version != DTO_B200_ABI_VERSION && d->abi_version != 3) return fail_create(nullptr, DTO_ERR_INVALID, "ABI version mismatch");
+    const bool with_programs = d->abi_version >= 4;
+    if (with_programs && (d->n_programs < 0 || (d->n_programs > 0 && !d->programs)))
+        return fail_create(nullptr, DTO_ERR_INVALID, "bad knot program table");
     if (d->N < 2 || d->z < 1 || d->batch < 1) return fail_create(nullptr, DTO_ERR_INVALID, "need N >= 2, z >= 1, batch >= 1");
     if (d->dt_off < 0 || d->dt_off >= d->z) return fail_create(nullptr, DTO_ERR_INVALID, "timestep component outside the knot");
     if (d->n_integrators < 1)
@@ -525,7 +698,8 @@ extern "C" int dto_create(const dto_problem_desc* d, dto_handle** out) {
         if (s.kind != DTO_OBJ_QUADREG && s.kind != DTO_OBJ_KNOT && s.kind != DTO_OBJ_LINREG && s.kind != DTO_OBJ_GLOBAL_KNOT)
             return fail_create(h, DTO_ERR_UNSUPPORTED, "unknown objective kind");
         const bool with_globals = s.kind == DTO_OBJ_GLOBAL_KNOT;
-        if ((s.kind == DTO_OBJ_KNOT || with_globals) && !knot_lfun_known(s.fn))
+        const bool program = with_programs && s.fn == DTO_L_PROGRAM;
+        if ((s.kind == DTO_OBJ_KNOT || with_globals) && !knot_lfun_known(s.fn) && !program)
             return fail_create(h, DTO_ERR_UNSUPPORTED, "knot objective function is not in the device catalogue");
         const int ngv = with_globals ? s.n_gvars : 0;
         if (s.n_vars < (with_globals ? 0 : 1) || s.n_vars + ngv > DTO_MAX_KNOTFN_VARS || (s.n_vars > 0 && !s.var_offs))
@@ -574,6 +748,10 @@ extern "C" int dto_create(const dto_problem_desc* d, dto_handle** out) {
             if (!s.Qs || (s.n_params > 0 && !s.params)) return fail_create(h, DTO_ERR_INVALID, "knot objective: missing Qs/params");
             O.params = dev_upload(h, s.params, (size_t)std::max(1, s.n_params) * s.n_times);
             O.Qs = dev_upload(h, s.Qs, s.n_times);
+            if (program) {
+                const int rc = upload_knot_program(h, d, s.program, O.nv, s.n_params, 1, O.prog);
+                if (rc != DTO_OK) return rc;
+            }
         }
     }
 
@@ -614,14 +792,16 @@ extern "C" int dto_create(const dto_problem_desc* d, dto_handle** out) {
     for (int i = 0; i < d->n_constraints; ++i) {
         const dto_constraint_desc& s = d->constraints[i];
         h->cons.push_back(s);
-        if (!knot_cfun_known(s.fn)) return fail_create(h, DTO_ERR_UNSUPPORTED, "knot constraint function is not in the device catalogue");
+        const bool program = with_programs && s.fn == DTO_G_PROGRAM;
+        if (!knot_cfun_known(s.fn) && !program)
+            return fail_create(h, DTO_ERR_UNSUPPORTED, "knot constraint function is not in the device catalogue");
         const int ngv = s.n_gvars;
         if (ngv < 0 || s.n_vars < 0 || s.n_vars + ngv < 1 || s.n_vars + ngv > DTO_MAX_KNOTFN_VARS || s.g_dim < 1 || s.g_dim > 16 ||
             (s.n_vars > 0 && !s.var_offs) || (ngv > 0 && !s.gvar_offs))
             return fail_create(h, DTO_ERR_INVALID, "constraint: bad variable list or g_dim");
         if (s.fn == DTO_G_NORM_PRODUCT) {
             if (s.g_dim != 2 || s.n_params < 3) return fail_create(h, DTO_ERR_INVALID, "constraint: norm_product has g_dim 2 and 3 parameters");
-        } else if (s.fn != DTO_G_LINEAR && s.g_dim != 1)
+        } else if (s.fn != DTO_G_LINEAR && !program && s.g_dim != 1)
             return fail_create(h, DTO_ERR_INVALID, "constraint: g_dim must be 1 for this function");
         std::vector<int> all_offs(s.var_offs, s.var_offs + s.n_vars), g2l(G, -1);
         for (int v = 0; v < ngv; ++v) {
@@ -663,6 +843,11 @@ extern "C" int dto_create(const dto_problem_desc* d, dto_handle** out) {
         C.own_knot = dev_upload(h, con_own_knot[i].data(), con_own_knot[i].size());
         C.knot_to_own = dev_upload(h, k2o.data(), k2o.size());
         C.params = dev_upload(h, s.params, (size_t)std::max(1, s.n_params) * s.n_times);
+        if (program) {
+            if (s.n_params > 0 && !s.params) return fail_create(h, DTO_ERR_INVALID, "constraint: missing params");
+            const int rc = upload_knot_program(h, d, s.program, C.nv, s.n_params, s.g_dim, C.prog);
+            if (rc != DTO_OK) return rc;
+        }
         h->con_goff.push_back(cgoff);
         cgoff += (long long)s.g_dim * s.n_times;
         cloff += (long long)s.g_dim * C.nt_own;

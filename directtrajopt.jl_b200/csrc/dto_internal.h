@@ -15,6 +15,15 @@
 #define DTO_MAX_KNOTFN_VARS 128
 
 // ---- device views (passed by value to kernels) ------------------------------------------------
+// A compiled knot program (knot_program.cuh): n_code words {opcode, dst slot, a, b}, then the constants as doubles, in
+// one device allocation.  Outputs are DTO_OP_OUT words (dst = output index, a = slot).
+enum { DTO_OP_OUT = 16 };
+struct DProgram {
+    const int4* code;  // null: the term is a catalogue function
+    int n_code;
+    int _pad;
+    __host__ __device__ const double* consts() const { return reinterpret_cast<const double*>(code + n_code); }
+};
 struct DInt {
     int kind, x_off, n, u_off, m, t_off, order, n_carrier;
     int doff;           // sum of x_dim of the integrators before this one
@@ -67,6 +76,7 @@ struct DObj {
     const double* baseline;   // nv x N (global knots), may be null
     const double* params;
     const double* Qs;
+    DProgram prog;            // fn == DTO_L_PROGRAM
 };
 
 struct DCon {
@@ -80,6 +90,7 @@ struct DCon {
     const int* knot_to_own;
     const double* params;
     const long long* jac_pos;     // [nt_own][gd][nv] local Jacobian position or -1
+    DProgram prog;                // fn == DTO_G_PROGRAM
 };
 
 // Terms that read global variables (global_objectives.jl, global_constraint.jl, global_knot_point_constraint.jl):
@@ -126,6 +137,8 @@ struct DProb {
     DObj ob[DTO_MAX_OBJ];
     DCon co[DTO_MAX_CON];
 };
+// every kernel takes the problem by value: it must fit the kernel-parameter space of sm_70+ (32764 bytes since CUDA 12.1)
+static_assert(sizeof(DProb) <= 32764, "DProb exceeds the kernel-parameter limit");
 
 // Macro steps of one tdbilinear interval.  The extrapolation scheme (8 columns of the modified midpoint rule, order 16) is
 // accurate to ~1e-13 per macro step while theta = |dt| (||G(u, .)||_1 bound + carrier frequency) stays below 1: the error of
@@ -288,5 +301,8 @@ void launch_jac_product(const DProb& P, const double* jac, const long long* rows
                         double* y, bool transpose, cudaStream_t st, long long* launches);
 // knot-constraint Jacobian at a host point (used at construction for the stored pattern): runs the
 // same device templates so that pattern and values come from one implementation.
+// knot programs: one thread per (problem, owned time, seed) for the values and Jacobian of a DTO_G_PROGRAM constraint
+void launch_knot_program(const DProb& P, int ci, const double* Z, double* g, double* jac, double* dense_probe, cudaStream_t st,
+                         long long* launches);
 void launch_constraint_pattern_probe(const DProb& P, const double* Z, double* dense_jac /*[sum nt_own*gd*nv]*/, cudaStream_t st,
                                      long long* launches);

@@ -25,6 +25,7 @@ __device__ __forceinline__ double warp_sum(double v) {
 }
 
 // thread per (problem, objective slot, global variable)
+template <bool Prog>
 __global__ void global_grad_kernel(DProb P, const double* __restrict__ Z, long long total) {
     const long long t = (long long)blockIdx.x * blockDim.x + threadIdx.x;
     if (t >= total) return;
@@ -40,13 +41,14 @@ __global__ void global_grad_kernel(DProb P, const double* __restrict__ Z, long l
         const double* zk = Z + (long long)b * P.n_vars_local + (long long)O.own_knot[j] * P.z;
         const double* gp = Z + (long long)b * P.n_vars_local + (long long)P.nK * P.z;
         const double* prm = O.params + (long long)O.own_ti[j] * O.np;
-        const HDual res = knot_lfun<HDual>(O.fn, SeededVars{zk, gp, O.var_offs, O.nvk, v, -1}, O.nv, prm);
+        const HDual res = knot_lfun<Prog, HDual>(O.fn, O.prog, SeededVars{zk, gp, O.var_offs, O.nvk, v, -1}, O.nv, prm);
         val = O.weight * O.Qs[O.own_ti[j]] * res.d1;
     }
     L.scratchG[((long long)b * L.S_obj + s) * L.G + gi] = val;
 }
 
 // thread per (problem, slot, item): item < Gtri -> (gi <= gj) pair into the scratch; then (knot variable a, global gi)
+template <bool Prog>
 __global__ void global_hess_kernel(DProb P, const double* __restrict__ Z, double sigma, const double* __restrict__ mu,
                                    double* __restrict__ hess, double* __restrict__ kg_probe, long long total) {
     const long long t = (long long)blockIdx.x * blockDim.x + threadIdx.x;
@@ -86,7 +88,7 @@ __global__ void global_hess_kernel(DProb P, const double* __restrict__ Z, double
                 const DObj& O = P.ob[L.slot_term[s]];
                 const double* zk = Z + (long long)b * P.n_vars_local + (long long)O.own_knot[j] * P.z;
                 const double* prm = O.params + (long long)O.own_ti[j] * O.np;
-                const HDual res = knot_lfun<HDual>(O.fn, SeededVars{zk, gp, O.var_offs, O.nvk, a, c}, O.nv, prm);
+                const HDual res = knot_lfun<Prog, HDual>(O.fn, O.prog, SeededVars{zk, gp, O.var_offs, O.nvk, a, c}, O.nv, prm);
                 val = sigma * O.weight * O.Qs[O.own_ti[j]] * res.d12;
             }
         } else {
@@ -94,7 +96,7 @@ __global__ void global_hess_kernel(DProb P, const double* __restrict__ Z, double
             const double* zk = Z + (long long)b * P.n_vars_local + (long long)C.own_knot[j] * P.z;
             const double* prm = C.params + (long long)C.own_ti[j] * C.np;
             HDual out[16];
-            knot_cfun<HDual>(C.fn, SeededVars{zk, gp, C.var_offs, C.nvk, a, c}, C.nv, prm, out, C.gd);
+            knot_cfun<Prog, HDual>(C.fn, C.prog, SeededVars{zk, gp, C.var_offs, C.nvk, a, c}, C.nv, prm, out, C.gd);
             if (kg_probe != nullptr) {  // structure probe: mu = ones (evaluator.jl:170-171)
                 for (int q = 0; q < C.gd; ++q) val += out[q].d12;
             } else {
@@ -131,6 +133,15 @@ __global__ void column_sum_kernel(int batch, int S, int W, const double* __restr
     if (lane == 0) out[(long long)b * out_stride + out_off + p] = acc;
 }
 
+// some term with global variables is a knot program (objectives: obj = true, constraints: obj = false)
+bool global_programs(const DProb& P, bool obj) {
+    for (int i = 0; i < P.n_obj && obj; ++i)
+        if (P.ob[i].kind == DTO_OBJ_GLOBAL_KNOT && P.ob[i].fn == DTO_L_PROGRAM) return true;
+    for (int i = 0; i < P.n_con && !obj; ++i)
+        if (P.co[i].nv > P.co[i].nvk && P.co[i].fn == DTO_G_PROGRAM) return true;
+    return false;
+}
+
 }  // namespace
 
 void launch_global_gradient(const DProb& P, const double* Z, double* grad, cudaStream_t st, long long* launches) {
@@ -138,7 +149,8 @@ void launch_global_gradient(const DProb& P, const double* Z, double* grad, cudaS
     if (L.G == 0 || grad == nullptr) return;
     if (L.S_obj > 0) {
         const long long total = (long long)P.batch * L.S_obj * L.G;
-        global_grad_kernel<<<(unsigned)((total + 127) / 128), 128, 0, st>>>(P, Z, total);
+        if (global_programs(P, true)) global_grad_kernel<true><<<(unsigned)((total + 127) / 128), 128, 0, st>>>(P, Z, total);
+        else global_grad_kernel<false><<<(unsigned)((total + 127) / 128), 128, 0, st>>>(P, Z, total);
         ++*launches;
     }
     const long long cols = (long long)P.batch * L.G;
@@ -157,7 +169,10 @@ void launch_global_hessian(const DProb& P, const double* Z, double sigma, const 
         cudaMemset2DAsync(hess + L.hess_tail_off, sizeof(double) * P.nnz_hess_local, 0, sizeof(double) * L.n_hess_tail, P.batch, st);
     }
     const long long total = (long long)P.batch * L.S * (gtri + L.KV * L.G);
-    global_hess_kernel<<<(unsigned)((total + 127) / 128), 128, 0, st>>>(P, Z, sigma, mu, hess, kg_probe, total);
+    if (global_programs(P, true) || global_programs(P, false))
+        global_hess_kernel<true><<<(unsigned)((total + 127) / 128), 128, 0, st>>>(P, Z, sigma, mu, hess, kg_probe, total);
+    else
+        global_hess_kernel<false><<<(unsigned)((total + 127) / 128), 128, 0, st>>>(P, Z, sigma, mu, hess, kg_probe, total);
     ++*launches;
     if (kg_probe == nullptr) {
         const long long cols = (long long)P.batch * gtri;

@@ -1,5 +1,5 @@
 // Device catalogue of knot-point functions and the forward-mode hyper-dual number they are
-// differentiated with.  This replaces the ForwardDiff closures of the reference
+// differentiated with; user functions given as knot programs dispatch to the interpreter of knot_program.cuh.  This replaces the ForwardDiff closures of the reference
 // (src/constraints/nonlinear/knot_point_constraint.jl:254-294, src/objectives/knot_point_objectives.jl:184-243):
 // every catalogue function is written once as a template over the scalar type and instantiated with
 // `double` (values) and `HDual` (first and second derivatives in one pass: seeds e_a, e_b give
@@ -56,9 +56,24 @@ struct SeededVars {
     }
 };
 
+#ifdef __CUDACC__
+#include "knot_program.cuh"
+#endif
+
+// `Prog`: whether the caller handles knot programs (DTO_G_PROGRAM / DTO_L_PROGRAM, compiled into `pg`).  Kernels are
+// instantiated both ways and the host launches the program-capable form only for problems that have programs: the
+// interpreter call costs the caller registers, and the catalogue-only forms keep the allocation they were tuned with.
 // ---- constraint functions g(v; p) -> out[gd] ---------------------------------------------------
-template <class T, class Vars>
-__host__ __device__ inline void knot_cfun(int fn, const Vars& v, int nv, const double* p, T* out, int gd) {
+template <bool Prog, class T, class Vars>
+__host__ __device__ inline void knot_cfun(int fn, const DProgram& pg, const Vars& v, int nv, const double* p, T* out, int gd) {
+#ifdef __CUDA_ARCH__
+    if constexpr (Prog) {
+        if (fn == DTO_G_PROGRAM) {
+            run_knot_program<T, Vars>(pg.code, pg.n_code, v, p, out);
+            return;
+        }
+    }
+#endif
     switch (fn) {
         case DTO_G_NORM_MINUS_C: {  // [norm(v) - c]
             T s = T(0.0);
@@ -100,8 +115,17 @@ __host__ __device__ inline void knot_cfun(int fn, const Vars& v, int nv, const d
 }
 
 // ---- objective functions l(v; p) -> scalar ------------------------------------------------------
-template <class T, class Vars>
-__host__ __device__ inline T knot_lfun(int fn, const Vars& v, int nv, const double* p) {
+template <bool Prog, class T, class Vars>
+__host__ __device__ inline T knot_lfun(int fn, const DProgram& pg, const Vars& v, int nv, const double* p) {
+#ifdef __CUDA_ARCH__
+    if constexpr (Prog) {
+        if (fn == DTO_L_PROGRAM) {
+            T r[1];
+            run_knot_program<T, Vars>(pg.code, pg.n_code, v, p, r);
+            return r[0];
+        }
+    }
+#endif
     switch (fn) {
         case DTO_L_NORMSQ_PLUS_P: {
             T s = T(0.0);

@@ -10,6 +10,7 @@ import ctypes as C
 import numpy as np
 
 from . import _lib
+from .knot_program import KnotProgram
 from .components import (AbstractIntegrator, AbstractNonlinearConstraint, AbstractObjective, BilinearIntegrator,
                          CompositeObjective, DerivativeIntegrator, GlobalKnotPointObjective, KnotPointObjective,
                          MinimumTimeObjective, NullObjective, NonlinearGlobalKnotPointConstraint,
@@ -89,6 +90,15 @@ class Evaluator:
         self.batch = int(batch)
         t = prob.trajectory
         keep = []  # keep every array alive until dto_create returns
+        programs = []  # (ops, out, consts) of every KnotProgram term, indexed by the descriptors' `program`
+
+        def knot_fn(fn, catalogue, program_id, n_vars):
+            """(fn id, program index) of a term's knot function"""
+            if isinstance(fn, KnotProgram):
+                tape = fn.trace(n_vars)
+                programs.append((np.ascontiguousarray(tape.ops), np.ascontiguousarray(tape.out), _f64(tape.consts)))
+                return program_id, len(programs) - 1
+            return catalogue[fn.name], 0
 
         ints = (_lib.IntegratorDesc * max(1, len(prob.integrators)))()
         for i, it in enumerate(prob.integrators):
@@ -152,7 +162,7 @@ class Evaluator:
                 d.D = ob.D
             elif isinstance(ob, KnotPointObjective):
                 d.kind = _lib.OBJ_KNOT
-                d.fn = _lib.L_FUNCS[ob.l.name]
+                d.fn, d.program = knot_fn(ob.l, _lib.L_FUNCS, _lib.L_PROGRAM, len(ob.var_offs))
                 vo, tm = np.asarray(ob.var_offs, np.int32), np.asarray(ob.times, np.int32)
                 pr, Qs = _f64(ob.params), _f64(ob.Qs)
                 keep += [vo, tm, pr, Qs]
@@ -160,7 +170,7 @@ class Evaluator:
                 d.n_params, d.params, d.Qs = pr.shape[1], _dp(pr), _dp(Qs)
             elif isinstance(ob, GlobalKnotPointObjective):
                 d.kind = _lib.OBJ_GLOBAL_KNOT
-                d.fn = _lib.L_FUNCS[ob.l.name]
+                d.fn, d.program = knot_fn(ob.l, _lib.L_FUNCS, _lib.L_PROGRAM, len(ob.var_offs) + len(ob.gvar_offs))
                 vo, go, tm = np.asarray(ob.var_offs, np.int32), np.asarray(ob.gvar_offs, np.int32), np.asarray(ob.times, np.int32)
                 pr, Qs = _f64(ob.params), _f64(ob.Qs)
                 keep += [vo, go, tm, pr, Qs]
@@ -177,7 +187,8 @@ class Evaluator:
         cons = (_lib.ConstraintDesc * max(1, len(self.constraints)))()
         for i, c in enumerate(self.constraints):
             d = cons[i]
-            d.fn = _lib.G_FUNCS[c.g.name]
+            d.fn, d.program = knot_fn(c.g, _lib.G_FUNCS, _lib.G_PROGRAM,
+                                      len(c.var_offs) + (len(c.gvar_offs) if isinstance(c, NonlinearGlobalKnotPointConstraint) else 0))
             d.equality = int(c.equality)
             vo, tm, pr = np.asarray(c.var_offs, np.int32), np.asarray(c.times, np.int32), _f64(c.params)
             keep += [vo, tm, pr]
@@ -200,6 +211,13 @@ class Evaluator:
         desc.integrators, desc.objectives, desc.constraints = ints, objs, cons
         desc.Z0 = _dp(Z0a)
         desc.global_dim = t.global_dim
+        progs = (_lib.KnotProgramDesc * max(1, len(programs)))()
+        for i, (ops, out, consts) in enumerate(programs):
+            keep += [ops, out, consts]
+            progs[i].n_ops, progs[i].ops = ops.shape[0], _ip(ops)
+            progs[i].n_out, progs[i].out = out.size, _ip(out)
+            progs[i].n_consts, progs[i].consts = consts.size, _dp(consts)
+        desc.n_programs, desc.programs = len(programs), progs
         h = C.c_void_p()
         rc = lib.dto_create(C.byref(desc), C.byref(h))
         if rc != _lib.DTO_OK:

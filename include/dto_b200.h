@@ -56,7 +56,7 @@
 extern "C" {
 #endif
 
-#define DTO_B200_ABI_VERSION 3
+#define DTO_B200_ABI_VERSION 4
 
 typedef struct dto_handle dto_handle;
 
@@ -83,14 +83,49 @@ enum {
     DTO_G_NORM_MINUS_C = 1, DTO_G_NORMSQ_MINUS_C = 2, DTO_G_SQDIST_MINUS_C = 3, DTO_G_LINEAR = 4,
     /* [norm(v1) - c1; norm(v1) norm(v2) - c2], v = [v1 (n1 entries); v2], p = [c1, c2, n1]: the reference's test
      * function for knot + global variables (global_knot_point_constraint.jl:267-270) */
-    DTO_G_NORM_PRODUCT = 5
+    DTO_G_NORM_PRODUCT = 5,
+    /* a user function given as a knot program (dto_knot_program, below): `program` of the descriptor indexes
+     * dto_problem_desc::programs (ABI version 4) */
+    DTO_G_PROGRAM = 100
 };
 /* device catalogue of knot objective functions l(v; p) (src/objectives/knot_point_objectives.jl:65-72) */
 enum {
     DTO_L_NORMSQ_PLUS_P = 1, DTO_L_SQDIST = 2, DTO_L_LINEAR = 3, DTO_L_ISO_INFIDELITY = 4,
     /* norm(v[0:h] - v[h:2h])^2, h = n/2: state against a goal held in a global (global_objectives.jl:364-369) */
-    DTO_L_SPLIT_SQDIST = 5
+    DTO_L_SPLIT_SQDIST = 5,
+    DTO_L_PROGRAM = 100 /* a knot program with one output (ABI version 4) */
 };
+
+/* Knot programs: a user-written g(v; p) / l(v; p) as an SSA tape (the reference's closures of
+ * knot_point_constraint.jl:76-83 and knot_point_objectives.jl:65-72, traced once by the front end).
+ * Value i of the tape is defined by ops[3 i .. 3 i + 2] = {opcode, a, b}:
+ *   DTO_OP_VAR    a = variable index < n_vars + n_gvars of the term (knot variables first, then global variables)
+ *   DTO_OP_PARAM  a = index into this time's parameter row, < n_params
+ *   DTO_OP_CONST  a = index into consts
+ *   ADD SUB MUL DIV                  values a and b
+ *   NEG SQRT EXP LOG SIN COS TANH    value a
+ *   POWC          value a raised to consts[b] (an integer-valued exponent is valid for negative bases)
+ * Operands of non-leaf operations reference earlier values (< i): the tape is acyclic by construction.  out[k] is the
+ * value of output k (g_dim outputs for a constraint, one for an objective).  dto_create drops dead values, orders the
+ * rest depth-first from the outputs and allocates registers of the device interpreter by linear scan; a program longer
+ * than DTO_MAX_PROGRAM_OPS or needing more than DTO_MAX_PROGRAM_SLOTS live values is DTO_ERR_UNSUPPORTED, a malformed
+ * one DTO_ERR_INVALID -- at construction, never mid-solve. */
+enum {
+    DTO_OP_VAR = 1, DTO_OP_PARAM = 2, DTO_OP_CONST = 3,
+    DTO_OP_ADD = 4, DTO_OP_SUB = 5, DTO_OP_MUL = 6, DTO_OP_DIV = 7,
+    DTO_OP_NEG = 8, DTO_OP_SQRT = 9, DTO_OP_EXP = 10, DTO_OP_LOG = 11, DTO_OP_SIN = 12, DTO_OP_COS = 13, DTO_OP_TANH = 14,
+    DTO_OP_POWC = 15
+};
+#define DTO_MAX_PROGRAM_OPS 4096
+#define DTO_MAX_PROGRAM_SLOTS 32
+
+typedef struct {
+    int32_t n_ops, n_out;
+    const int32_t* ops;    /* n_ops x {opcode, a, b} */
+    const int32_t* out;    /* n_out value indices */
+    int32_t n_consts, _pad;
+    const double* consts;
+} dto_knot_program;
 
 /* One dynamics integrator (src/integrators/{bilinear,derivative,time_dependent_bilinear}_integrator.jl).
  * Component offsets are 0-based positions inside one knot. */
@@ -133,7 +168,7 @@ typedef struct {
     const double* baseline;  /* quadreg: n_vars x N column-major, may be NULL (= zeros) */
     double D;                /* mintime scale (src/objectives/minimum_time_objective.jl:24-26) */
     int32_t n_params;        /* knot: doubles of parameters per listed time */
-    int32_t _pad;
+    int32_t program;         /* fn == DTO_L_PROGRAM: index into dto_problem_desc::programs (ABI 3: padding) */
     const double* params;    /* knot: n_times x n_params, row-major */
     const double* Qs;        /* knot: n_times weights */
     int32_t n_gvars;         /* global_knot: global variables appended to the knot variables */
@@ -155,7 +190,7 @@ typedef struct {
     /* global variables appended to the knot variables: g([knot vars; global vars], p).  n_vars == 0 with
      * times = [1] is a NonlinearGlobalConstraint (rows = g_dim). */
     int32_t n_gvars;
-    int32_t _pad;
+    int32_t program;          /* fn == DTO_G_PROGRAM: index into dto_problem_desc::programs (ABI 3: padding) */
     const int32_t* gvar_offs; /* 0-based positions inside global_data */
 } dto_constraint_desc;
 
@@ -180,7 +215,10 @@ typedef struct {
      * With batch > 1 problem 0 defines the pattern.  May be NULL when there are no knot constraints. */
     const double* Z0;
     int32_t global_dim;  /* traj.global_dim: variables after the knots in Z (0 = none) */
-    int32_t _pad;
+    /* ABI version 4: the knot programs that DTO_G_PROGRAM / DTO_L_PROGRAM terms index.  dto_create accepts version 3
+     * descriptors, which end before these fields and cannot name programs. */
+    int32_t n_programs;
+    const dto_knot_program* programs;
 } dto_problem_desc;
 
 typedef struct {
