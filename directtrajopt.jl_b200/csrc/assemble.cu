@@ -160,10 +160,12 @@ __device__ __forceinline__ double group_sum(double v, unsigned gmask) {
 // Narrow knots are register-limited at the compiler's own allocation (68 registers: 3 CTAs of 256 threads per SM, a third
 // of the warp slots, too few loads in flight for a latency-bound stream-out): capped to 5 (GS = 8) / 4 (GS = 16) CTAs per SM
 // (c5: 560 -> 477 us, 0.62 of the measured HBM copy rate).
-template <int GS, bool Prog>
-__global__ void __launch_bounds__(256, GS == 8 ? 5 : (GS == 16 ? 4 : 1))
-hessian_assemble_kernel(DProb P, const double* __restrict__ Z, double sigma, const double* __restrict__ mu, double* __restrict__ hess,
-                        int warps_per_cta, long long total) {
+// Left: the launch covers only local knot 0 of a linked shard that starts after knot 1 (hessian_assemble_left_kernel); the
+// previous interval's rows were received from the left neighbour into the leading row of DInt::hs (shard_link.cu).
+template <int GS, bool Prog, bool Left>
+__device__ __forceinline__ void hessian_assemble_body(const DProb& P, const double* __restrict__ Z, double sigma,
+                                                      const double* __restrict__ mu, double* __restrict__ hess, int warps_per_cta,
+                                                      long long total) {
     extern __shared__ double sm[];
     constexpr int GPW = 32 / GS;  // groups per warp
     const int z = P.z, lane = threadIdx.x & 31, tid = lane % GS, nt = GS;
@@ -231,8 +233,8 @@ hessian_assemble_kernel(DProb P, const double* __restrict__ Z, double sigma, con
             }
             __syncwarp(gmask);
         }
-        if (I.kind == DTO_INT_TDBILINEAR && I.order == 1 && kl >= 1) {
-            // previous interval: (next,next) -> this knot's diagonal block; (own,next) -> cross block
+        if (I.kind == DTO_INT_TDBILINEAR && I.order == 1 && (kl >= 1 || Left)) {
+            // previous interval: (next,next) -> this knot's diagonal block; (own,next) -> cross block (Left: row -1)
             const double* hs = I.hs + ((long long)b * P.nI + (kl - 1)) * I.hs_stride;
             const double* hpp = hs + (long long)np * n;
             for (int e = tid; e < np * n; e += nt) {
@@ -374,6 +376,20 @@ hessian_assemble_kernel(DProb P, const double* __restrict__ Z, double sigma, con
             }
         }
     }
+}
+
+template <int GS, bool Prog>
+__global__ void __launch_bounds__(256, GS == 8 ? 5 : (GS == 16 ? 4 : 1))
+hessian_assemble_kernel(DProb P, const double* __restrict__ Z, double sigma, const double* __restrict__ mu, double* __restrict__ hess,
+                        int warps_per_cta, long long total) {
+    hessian_assemble_body<GS, Prog, false>(P, Z, sigma, mu, hess, warps_per_cta, total);
+}
+
+template <int GS, bool Prog>
+__global__ void __launch_bounds__(256, GS == 8 ? 5 : (GS == 16 ? 4 : 1))
+hessian_assemble_left_kernel(DProb P, const double* __restrict__ Z, double sigma, const double* __restrict__ mu,
+                             double* __restrict__ hess, int warps_per_cta, long long total) {
+    hessian_assemble_body<GS, Prog, true>(P, Z, sigma, mu, hess, warps_per_cta, total);
 }
 
 // Knot-objective Hessians: w * Q * Hess l, one thread per (problem, listed knot, variable pair), into DProb::knot_side (a
@@ -749,7 +765,7 @@ size_t hessian_assemble_smem_bytes(const DProb& P) {
 }
 
 void launch_hessian_assemble(const DProb& P, const double* Z, double sigma, const double* mu, double* hess, cudaStream_t st,
-                             long long* launches) {
+                             long long* launches, bool left_block) {
     const int nKc = std::min(P.kc1, P.nOwn) - P.kc0;
     if (nKc <= 0) return;
     const int GS = P.z <= 16 ? 8 : (P.z <= 24 ? 16 : 32), GPW = 32 / GS;
@@ -763,10 +779,21 @@ void launch_hessian_assemble(const DProb& P, const double* Z, double sigma, cons
         cudaFuncSetAttribute(hessian_assemble_kernel<32, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
         cudaFuncSetAttribute(hessian_assemble_kernel<16, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
         cudaFuncSetAttribute(hessian_assemble_kernel<8, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
+        cudaFuncSetAttribute(hessian_assemble_left_kernel<32, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
+        cudaFuncSetAttribute(hessian_assemble_left_kernel<16, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
+        cudaFuncSetAttribute(hessian_assemble_left_kernel<8, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
+        cudaFuncSetAttribute(hessian_assemble_left_kernel<32, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
+        cudaFuncSetAttribute(hessian_assemble_left_kernel<16, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
+        cudaFuncSetAttribute(hessian_assemble_left_kernel<8, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
     }
     const long long total = (long long)nKc * P.batch;
     const unsigned grid = (unsigned)((total + (long long)W * GPW - 1) / ((long long)W * GPW));
-    if (any_program_constraint(P)) {
+    if (left_block) {  // local knot 0 only (kc0 = 0, kc1 = 1)
+        const bool prog = any_program_constraint(P);
+        if (GS == 8) (prog ? hessian_assemble_left_kernel<8, true> : hessian_assemble_left_kernel<8, false>)<<<grid, W * 32, smem, st>>>(P, Z, sigma, mu, hess, W, total);
+        else if (GS == 16) (prog ? hessian_assemble_left_kernel<16, true> : hessian_assemble_left_kernel<16, false>)<<<grid, W * 32, smem, st>>>(P, Z, sigma, mu, hess, W, total);
+        else (prog ? hessian_assemble_left_kernel<32, true> : hessian_assemble_left_kernel<32, false>)<<<grid, W * 32, smem, st>>>(P, Z, sigma, mu, hess, W, total);
+    } else if (any_program_constraint(P)) {
         if (GS == 8) hessian_assemble_kernel<8, true><<<grid, W * 32, smem, st>>>(P, Z, sigma, mu, hess, W, total);
         else if (GS == 16) hessian_assemble_kernel<16, true><<<grid, W * 32, smem, st>>>(P, Z, sigma, mu, hess, W, total);
         else hessian_assemble_kernel<32, true><<<grid, W * 32, smem, st>>>(P, Z, sigma, mu, hess, W, total);

@@ -129,7 +129,13 @@ struct dto_handle {
     unsigned long long epoch = 0;         // iterates uploaded since the link was made
     unsigned long long waited_epoch = 0;  // the halo of this iterate has been waited for
     unsigned long long scal_seq = 0;
-    bool link_ipc = false;                      // linked across processes: the publish kernel also waits for the right neighbour's knot
+    // boundary Hessian block (linear-spline tdbilinear, shard_link.cu): a shard after knot 1 receives it from its left
+    // neighbour, a shard with a right neighbour pushes it; hseq counts the Hessian evaluations since the link
+    long long hblk_len = 0;               // doubles of the block: sum of hs_stride over the linear-spline tdbilinear integrators
+    int hs_left = 0;                      // this shard's first knot needs the block (k0 > 1 and hblk_len > 0)
+    unsigned long long hseq = 0;
+    bool hs_push_now = false, hs_recv_now = false;  // the evaluation being enqueued pushes / receives the block of hseq
+    bool link_ipc = false;                     // linked across processes: the publish kernel also waits for the right neighbour's knot
     unsigned long long* d_scal_scratch = nullptr;  // {violation bits, arrival counter} of shard_scalars_kernel
     long long launches = 0;
     long long last_d2h_bytes = 0;
@@ -580,8 +586,6 @@ extern "C" int dto_create(const dto_problem_desc* d, dto_handle** out) {
                 return fail_create(h, DTO_ERR_INVALID, "tdbilinear integrator: bad components");
             if (!tdb_available()) return fail_create(h, DTO_ERR_UNSUPPORTED, "tdbilinear integrator kernel is not built into this library");
             if (s.spline_order != 0 && s.spline_order != 1) return fail_create(h, DTO_ERR_UNSUPPORTED, "Unsupported spline order");
-            if (s.spline_order == 1 && h->sharded && h->k0 > 1)
-                return fail_create(h, DTO_ERR_UNSUPPORTED, "tdbilinear with spline_order 1 cannot be knot-range sharded (needs a left halo)");
             I.G = dev_upload(h, s.G, nn);
             I.A = dev_upload(h, s.A, nn * s.u_dim);
             I.B = dev_upload(h, s.B, nn * s.u_dim);
@@ -644,7 +648,11 @@ extern "C" int dto_create(const dto_problem_desc* d, dto_handle** out) {
             }
             const int np = (s.spline_order == 1 ? 2 * s.u_dim : s.u_dim) + 2;
             I.hs_stride = np * s.x_dim + np * np;
-            if (s.spline_order == 1) P.any_cross = 1;
+            if (s.spline_order == 1) {
+                P.any_cross = 1;
+                h->hblk_len += I.hs_stride;
+                if (h->k0 > 1) h->hs_left = 1;
+            }
             {
                 const char* pin = getenv("DTO_B200_KERNEL");
                 I.variant = (I.Asw != nullptr && tdb_dmma_supported(I) && !(pin && strcmp(pin, "generic") == 0)) ? DTO_VAR_DMMA : DTO_VAR_GENERIC;
@@ -657,8 +665,12 @@ extern "C" int dto_create(const dto_problem_desc* d, dto_handle** out) {
             return fail_create(h, DTO_ERR_UNSUPPORTED, "unknown integrator kind");
         }
         if (I.hs_stride > 0 && d->eval_hessian) {
-            I.hs = dev_upload<double>(h, nullptr, (size_t)P.batch * std::max(P.nI, 1) * I.hs_stride);
+            // a shard whose first knot receives the previous interval's block (linear-spline tdbilinear) keeps it in a
+            // leading row: the assembler reads row kl - 1 = -1
+            const int lead = (s.kind == DTO_INT_TDBILINEAR && s.spline_order == 1 && h->k0 > 1) ? 1 : 0;
+            I.hs = dev_upload<double>(h, nullptr, (size_t)P.batch * (std::max(P.nI, 1) + lead) * I.hs_stride);
             if (!I.hs) return fail_create(h, DTO_ERR_ALLOC, "device allocation failed (Hessian scratch)");
+            I.hs += (size_t)lead * I.hs_stride;
         }
         h->int_goff.push_back(goff);
         goff += (long long)s.x_dim * (N - 1);
@@ -1501,6 +1513,19 @@ static bool ensure_aux(dto_handle* h) {
     return true;
 }
 
+// The boundary block's rows, one per linear-spline tdbilinear integrator: the last local interval's (pushed to the right
+// neighbour) or the leading row the left neighbour's block is received into
+static HsRows hs_rows(const DProb& P, bool leading) {
+    HsRows r{};
+    for (int i = 0; i < P.n_int; ++i) {
+        const DInt& I = P.in[i];
+        if (I.kind != DTO_INT_TDBILINEAR || I.order != 1) continue;
+        r.row[r.n] = I.hs + (leading ? -1LL : (long long)P.nI - 1) * I.hs_stride;
+        r.len[r.n++] = I.hs_stride;
+    }
+    return r;
+}
+
 // Interval kernels, analytic integrators and the Hessian assembler over the active knot range of P.
 static int eval_range(dto_handle* h, const DProb& P, const double* dZ, double sigma, const double* dmu, double* dg, double* djac,
                       double* dhess, EvalFlags f) {
@@ -1545,6 +1570,10 @@ static int eval_range(dto_handle* h, const DProb& P, const double* dZ, double si
         }
         if (timed) cudaEventRecord(h->ev_pool[h->ev_used++].second, h->stream);
     }
+    // the last local interval's second derivatives are written: on their way to the right neighbour, which assembles the
+    // knot they belong to
+    if (f.want_hess && h->hs_push_now && P.nI - 1 >= P.kc0 && P.nI - 1 < P.kc1)
+        launch_hs_push(h->xwin, h->peer_win[h->link_rank + 1], hs_rows(P, false), P.z, h->hblk_len, h->hseq, h->stream, &h->launches);
     if (f.want_g || f.want_jac) {
         if (fused_missed) {
             DProb Pn = P;
@@ -1556,6 +1585,20 @@ static int eval_range(dto_handle* h, const DProb& P, const double* dZ, double si
     }
     if (side_on_aux) CUDA_TRY(h, cudaStreamWaitEvent(h->stream, h->ev_side, 0));
     if (h->want_g_ready && h->ev_g_ready) CUDA_TRY(h, cudaEventRecord(h->ev_g_ready, h->stream));  // every residual row is written
+    if (f.want_hess && h->hs_recv_now) {
+        // the first knot waits for the left neighbour's block: it is assembled in its own launch after every other knot (the
+        // last range), so that the wait never holds up the rest of this shard's Hessian
+        DProb Pa = P;
+        Pa.kc0 = std::max(P.kc0, 1);
+        launch_hessian_assemble(Pa, dZ, sigma, dmu, dhess, h->stream, &h->launches);
+        if (P.kc1 >= P.nK) {
+            launch_hs_receive(h->xwin, h->peer_win[h->link_rank - 1], hs_rows(P, true), P.z, h->hblk_len, h->hseq, h->stream, &h->launches);
+            Pa.kc0 = 0;
+            Pa.kc1 = 1;
+            launch_hessian_assemble(Pa, dZ, sigma, dmu, dhess, h->stream, &h->launches, true);
+        }
+        return DTO_OK;  // knot-range shards have no global variables
+    }
     if (f.want_hess) launch_hessian_assemble(P, dZ, sigma, dmu, dhess, h->stream, &h->launches);
     if (f.want_hess) launch_global_hessian(P, dZ, sigma, dmu, dhess, nullptr, h->stream, &h->launches);
     return DTO_OK;
@@ -1576,7 +1619,23 @@ static int check_eval_args(dto_handle* h, const double* dmu, const double* dhess
         h->err = "Hessian evaluation needs mu";
         return DTO_ERR_INVALID;
     }
+    if (dhess && h->hs_left && h->link_rank < 1) {
+        h->err = "Hessian of a knot-range shard that starts after knot 1 with a linear-spline time-dependent bilinear integrator: "
+                 "its first knot's block needs the left neighbour's last interval, so the shards must be linked "
+                 "(dto_shard_link / dto_shard_link_local)";
+        return DTO_ERR_INVALID;
+    }
     return DTO_OK;
+}
+
+// A Hessian evaluation of a linked shard with a boundary block: its sequence number, and whether it pushes the block to the
+// right neighbour and receives one from the left
+static void begin_hs_exchange(dto_handle* h, bool hess) {
+    h->hs_push_now = h->hs_recv_now = false;
+    if (!hess || h->hblk_len == 0 || h->link_rank < 0) return;
+    h->hs_recv_now = h->hs_left && h->link_rank > 0;
+    h->hs_push_now = h->link_rank + 1 < h->link_world;
+    if (h->hs_recv_now || h->hs_push_now) ++h->hseq;
 }
 
 static int prepare_halo(dto_handle* h);
@@ -1588,6 +1647,7 @@ static int run_eval(dto_handle* h, const double* dZ, double sigma, const double*
     if (rc != DTO_OK) return rc;
     h->g_ready_valid = false;
     if ((rc = prepare_halo(h)) != DTO_OK) return rc;
+    begin_hs_exchange(h, dhess != nullptr);
     const DProb& P = h->P;
     EvalFlags f{dg != nullptr, djac != nullptr, dhess != nullptr};
     // The objective / gradient kernels are independent of the interval kernels and tiny (launch- and latency-bound): they run
@@ -1775,6 +1835,7 @@ static int eval_core(dto_handle* h, double sigma, const EvalFlags* passes, int n
         comp_jac |= passes[i].want_jac;
         comp_hess |= passes[i].want_hess;
     }
+    begin_hs_exchange(h, comp_hess);
     if (spec_jac) jac = h->reg_jac;
     long long d2h = 8LL * B * ((J ? 1 : 0) + (grad ? P.n_grad_local : 0) + (g ? P.n_cons_local : 0));
     double* dJ = comp_obj ? h->dJ : nullptr;
@@ -1983,7 +2044,12 @@ static int eval_core(dto_handle* h, double sigma, const EvalFlags* passes, int n
             // columns of knots [kc0, kc1): their own-interval rows were written by this range, the previous-interval rows
             // of knot kc0 by the range before
             if (jac_now && (rc = deliver_jac(Pr.kc0, Pr.kc1, h->copy_stream)) != DTO_OK) return rc;
-            if (hess_now && (rc = deliver_hess(Pr.kc0, Pr.kc1, h->copy_stream)) != DTO_OK) return rc;
+            if (hess_now && h->hs_recv_now) {  // the first knot is assembled after the last range (eval_range): it leaves last
+                if ((rc = deliver_hess(std::max(Pr.kc0, 1), Pr.kc1, h->copy_stream)) != DTO_OK) return rc;
+                if (Pr.kc1 >= P.nK && (rc = deliver_hess(0, 1, h->copy_stream)) != DTO_OK) return rc;
+            } else if (hess_now && (rc = deliver_hess(Pr.kc0, Pr.kc1, h->copy_stream)) != DTO_OK) {
+                return rc;
+            }
             tr.mark("range-delivered", h->copy_stream);
         }
         CUDA_TRY(h, cudaGetLastError());
@@ -2309,7 +2375,8 @@ extern "C" int dto_violation_dev(dto_handle* h, const double* dg, double* dviol)
 // ---- links between knot-range shards ---------------------------------------------------------------------
 extern "C" double* dto_local_Z(dto_handle* h) { return h ? h->dZ : nullptr; }
 
-static size_t xwin_bytes(const dto_handle* h) { return sizeof(XWin) + sizeof(double) * 2 * (size_t)h->P.z; }
+// the halo slots [2][z], then the boundary Hessian block slots [2][hblk_len]: the same size on every shard of a problem
+static size_t xwin_bytes(const dto_handle* h) { return sizeof(XWin) + sizeof(double) * 2 * ((size_t)h->P.z + (size_t)h->hblk_len); }
 
 static int ensure_xwin(dto_handle* h) {
     if (h->xwin) return DTO_OK;
@@ -2336,7 +2403,7 @@ extern "C" int dto_shard_export(dto_handle* h, void* out64) {
 static int finish_link(dto_handle* h, int rank, int world) {
     h->link_rank = rank;
     h->link_world = world;
-    h->epoch = h->waited_epoch = h->scal_seq = 0;
+    h->epoch = h->waited_epoch = h->scal_seq = h->hseq = 0;
     h->z_valid = false;  // the next callback uploads (and publishes) whatever it is given
     if (!h->d_peer_win) {
         void* p = nullptr;
@@ -2372,6 +2439,9 @@ extern "C" int dto_shard_link(dto_handle* h, int rank, int world, const void* ha
     if (rc != DTO_OK) return rc;
     CUDA_TRY(h, cudaStreamSynchronize(h->stream));
     drop_links(h);  // a second link closes the first mappings
+    // a re-link starts from a clean window: tags left by the previous link would let the first waits pass on stale data
+    // (callers synchronise all ranks after linking, before anyone publishes into this window)
+    CUDA_TRY(h, cudaMemset(h->xwin, 0, xwin_bytes(h)));
     for (int r = 0; r < world; ++r) {
         if (r == rank) {
             h->peer_win[r] = h->xwin;
@@ -2397,6 +2467,7 @@ extern "C" int dto_shard_link_local(dto_handle* const* hs, int world) {
         if (rc != DTO_OK) return rc;
         cudaStreamSynchronize(hs[r]->stream);
         drop_links(hs[r]);
+        CUDA_TRY(hs[r], cudaMemset(hs[r]->xwin, 0, xwin_bytes(hs[r])));  // a re-link starts from a clean window
     }
     for (int r = 0; r < world; ++r) {
         dto_handle* h = hs[r];
@@ -2458,9 +2529,19 @@ static int check_link_errors(dto_handle* h) {
     CUDA_TRY(h, cudaMemcpyAsync(&e, &h->xwin->err, sizeof(e), cudaMemcpyDeviceToHost, h->stream));
     CUDA_TRY(h, cudaStreamSynchronize(h->stream));
     if (e != 0) {
-        h->err = e == 1 ? "shard link: the left neighbour never released the halo slot (timeout)"
-                        : (e == 2 ? "shard link: the right neighbour's knot of this iterate never arrived (timeout); every rank must upload every iterate"
-                                  : "shard link: scalar exchange timed out");
+        switch (e) {
+            case 1: h->err = "shard link: the left neighbour never released the halo slot (timeout)"; break;
+            case 2: h->err = "shard link: the right neighbour's knot of this iterate never arrived (timeout); every rank must upload every iterate"; break;
+            case 3: h->err = "shard link: scalar exchange timed out"; break;
+            case 4:
+                h->err = "shard link: Hessian exchange: the right neighbour never took the previous boundary block (timeout); a linked shard's "
+                         "Hessian evaluation s reads what its left neighbour's evaluation s produced, so every rank evaluates every Hessian";
+                break;
+            default:
+                h->err = "shard link: Hessian exchange: the left neighbour's boundary block of this Hessian evaluation never arrived (timeout); "
+                         "a linked shard's Hessian evaluation s reads what its left neighbour's evaluation s produced, so every rank evaluates "
+                         "every Hessian, and a thread that drives several linked shards calls them in rank order";
+        }
         cudaMemsetAsync(&h->xwin->err, 0, sizeof(e), h->stream);
         return DTO_ERR_CUDA;
     }

@@ -213,14 +213,32 @@ __host__ __device__ inline bool hess_knot_has_cross(const DProb& P, int kl) { re
 struct XWin {
     unsigned long long halo_epoch;  // written by the RIGHT neighbour: halo[epoch & 1] holds its first knot of iterate `epoch`
     unsigned long long ack;         // written by the LEFT neighbour: it no longer reads this shard's knot of iterates <= ack
-    unsigned long long err;         // a wait timed out (1: acknowledgement, 2: halo, 3: scalar exchange)
+    unsigned long long err;         // a wait timed out (1: acknowledgement, 2: halo, 3: scalar exchange, 4: Hessian block
+                                    // acknowledgement, 5: Hessian block)
+    unsigned long long hs_seq;      // written by the LEFT neighbour: hblk slot hs_seq & 1 holds its boundary block of Hessian evaluation hs_seq
+    unsigned long long hs_ack;      // written by the RIGHT neighbour: it has copied this shard's boundary blocks <= hs_ack out of its window
     unsigned long long pad;
     double scal[2][DTO_MAX_RANKS][4];  // [seq & 1][rank] = {objective, violation, seq (as u64), -}
-    double halo[2];                    // really [2][z]: allocated with the window
+    double halo[2];                    // really [2][z], then hblk [2][hblk_len]: allocated with the window
 };
+// The boundary Hessian block of a linked shard (linear-spline time-dependent bilinear integrators): one compact-scratch
+// row per such integrator.  Pushing side: the rows of the last local interval; receiving side: the leading row of DInt::hs.
+struct HsRows {
+    double* row[DTO_MAX_INT];
+    int len[DTO_MAX_INT];
+    int n;
+};
+// hblk slots of a window: they follow the [2][z] halo slots
+__host__ __device__ inline double* xwin_hblk(XWin* w, int z) { return w->halo + 2 * (size_t)z; }
 void launch_shard_publish(XWin* own, XWin* left, XWin* right, double* dst, const double* src, long long n, int z,
                           unsigned long long epoch, bool wait_right, cudaStream_t st, long long* launches);
 void launch_shard_wait(XWin* own, unsigned long long epoch, cudaStream_t st, long long* launches);
+// push this shard's boundary rows into the right neighbour's window (Hessian evaluation `seq`) / wait for the left
+// neighbour's block of `seq`, copy it into the local rows and acknowledge it
+void launch_hs_push(XWin* own, XWin* right, const HsRows& rows, int z, long long hblk_len, unsigned long long seq, cudaStream_t st,
+                    long long* launches);
+void launch_hs_receive(XWin* own, XWin* left, const HsRows& rows, int z, long long hblk_len, unsigned long long seq, cudaStream_t st,
+                       long long* launches);
 void launch_scalar_exchange(XWin* own, XWin* const* peers, int rank, int world, unsigned long long seq, double* J, double* viol,
                             cudaStream_t st, long long* launches);
 
@@ -287,8 +305,10 @@ void launch_tdb(const DProb& P, int ii, const double* Z, const double* mu, doubl
 void launch_analytic(const DProb& P, const double* Z, double* g, double* jac, EvalFlags f, cudaStream_t st, long long* launches);
 void launch_constraints(const DProb& P, const double* Z, double* g, double* jac, EvalFlags f, cudaStream_t st, long long* launches);
 bool launch_knot_objective_pairs(const DProb& P, const double* Z, cudaStream_t st, long long* launches);
+// left_block: a linked shard's first knot (the only knot of the active range, kc0 = 0) also gets the previous interval's
+// share, from the leading row of DInt::hs that launch_hs_receive filled (hessian_assemble_left_kernel)
 void launch_hessian_assemble(const DProb& P, const double* Z, double sigma, const double* mu, double* hess, cudaStream_t st,
-                             long long* launches);
+                             long long* launches, bool left_block = false);
 size_t hessian_assemble_smem_bytes(const DProb& P);  // dynamic shared memory of one assembler block (depends on z, any_cross)
 void launch_objective(const DProb& P, const double* Z, double* J, double* grad, double* partials, cudaStream_t st,
                       long long* launches);

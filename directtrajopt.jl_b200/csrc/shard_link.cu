@@ -8,6 +8,14 @@
 //   * the two scalars every rank needs (objective: sum, constraint violation: max): one kernel writes {J, viol, seq} into
 //     this rank's slot of EVERY peer's window and spins until all slots of its own window carry seq; the sum runs in
 //     rank order on every rank (bit-identical results everywhere).
+//   * the boundary Hessian block (time-dependent bilinear integrators with a linear control spline, whose interval k
+//     reads u_{k+1}): interval k0 - 1 belongs to the left neighbour but adds to the (u, u) entries of knot k0 and to the
+//     whole (knot k0 - 1, knot k0) cross block, which the right shard assembles.  Every Hessian evaluation the left
+//     neighbour PUSHES the compact second-derivative row(s) of its last interval -- computed anyway, identical bits to the
+//     unsharded evaluation -- into slot seq & 1 of the right neighbour's window and publishes seq (hs_push_kernel); the
+//     right shard waits for seq right before it assembles its first knot, copies the block into the leading row of its
+//     scratch and acknowledges (hs_receive_kernel).  seq counts Hessian evaluations since the link, so a linked shard's
+//     Hessian evaluation s reads what its left neighbour's evaluation s produced: every rank evaluates every Hessian.
 // A wait that sees no progress for kTimeoutNs sets XWin::err and gives up (reported by the host as DTO_ERR_CUDA).
 #include "dto_internal.h"
 #include <algorithm>
@@ -86,6 +94,56 @@ __global__ void __launch_bounds__(256) shard_publish_kernel(XWin* own, XWin* lef
 __global__ void shard_wait_kernel(XWin* own, unsigned long long epoch) {
     if (!wait_geq(&own->halo_epoch, epoch)) own->err = 2;
     __threadfence_system();
+}
+
+// Hessian evaluation `seq`, pushing side (enqueued after the interval kernel that wrote the last local interval's rows):
+// wait until the right neighbour has copied block seq - 2 (same slot) out, store this evaluation's rows into slot seq & 1
+// of its window, then publish seq.
+__global__ void __launch_bounds__(256) hs_push_kernel(XWin* own, XWin* right, HsRows rows, int z, long long hblk_len,
+                                                      unsigned long long seq) {
+    __shared__ int ok;
+    if (threadIdx.x == 0) {
+        ok = seq < 3 || wait_geq(&own->hs_ack, seq - 2);
+        if (!ok) own->err = 4;
+    }
+    __syncthreads();
+    if (!ok) return;
+    double* slot = xwin_hblk(right, z) + (size_t)(seq & 1) * hblk_len;
+    for (int r = 0; r < rows.n; ++r) {
+        for (int e = threadIdx.x; e < rows.len[r]; e += blockDim.x) slot[e] = rows.row[r][e];
+        slot += rows.len[r];
+    }
+    __threadfence_system();
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        *(volatile unsigned long long*)&right->hs_seq = seq;
+        __threadfence_system();
+    }
+}
+
+// Hessian evaluation `seq`, receiving side (enqueued before the assembler launch of local knot 0): wait for the left
+// neighbour's block of seq, copy it into the local rows, acknowledge it in the left neighbour's window.
+__global__ void __launch_bounds__(256) hs_receive_kernel(XWin* own, XWin* left, HsRows rows, int z, long long hblk_len,
+                                                         unsigned long long seq) {
+    __shared__ int ok;
+    if (threadIdx.x == 0) {
+        ok = wait_geq(&own->hs_seq, seq);
+        if (!ok) own->err = 5;
+        __threadfence_system();
+    }
+    __syncthreads();
+    if (!ok) return;
+    const volatile double* slot = xwin_hblk(own, z) + (size_t)(seq & 1) * hblk_len;
+    for (int r = 0; r < rows.n; ++r) {
+        for (int e = threadIdx.x; e < rows.len[r]; e += blockDim.x) rows.row[r][e] = slot[e];
+        slot += rows.len[r];
+    }
+    __syncthreads();  // every read of the slot is done before the slot is released
+    if (threadIdx.x == 0) {
+        __threadfence_system();
+        *(volatile unsigned long long*)&left->hs_ack = seq;
+        __threadfence_system();
+    }
 }
 
 // store {J, viol, seq} into this rank's slot of every peer's window, wait for everybody's, reduce in rank order (one warp)
@@ -174,6 +232,18 @@ void launch_shard_publish(XWin* own, XWin* left, XWin* right, double* dst, const
 
 void launch_shard_wait(XWin* own, unsigned long long epoch, cudaStream_t st, long long* launches) {
     shard_wait_kernel<<<1, 1, 0, st>>>(own, epoch);
+    ++*launches;
+}
+
+void launch_hs_push(XWin* own, XWin* right, const HsRows& rows, int z, long long hblk_len, unsigned long long seq, cudaStream_t st,
+                    long long* launches) {
+    hs_push_kernel<<<1, 256, 0, st>>>(own, right, rows, z, hblk_len, seq);
+    ++*launches;
+}
+
+void launch_hs_receive(XWin* own, XWin* left, const HsRows& rows, int z, long long hblk_len, unsigned long long seq, cudaStream_t st,
+                       long long* launches) {
+    hs_receive_kernel<<<1, 256, 0, st>>>(own, left, rows, z, hblk_len, seq);
     ++*launches;
 }
 

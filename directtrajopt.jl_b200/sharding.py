@@ -8,6 +8,11 @@
       evaluation stream: after uploading an iterate a rank pushes its first knot into the left neighbour's exchange
       window (CUDA-IPC mapped HBM) and flags it; the neighbour's kernels wait for the flag on the device
       (csrc/shard_link.cu).  Protocol: every rank calls ``upload`` (or ``upload_dev``) once per iterate.
+      Time-dependent bilinear integrators with ``spline_order = 1`` read u_{k+1} on interval k, so interval k0 - 1
+      of the left neighbour adds to the Hessian of this rank's first knot: every Hessian evaluation, the left neighbour
+      pushes its last interval's compact second derivatives into this rank's window, and this rank assembles its
+      first knot after they arrive (bit-identical to the unsharded Hessian).  Every rank then evaluates every Hessian
+      (evaluation s of a rank reads evaluation s of its left neighbour); an unlinked such shard has no Hessian.
       The two scalars every rank needs -- objective (sum) and constraint violation (max) -- go through the same
       windows (``allreduce_scalars_dev``: one small kernel per rank, no collective library) or, as the
       fallback / in the CPU tests, through ``torch.distributed`` (NCCL on GPUs, gloo on CPU).
@@ -74,6 +79,8 @@ class ShardedEvaluator:
             handles = [None] * world
             dist.all_gather_object(handles, self.local.shard_export())
             self.local.shard_link(rank, world, handles)
+            # linking clears this rank's window: no peer may publish into it before every rank has linked
+            dist.barrier()
             self.peer_halo = True
 
     def local_slice(self, Z):

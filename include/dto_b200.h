@@ -314,12 +314,22 @@ int dto_synchronize(dto_handle* h);
  *     when it moves on, so a rank runs at most one iterate ahead of the neighbour reading its knot.
  *   - dto_allreduce_scalars_dev: objective (sum) and violation (max) of all shards with one kernel per rank that
  *     stores into every peer's window and spins on its own (rank-ordered sum: identical bits on every rank; no NCCL).
+ *   - time-dependent bilinear integrators with spline_order = 1: interval k0 - 1, which the left neighbour owns, adds
+ *     to the Hessian region of this shard's first knot k0 (its (u, u) entries and the whole (k0 - 1, k0) cross block).
+ *     Every Hessian evaluation the left neighbour pushes the compact second derivatives of its last interval into this
+ *     shard's window; this shard assembles its first knot last, after waiting for them.  The reassembled Hessian is
+ *     bit-identical to the unsharded one.
  * Protocol: EVERY rank uploads EVERY iterate exactly once, with dto_upload (host Z slice) or dto_upload_dev (device);
  * callbacks are then called with that same Z (iterate-cache hits) or through the _dev entry points on dto_local_Z.
+ * With a linear-spline time-dependent integrator, a linked shard's Hessian evaluation s (counted from the link, any
+ * entry point) reads what its left neighbour's Hessian evaluation s produced: EVERY rank evaluates EVERY Hessian, and a
+ * thread that drives several linked shards calls them in rank order.  Such a shard that starts after knot 1 and is not
+ * linked has no Hessian (DTO_ERR_INVALID; everything else evaluates).
  * A wait that sees no progress for 20 s fails the evaluation with DTO_ERR_CUDA instead of hanging. */
 /* 64-byte cudaIpcMemHandle_t of this shard's exchange window */
 int dto_shard_export(dto_handle* h, void* ipc_handle_64B);
-/* map the windows of all `world` shards (handles64 = world x 64 bytes in rank order; the own entry is ignored) */
+/* map the windows of all `world` shards (handles64 = world x 64 bytes in rank order; the own entry is ignored).  Linking
+ * (again) clears this shard's window: every rank links before any rank uploads an iterate. */
 int dto_shard_link(dto_handle* h, int rank, int world, const void* handles64);
 /* several shards in ONE process (tests, one-process multi-device drivers): handles in rank order */
 int dto_shard_link_local(dto_handle* const* handles, int world);
