@@ -225,13 +225,14 @@ __global__ void __launch_bounds__(NT == 1 ? 256 : 128, (NT == 1 && M <= 2) ? 2 :
 #pragma unroll
         for (int i = 0; i < M; ++i) u[i] = zk[I.u_off + i];
 
-        // ---- series plan of the row's interval: pre-computed (series_plan.cu), else from ||G(u_r)||_1: the lane sums its
-        // 2 NT columns over all rows, the quad takes the maximum ----
+        // ---- series plan of the row's interval from ||G(u_r)||_1: the lane sums its 2 NT columns over all rows, the quad
+        // takes the maximum ----
         double cmax = 0.0;
-        const bool planned = I.plan != nullptr;
 #pragma unroll
-        for (int t = 0; t < NT && !planned; ++t) {
+        for (int t = 0; t < NT; ++t) {
             double s0 = 0.0, s1 = 0.0;
+            // m = 3: unrolled in full, the loads of this sum make the n = 8 knot-program form spill
+#pragma unroll(M == 3 ? 4 : n)
             for (int s = 0; s < n; ++s) {
                 const double2 g0 = *reinterpret_cast<const double2*>(Gs + s * n + 8 * t + 2 * q);
                 double v0 = g0.x, v1 = g0.y;
@@ -246,7 +247,7 @@ __global__ void __launch_bounds__(NT == 1 ? 256 : 128, (NT == 1 && M <= 2) ? 2 :
             }
             cmax = fmax(cmax, fmax(s0, s1));
         }
-        const Series ser = planned ? choose_series(I.plan[(long long)b * P.nI + kk]) : choose_series(fabs(dt) * quad_max(cmax));
+        const Series ser = choose_series(fabs(dt) * quad_max(cmax));
         const int Tmax = __reduce_max_sync(0xffffffffu, ser.terms), Smax = __reduce_max_sync(0xffffffffu, ser.stages);
         const double cdt = dt * ser.inv_stages;
         const long long mu_off = (long long)b * P.n_cons_local + I.row_off + (long long)kk * n;

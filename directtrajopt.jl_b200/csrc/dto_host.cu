@@ -153,9 +153,8 @@ struct dto_handle {
     std::vector<double> pipeline_fracs;  // cumulative interval fractions of the chunk boundaries (empty = no pipelining)
     std::vector<HRun> hess_runs;         // empty: the Hessian is delivered whole
     std::vector<std::pair<long long, long long>> hess_zero_segs;  // structural-zero prefixes of the knot regions
-    // Jacobian: the previous-interval block of the first integrator is a constant (identity / zero) at the head of every
-    // column of knots 1..nI-1; jac_skip = its length (0: the Jacobian is delivered whole)
-    int jac_skip = 0;
+    // host threads that zero-fill an unregistered Hessian buffer (null: no structural-zero runs, or too few threads to
+    // beat the bus)
     ZeroFill* zero_fill = nullptr;
     std::vector<std::string> variants;
     // optional device timing of the interval kernels (bench.py's roofline numerator)
@@ -167,10 +166,9 @@ struct dto_handle {
     // ---- iterate cache (evaluator.jl:474-482: the reference copies Z once per callback; the solvers call the five
     // callbacks separately on one iterate, ipopt_solver/solver.jl:85).  The handle keeps a page-locked copy of the iterate
     // that is resident on the device; a callback whose Z equals it re-uses the upload and everything already computed.
-    // Early start (DTO_B200_PREFETCH=0 turns it off): the FIRST callback on a new iterate -- the objective or its gradient --
-    // also enqueues the mu-independent pass (residual, Jacobian, jets) and returns as soon as its own small result is on
-    // the host; the interval kernels then run while the solver goes through its next callbacks.
-    int prefetch_mode = 1;
+    // Early start: the FIRST callback on a new iterate -- the objective or its gradient -- also enqueues the mu-independent
+    // pass (residual, Jacobian, jets) and returns as soon as its own small result is on the host; the interval kernels then
+    // run while the solver goes through its next callbacks.
     int prefetch_score = 0;        // < 0: recent early starts were thrown away (the iterate changed before g / J were read): paused
     bool async_inflight = false;   // an early-started pass may still be running on `stream`
     bool prefetch_consumed = false;
@@ -178,7 +176,6 @@ struct dto_handle {
     double* hg_pin = nullptr;        // early start: the residual is staged here ahead of the Jacobian's last block (copy-engine FIFO)
     cudaEvent_t ev_g = nullptr;
     bool g_staged = false;
-    int cache_mode = 1;        // 0: off; 1: one mu-independent pass (g + Jacobian + second-order jets) per new iterate; 2: compute only what is asked
     double* hZpin = nullptr;   // [batch][n_vars_local]
     bool z_valid = false;      // dZ holds hZpin
     bool have_obj = false;     // dJ, dgrad
@@ -192,7 +189,6 @@ struct dto_handle {
     bool reg_jac_pinned = false, reg_hess_pinned = false;  // page lock taken by this handle
     bool reg_jac_sparse = false, reg_hess_sparse = false;  // constants are in place
     int jac_skip_ok = 0;             // length of the constant head of the inner knots' Jacobian columns (0: no common layout)
-    bool fill_threads_ok = false;    // enough host threads to zero-fill an unregistered Hessian buffer faster than PCIe delivers it
     // objective / gradient kernels run beside the interval kernel on a second stream (one SM is left free for them)
     cudaStream_t aux_stream = nullptr;
     cudaEvent_t ev_fork = nullptr, ev_join = nullptr;
@@ -203,7 +199,6 @@ struct dto_handle {
     const double* g_ready_ptr = nullptr;
     const double* j_ready_ptr = nullptr;
     bool g_ready_valid = false, want_g_ready = false;
-    int overlap_objective = 1;       // DTO_B200_OVERLAP=0 keeps everything on one stream
     int trace = 0;                   // DTO_B200_TRACE=1: device timeline of every host-pointer call on stderr
     bool spec_jac_inflight = false;  // a speculative delivery of the Jacobian into reg_jac is on the copy stream
     bool spec_jac_done = false;      // reg_jac holds the resident iterate's Jacobian (once the copy stream has drained)
@@ -464,8 +459,12 @@ extern "C" int dto_create(const dto_problem_desc* d, dto_handle** out) {
     } else {
         cudaGetDevice(&h->device);
     }
-    if (cudaStreamCreateWithFlags(&h->stream, cudaStreamNonBlocking) != cudaSuccess)
+    if (cudaStreamCreateWithFlags(&h->stream, cudaStreamNonBlocking) != cudaSuccess ||
+        cudaStreamCreateWithFlags(&h->aux_stream, cudaStreamNonBlocking) != cudaSuccess ||
+        cudaStreamCreateWithFlags(&h->copy_stream, cudaStreamNonBlocking) != cudaSuccess)
         return fail_create(h, DTO_ERR_CUDA, "cudaStreamCreate failed");
+    for (cudaEvent_t* e : {&h->ev_fork, &h->ev_join, &h->ev_side_fork, &h->ev_side, &h->ev_g_ready, &h->ev_scal_done, &h->ev_small, &h->ev_g})
+        if (cudaEventCreateWithFlags(e, cudaEventDisableTiming) != cudaSuccess) return fail_create(h, DTO_ERR_CUDA, "cudaEventCreate failed");
     // the kernels whose shared memory grows with the shape are checked against it here, so that a shape no kernel can
     // launch is rejected at construction instead of failing at its first evaluation
     int smem_optin = 0;
@@ -685,8 +684,7 @@ extern "C" int dto_create(const dto_problem_desc* d, dto_handle** out) {
         // small-state bilinear kernel + derivative integrators: one kernel writes whole Jacobian columns
         bool any_deriv = false;
         for (int i = 0; i < P.n_int; ++i) any_deriv |= P.in[i].kind == DTO_INT_DERIVATIVE;
-        const char* env = getenv("DTO_B200_FUSE_ANALYTIC");
-        if (any_deriv && !(env && strcmp(env, "0") == 0))
+        if (any_deriv)
             for (int i = 0; i < P.n_int && !P.analytic_fused; ++i)
                 if (P.in[i].kind == DTO_INT_BILINEAR && P.in[i].variant == DTO_VAR_OCTET) P.analytic_fused = i + 1;
     }
@@ -1121,21 +1119,13 @@ extern "C" int dto_create(const dto_problem_desc* d, dto_handle** out) {
     if (!h->dZ || !h->dmu || !h->dg || !h->djac || !h->dgrad || !h->dJ || !h->dpartials || (d->eval_hessian && !h->dhess))
         return fail_create(h, DTO_ERR_ALLOC, "device allocation failed (work buffers)");
     {
-        // iterate cache: DTO_B200_ITERATE_CACHE=0 disables it, =lazy computes only what each callback asks for
+        // iterate cache: the page-locked host copy of the resident iterate
         if (const char* tr = getenv("DTO_B200_TRACE")) h->trace = atoi(tr);
-        if (const char* ov = getenv("DTO_B200_OVERLAP")) h->overlap_objective = atoi(ov);
-        const char* env = getenv("DTO_B200_ITERATE_CACHE");
-        h->cache_mode = env && strcmp(env, "0") == 0 ? 0 : (env && strcmp(env, "lazy") == 0 ? 2 : 1);
-        {
-            const char* pf = getenv("DTO_B200_PREFETCH");
-            h->prefetch_mode = pf && strcmp(pf, "0") == 0 ? 0 : 1;
-        }
-        if (h->cache_mode && cudaHostAlloc((void**)&h->hZpin, sizeof(double) * B * (size_t)P.n_vars_local, cudaHostAllocDefault) != cudaSuccess) {
-            cudaGetLastError();
+        if (cudaHostAlloc((void**)&h->hZpin, sizeof(double) * B * (size_t)P.n_vars_local, cudaHostAllocDefault) != cudaSuccess) {
             h->hZpin = nullptr;
-            h->cache_mode = 0;
+            return fail_create(h, DTO_ERR_ALLOC, "page-locked host allocation failed (iterate cache)");
         }
-        bool ok = d->eval_hessian && h->cache_mode == 1;
+        bool ok = d->eval_hessian;
         bool any = false;
         for (int i = 0; i < P.n_int; ++i) {
             if (P.in[i].kind == DTO_INT_DERIVATIVE) continue;
@@ -1150,7 +1140,7 @@ extern "C" int dto_create(const dto_problem_desc* d, dto_handle** out) {
                 for (int i = 0; i < P.n_int; ++i) {
                     DInt& I = P.in[i];
                     if (I.kind != DTO_INT_BILINEAR || I.variant < DTO_VAR_PERSISTENT) continue;
-                    if (I.variant == DTO_VAR_OCTET && !(sp && strcmp(sp, "all") == 0)) continue;  // n = 8 / 16: see DESIGN.md section 3 (DTO_B200_SERIES_PLAN=all)
+                    if (I.variant == DTO_VAR_OCTET) continue;  // n = 8 / 16: see DESIGN.md section 3
                     const dto_integrator_desc& sd = d->integrators[i];
                     if (sd.G_batch_stride != 0 || series_plan_smem(I.n, I.m) == 0) continue;  // shared sets that fit shared memory
                     std::vector<float> pm;
@@ -1176,45 +1166,28 @@ extern "C" int dto_create(const dto_problem_desc* d, dto_handle** out) {
         }
     }
     {
-        // chunk boundaries of the host-pointer pipeline as cumulative fractions of the intervals; DTO_B200_PIPELINE=0
-        // disables it, DTO_B200_PIPELINE=0.1,0.4,0.7 overrides the plan
-        const char* env = getenv("DTO_B200_PIPELINE");
-        if (!env) {
-            // the persistent interval kernel needs many items per warp to fill the FP64 pipe (one forward item alone takes
-            // ~100 us): two ranges; the octet kernel's items are small: four
-            bool persistent = false;
-            for (int i = 0; i < P.n_int; ++i) persistent |= P.in[i].kind == DTO_INT_BILINEAR && P.in[i].variant == DTO_VAR_PERSISTENT;
-            bool tdbi = false;
-            for (int i = 0; i < P.n_int; ++i) tdbi |= P.in[i].kind == DTO_INT_TDBILINEAR;
-            if (tdbi) {
-                // one CTA per SM works through the intervals of a range in rounds (~1 ms each at n = 64): boundaries at
-                // multiples of two full rounds, so that cutting costs no partial round (c3: 296 / 592 / 888 of 999)
-                int sms = 148;
-                cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, h->device);
-                for (int k = 2 * sms; k + sms / 2 < P.nI; k += 2 * sms) h->pipeline_fracs.push_back((k + 0.5) / (double)std::max(P.nI, 1));
-            } else if (persistent) h->pipeline_fracs = {0.5};
-            else h->pipeline_fracs = {0.1, 0.4, 0.7};
-        }
-        else if (strcmp(env, "0") != 0) {
-            std::string t(env);
-            size_t pos = 0;
-            while (pos < t.size()) {
-                size_t nx = t.find(',', pos);
-                if (nx == std::string::npos) nx = t.size();
-                const double v = atof(t.substr(pos, nx - pos).c_str());
-                if (v > 0.0 && v < 1.0) h->pipeline_fracs.push_back(v);
-                pos = nx + 1;
-            }
-            std::sort(h->pipeline_fracs.begin(), h->pipeline_fracs.end());
-        }
+        // chunk boundaries of the host-pointer pipeline as cumulative fractions of the intervals.  The persistent interval
+        // kernel needs many items per warp to fill the FP64 pipe (one forward item alone takes ~100 us): two ranges; the
+        // octet kernel's items are small: four
+        bool persistent = false;
+        for (int i = 0; i < P.n_int; ++i) persistent |= P.in[i].kind == DTO_INT_BILINEAR && P.in[i].variant == DTO_VAR_PERSISTENT;
+        bool tdbi = false;
+        for (int i = 0; i < P.n_int; ++i) tdbi |= P.in[i].kind == DTO_INT_TDBILINEAR;
+        if (tdbi) {
+            // one CTA per SM works through the intervals of a range in rounds (~1 ms each at n = 64): boundaries at
+            // multiples of two full rounds, so that cutting costs no partial round (c3: 296 / 592 / 888 of 999)
+            int sms = 148;
+            cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, h->device);
+            for (int k = 2 * sms; k + sms / 2 < P.nI; k += 2 * sms) h->pipeline_fracs.push_back((k + 0.5) / (double)std::max(P.nI, 1));
+        } else if (persistent) h->pipeline_fracs = {0.5};
+        else h->pipeline_fracs = {0.1, 0.4, 0.7};
     }
     // ---- structural zeros of the Hessian (host-pointer path) -------------------------------------------------------
     // For bilinear/derivative problems every entry of a knot's region in a column below l0(k) is identically zero
     // (x enters the dynamics linearly: the cross block and the (x, x) block carry no term; SURVEY.md section 8a).
     // l0(k) = smallest column any term of the problem can write at knot k (column of a pair = its larger component).
     {
-        const char* env = getenv("DTO_B200_SPARSE_D2H");
-        bool ok = d->eval_hessian && d->batch == 1 && !P.any_cross && G == 0 && !(env && strcmp(env, "0") == 0);
+        bool ok = d->eval_hessian && d->batch == 1 && !P.any_cross && G == 0;
         for (int i = 0; i < P.n_int; ++i) ok = ok && (P.in[i].kind == DTO_INT_BILINEAR || P.in[i].kind == DTO_INT_DERIVATIVE);
         if (ok) {
             int l_int = z;  // knots that own an interval
@@ -1275,31 +1248,20 @@ extern "C" int dto_create(const dto_problem_desc* d, dto_handle** out) {
                 h->hess_zero_segs.clear();
             } else if (nth >= 3) {  // unregistered buffers need the fill threads; registered ones have their zeros in place
                 h->zero_fill = new (std::nothrow) ZeroFill();
-                if (h->zero_fill) {
-                    h->zero_fill->start(nth);
-                    h->fill_threads_ok = true;
-                }
+                if (h->zero_fill) h->zero_fill->start(nth);
             }
         }
     }
     {
         // Jacobian: d r_{k-1} / d z_k of a bilinear or derivative integrator is the constant [0 .. I .. 0] block
         // (bilinear_integrator.jl:81, derivative_integrator.jl:45: x_{k+1} enters linearly).  With one column layout for
-        // all inner knots (no knot-constraint rows) the rest of every column is one strided copy.
-        const char* env = getenv("DTO_B200_SPARSE_D2H");
+        // all inner knots (no knot-constraint rows) the rest of every column is one strided copy.  Only registered Jacobian
+        // arrays (dto_register_outputs) skip the heads: they get them once; an unregistered buffer would need them written
+        // on every call (74 000 small memsets at c2).
         const int k0i = P.in[0].kind;
         const long long L = 2LL * P.Dsum, d1 = P.in[0].n;
         if (d->batch == 1 && P.jac_closed && G == 0 && P.nI >= 3 && (k0i == DTO_INT_BILINEAR || k0i == DTO_INT_DERIVATIVE) && 8 * (L - d1) >= 256)
-            h->jac_skip_ok = (int)d1;  // registered Jacobian arrays (dto_register_outputs) get the constant heads once
-        if (h->jac_skip_ok && env && strcmp(env, "2") == 0) {  // unregistered buffers: opt-in (74 000 small memsets per call at c2)
-            if (!h->zero_fill) {
-                int nth = 4;
-                if (const char* e2 = getenv("DTO_B200_HOST_THREADS")) nth = std::max(1, std::min(32, atoi(e2)));
-                h->zero_fill = new (std::nothrow) ZeroFill();
-                if (h->zero_fill) h->zero_fill->start(nth);
-            }
-            if (h->zero_fill) h->jac_skip = (int)d1;
-        }
+            h->jac_skip_ok = (int)d1;
     }
     if (cudaStreamSynchronize(h->stream) != cudaSuccess || cudaGetLastError() != cudaSuccess)
         return fail_create(h, DTO_ERR_CUDA, "CUDA failure during construction");
@@ -1493,26 +1455,6 @@ static void eval_prologue(dto_handle* h, const DProb& P, const double* dZ, doubl
     if (dgrad) launch_global_gradient(P, dZ, dgrad, h->stream, &h->launches);
 }
 
-// the second stream (objective / gradient kernels, knot-objective pairs) and its events; false: keep everything on one stream
-static bool ensure_aux(dto_handle* h) {
-    if (!h->overlap_objective) return false;
-    if (h->aux_stream) return true;
-    if (cudaStreamCreateWithFlags(&h->aux_stream, cudaStreamNonBlocking) != cudaSuccess ||
-        cudaEventCreateWithFlags(&h->ev_fork, cudaEventDisableTiming) != cudaSuccess ||
-        cudaEventCreateWithFlags(&h->ev_join, cudaEventDisableTiming) != cudaSuccess ||
-        cudaEventCreateWithFlags(&h->ev_side_fork, cudaEventDisableTiming) != cudaSuccess ||
-        cudaEventCreateWithFlags(&h->ev_side, cudaEventDisableTiming) != cudaSuccess ||
-        cudaEventCreateWithFlags(&h->ev_g_ready, cudaEventDisableTiming) != cudaSuccess ||
-        cudaEventCreateWithFlags(&h->ev_scal_done, cudaEventDisableTiming) != cudaSuccess) {
-        cudaGetLastError();
-        if (h->aux_stream) cudaStreamDestroy(h->aux_stream);
-        h->aux_stream = nullptr;
-        h->overlap_objective = 0;
-        return false;
-    }
-    return true;
-}
-
 // The boundary block's rows, one per linear-spline tdbilinear integrator: the last local interval's (pushed to the right
 // neighbour) or the leading row the left neighbour's block is received into
 static HsRows hs_rows(const DProb& P, bool leading) {
@@ -1535,7 +1477,7 @@ static int eval_range(dto_handle* h, const DProb& P, const double* dZ, double si
     // assembler below waits for them
     bool side_on_aux = false;
     if (f.want_hess && sigma != 0.0 && P.knot_side != nullptr) {
-        if (P.nI >= 256 && ensure_aux(h)) {
+        if (P.nI >= 256) {
             CUDA_TRY(h, cudaEventRecord(h->ev_side_fork, h->stream));
             CUDA_TRY(h, cudaStreamWaitEvent(h->aux_stream, h->ev_side_fork, 0));
             side_on_aux = launch_knot_objective_pairs(P, dZ, h->aux_stream, &h->launches);
@@ -1584,7 +1526,7 @@ static int eval_range(dto_handle* h, const DProb& P, const double* dZ, double si
         }
     }
     if (side_on_aux) CUDA_TRY(h, cudaStreamWaitEvent(h->stream, h->ev_side, 0));
-    if (h->want_g_ready && h->ev_g_ready) CUDA_TRY(h, cudaEventRecord(h->ev_g_ready, h->stream));  // every residual row is written
+    if (h->want_g_ready) CUDA_TRY(h, cudaEventRecord(h->ev_g_ready, h->stream));  // every residual row is written
     if (f.want_hess && h->hs_recv_now) {
         // the first knot waits for the left neighbour's block: it is assembled in its own launch after every other knot (the
         // last range), so that the wait never holds up the rest of this shard's Hessian
@@ -1653,8 +1595,7 @@ static int run_eval(dto_handle* h, const double* dZ, double sigma, const double*
     // The objective / gradient kernels are independent of the interval kernels and tiny (launch- and latency-bound): they run
     // on a second stream BESIDE the interval kernel, which leaves one SM free for them (0.7 % of its throughput against
     // ~17 us of serial kernels at c2).
-    bool overlap = h->overlap_objective && (dJ || dgrad) && (f.want_g || f.want_jac || f.want_hess) && P.nI >= 256;
-    if (overlap && !ensure_aux(h)) overlap = false;
+    const bool overlap = (dJ || dgrad) && (f.want_g || f.want_jac || f.want_hess) && P.nI >= 256;
     if (overlap) {
         // forked BEFORE the series plans: the objective kernels then run beside the plan kernel and are gone when the
         // interval kernel wants its SMs (forked after it, they raced the interval kernel for them: up to 10 us)
@@ -1724,7 +1665,7 @@ static int publish_iterate(dto_handle* h, const double* src);
 static int ensure_iterate(dto_handle* h, const double* Z, bool force = false) {
     const DProb& P = h->P;
     const size_t bytes = sizeof(double) * (size_t)P.batch * (size_t)P.n_vars_local;
-    if (!force && h->cache_mode && h->z_valid && memcmp(h->hZpin, Z, bytes) == 0) {
+    if (!force && h->z_valid && memcmp(h->hZpin, Z, bytes) == 0) {
         ++h->cache_hits;
         return 1;
     }
@@ -1739,13 +1680,9 @@ static int ensure_iterate(dto_handle* h, const double* Z, bool force = false) {
         CUDA_TRY(h, cudaStreamSynchronize(h->copy_stream));
         h->spec_jac_inflight = false;
     }
-    if (h->cache_mode) {
-        memcpy(h->hZpin, Z, bytes);
-        CUDA_TRY(h, cudaMemcpyAsync(h->dZ, h->hZpin, bytes, cudaMemcpyHostToDevice, h->stream));
-        h->z_valid = true;
-    } else {
-        CUDA_TRY(h, cudaMemcpyAsync(h->dZ, Z, bytes, cudaMemcpyHostToDevice, h->stream));
-    }
+    memcpy(h->hZpin, Z, bytes);
+    CUDA_TRY(h, cudaMemcpyAsync(h->dZ, h->hZpin, bytes, cudaMemcpyHostToDevice, h->stream));
+    h->z_valid = true;
     const int rc = publish_iterate(h, h->dZ);
     return rc < 0 ? rc : 0;
 }
@@ -1841,17 +1778,15 @@ static int eval_core(dto_handle* h, double sigma, const EvalFlags* passes, int n
     double* dJ = comp_obj ? h->dJ : nullptr;
     double* dgrad = comp_obj ? h->dgrad : nullptr;
     EvalFlags fany{comp_g, comp_jac, comp_hess};
-    if (!h->copy_stream) CUDA_TRY(h, cudaStreamCreateWithFlags(&h->copy_stream, cudaStreamNonBlocking));
 
     // Structural constants stay off the bus: a registered array has them in place (written once by dto_register_outputs);
     // an unregistered Hessian buffer gets them from the handle's host threads while the GPU computes.
     const bool reg_h = hess && hess == h->reg_hess && h->reg_hess_sparse;
     const bool reg_j = jac && jac == h->reg_jac && h->reg_jac_sparse;
     const bool big = 8LL * ((jac ? P.nnz_jac_local : 0) + (hess ? P.nnz_hess_local : 0)) >= (8LL << 20) && P.nI >= 512;
-    const bool sparse_hess = hess && big && !h->hess_runs.empty() && (reg_h || (h->fill_threads_ok && range_capable(h)));
-    const bool sparse_jac = jac && big && ((reg_j && h->jac_skip_ok > 0) || (h->jac_skip > 0 && h->zero_fill && range_capable(h)));
-    const int jskip = sparse_jac ? (reg_j ? h->jac_skip_ok : h->jac_skip) : 0;
-    const bool fill_h = sparse_hess && !reg_h, fill_j = sparse_jac && !reg_j;
+    const bool sparse_hess = hess && big && !h->hess_runs.empty() && (reg_h || (h->zero_fill && range_capable(h)));
+    const bool sparse_jac = jac && big && reg_j && h->jac_skip_ok > 0;
+    const bool fill_h = sparse_hess && !reg_h;
 
     // Jacobian columns / Hessian regions of the local knots [ka, kb) on stream `st`
     auto deliver_jac = [&](int ka, int kb, cudaStream_t st) -> int {
@@ -1869,7 +1804,7 @@ static int eval_core(dto_handle* h, double sigma, const EvalFlags* passes, int n
         if (rc != DTO_OK) return rc;
         const int a = std::max(ka, 1), b2 = std::min(kb, P.nI);
         if (a < b2) {
-            const long long Lc = 2LL * P.Dsum, sk = jskip;
+            const long long Lc = 2LL * P.Dsum, sk = h->jac_skip_ok;
             const long long p0 = h->jac_colptr[(size_t)a * P.z] + sk;
             CUDA_TRY(h, cudaMemcpy2DAsync(jac + p0, sizeof(double) * Lc, h->djac + p0, sizeof(double) * Lc, sizeof(double) * (Lc - sk),
                                           (size_t)(b2 - a) * P.z, cudaMemcpyDeviceToHost, st));
@@ -1911,7 +1846,6 @@ static int eval_core(dto_handle* h, double sigma, const EvalFlags* passes, int n
             h->hg_pin = nullptr;
             return DTO_OK;  // no staging: the constraint callback copies from the device
         }
-        if (!h->ev_g) CUDA_TRY(h, cudaEventCreateWithFlags(&h->ev_g, cudaEventDisableTiming));
         CUDA_TRY(h, cudaMemcpyAsync(h->hg_pin, h->dg, sizeof(double) * P.n_cons_local, cudaMemcpyDeviceToHost, h->stream));
         CUDA_TRY(h, cudaEventRecord(h->ev_g, h->stream));
         d2h += 8LL * P.n_cons_local;
@@ -1924,29 +1858,14 @@ static int eval_core(dto_handle* h, double sigma, const EvalFlags* passes, int n
     // series plans of this iterate (a Hessian pass from stored jets re-uses the plans of the pass that stored them)
     if ((comp_g || comp_jac || comp_hess) && !(n_passes == 1 && passes[0].jets == DTO_JETS_USE)) launch_plans(h, P, h->dZ);
     FillGuard guard;
-    if (fill_h || fill_j) {
-        // host threads write the structural constants into the caller's buffers while the GPU computes
+    if (fill_h) {
+        // host threads write the structural zeros into the caller's Hessian buffer while the GPU computes
         const dto_handle* hh = h;
-        double* hz = fill_h ? hess : nullptr;
-        double* jz = fill_j ? jac : nullptr;
-        h->zero_fill->launch([hh, hz, jz](int part, int parts) {
-            const DProb& Q = hh->P;
-            if (hz) {
-                const size_t n = hh->hess_zero_segs.size(), lo = n * part / parts, hi = n * (part + 1) / parts;
-                for (size_t i = lo; i < hi; ++i)
-                    memset(hz + hh->hess_zero_segs[i].first, 0, sizeof(double) * (size_t)hh->hess_zero_segs[i].second);
-            }
-            if (jz) {
-                // head of every column of knots 1..nI-1: [0 .. 1 (row l - x_off) .. 0]
-                const long long nk = Q.nI - 1, k_lo = 1 + nk * part / parts, k_hi = 1 + nk * (part + 1) / parts;
-                const int d1 = hh->jac_skip, xo = Q.in[0].x_off;
-                for (long long kl = k_lo; kl < k_hi; ++kl)
-                    for (int l = 0; l < Q.z; ++l) {
-                        double* c = jz + hh->jac_colptr[(size_t)kl * Q.z + l];
-                        memset(c, 0, sizeof(double) * (size_t)d1);
-                        if (l >= xo && l < xo + d1) c[l - xo] = 1.0;
-                    }
-            }
+        double* hz = hess;
+        h->zero_fill->launch([hh, hz](int part, int parts) {
+            const size_t n = hh->hess_zero_segs.size(), lo = n * part / parts, hi = n * (part + 1) / parts;
+            for (size_t i = lo; i < hi; ++i)
+                memset(hz + hh->hess_zero_segs[i].first, 0, sizeof(double) * (size_t)hh->hess_zero_segs[i].second);
         });
         guard.z = h->zero_fill;  // joined on every exit path below
     }
@@ -1974,7 +1893,6 @@ static int eval_core(dto_handle* h, double sigma, const EvalFlags* passes, int n
         eval_prologue(h, P, h->dZ, dJ, dgrad, nullptr, nullptr, EvalFlags{false, false, false});
         if (J) CUDA_TRY(h, cudaMemcpyAsync(J, h->dJ, sizeof(double) * B, cudaMemcpyDeviceToHost, h->stream));
         if (grad) CUDA_TRY(h, cudaMemcpyAsync(grad, h->dgrad, sizeof(double) * B * P.n_grad_local, cudaMemcpyDeviceToHost, h->stream));
-        if (!h->ev_small) CUDA_TRY(h, cudaEventCreateWithFlags(&h->ev_small, cudaEventDisableTiming));
         CUDA_TRY(h, cudaEventRecord(h->ev_small, h->stream));
         J = grad = nullptr;
         dJ = dgrad = nullptr;
@@ -2098,9 +2016,9 @@ extern "C" int dto_eval_all(dto_handle* h, const double* Z, double sigma, const 
     EvalFlags f{g != nullptr, jac != nullptr, hess != nullptr};
     rc = eval_core(h, sigma, &f, 1, J || grad, J, grad, g, jac, hess);
     if (rc == DTO_OK) {
-        h->have_obj = h->z_valid && (J || grad);
-        h->have_g = h->z_valid && g;
-        h->have_jac = h->z_valid && jac;
+        h->have_obj = J || grad;
+        h->have_g = g;
+        h->have_jac = jac;
     }
     return rc;
 }
@@ -2117,11 +2035,6 @@ static int eval_callback(dto_handle* h, const double* Z, double sigma, const dou
     if (rc != DTO_OK) return rc;
     CUDA_TRY(h, cudaSetDevice(h->device));
     if ((rc = ensure_iterate(h, Z)) < 0) return rc;
-    if (!h->z_valid) {  // cache off: every callback is its own pass
-        if (hess) CUDA_TRY(h, cudaMemcpyAsync(h->dmu, mu, sizeof(double) * (size_t)P.batch * P.n_cons_local, cudaMemcpyHostToDevice, h->stream));
-        EvalFlags f{g != nullptr, jac != nullptr, hess != nullptr};
-        return eval_core(h, sigma, &f, 1, J || grad, J, grad, g, jac, hess);
-    }
     if (jac && jac == h->reg_jac && h->have_jac && h->spec_jac_done && !J && !grad && !g && !hess) {
         // the Jacobian of this iterate went to the registered array while the constraint callback computed it
         h->prefetch_consumed = true;
@@ -2132,19 +2045,16 @@ static int eval_callback(dto_handle* h, const double* Z, double sigma, const dou
         h->last_d2h_bytes = 0;
         return DTO_OK;
     }
-    const bool eager = h->cache_mode == 1;
     const bool only_small = (J || grad) && !g && !jac && !hess;
     if (only_small && h->have_obj && h->async_inflight) {
         // resident objective / gradient while an early-started pass still runs on the main stream: a side stream ordered
         // after the objective kernels only
-        if (ensure_aux(h) && h->ev_small) {
-            CUDA_TRY(h, cudaStreamWaitEvent(h->aux_stream, h->ev_small, 0));
-            if (J) CUDA_TRY(h, cudaMemcpyAsync(J, h->dJ, sizeof(double) * P.batch, cudaMemcpyDeviceToHost, h->aux_stream));
-            if (grad) CUDA_TRY(h, cudaMemcpyAsync(grad, h->dgrad, sizeof(double) * (size_t)P.batch * P.n_grad_local, cudaMemcpyDeviceToHost, h->aux_stream));
-            CUDA_TRY(h, cudaStreamSynchronize(h->aux_stream));
-            h->last_d2h_bytes = 8LL * P.batch * ((J ? 1 : 0) + (grad ? P.n_grad_local : 0));
-            return DTO_OK;
-        }
+        CUDA_TRY(h, cudaStreamWaitEvent(h->aux_stream, h->ev_small, 0));
+        if (J) CUDA_TRY(h, cudaMemcpyAsync(J, h->dJ, sizeof(double) * P.batch, cudaMemcpyDeviceToHost, h->aux_stream));
+        if (grad) CUDA_TRY(h, cudaMemcpyAsync(grad, h->dgrad, sizeof(double) * (size_t)P.batch * P.n_grad_local, cudaMemcpyDeviceToHost, h->aux_stream));
+        CUDA_TRY(h, cudaStreamSynchronize(h->aux_stream));
+        h->last_d2h_bytes = 8LL * P.batch * ((J ? 1 : 0) + (grad ? P.n_grad_local : 0));
+        return DTO_OK;
     }
     if (g && !J && !grad && !jac && !hess && h->have_g && h->g_staged) {
         // the residual of this iterate was staged by the early-started pass
@@ -2165,18 +2075,15 @@ static int eval_callback(dto_handle* h, const double* Z, double sigma, const dou
     int np = 0;
     const bool comp_obj = (J || grad) && !h->have_obj;
     // early start: the first callback on a new iterate asks for the objective or its gradient only
-    const bool prefetch = h->prefetch_mode && eager && only_small && comp_obj && !h->have_g && !h->have_jac && P.batch == 1 &&
-                          h->link_rank < 0 && h->prefetch_score >= 0 && P.nI >= 256 && h->jets_ok;
+    const bool prefetch = only_small && comp_obj && !h->have_g && !h->have_jac && P.batch == 1 && h->link_rank < 0 &&
+                          h->prefetch_score >= 0 && P.nI >= 256 && h->jets_ok;
     const bool use_jets = hess && h->jets_ok;
-    bool need_g = g && !h->have_g, need_jac = jac && !h->have_jac;
+    const bool need_g = g && !h->have_g, need_jac = jac && !h->have_jac;
     const bool need_jets = use_jets && !h->have_jets;
     if (need_g || need_jac || need_jets || prefetch) {
-        EvalFlags f1{need_g, need_jac, false};
-        if (prefetch) need_g = need_jac = true;
-        if (eager || need_jets || prefetch) {
-            f1.want_g = f1.want_jac = true;
-            f1.jets = h->jets_ok ? DTO_JETS_STORE : DTO_JETS_NONE;
-        }
+        // the one mu-independent pass of this iterate: residual + Jacobian (+ the jets the Hessian callback uses)
+        EvalFlags f1{true, true, false};
+        f1.jets = h->jets_ok ? DTO_JETS_STORE : DTO_JETS_NONE;
         passes[np++] = f1;
     }
     if (hess) {
@@ -2348,7 +2255,7 @@ static int jac_product(dto_handle* h, const double* Z, const double* w, double* 
         if (!h->have_jac) {
             int rc = run_eval(h, h->dZ, 0.0, nullptr, nullptr, nullptr, nullptr, h->djac, nullptr);
             if (rc != DTO_OK) return rc;
-            h->have_jac = h->z_valid;
+            h->have_jac = true;
         }
         launch_jac_product(P, h->djac, h->d_rows0, h->d_cols0, h->dw, h->dy, transpose, h->stream, &h->launches);
     }
@@ -2580,7 +2487,7 @@ extern "C" int dto_shard_scalars_dev(dto_handle* h, const double* dg, double* dJ
     // its Hessian assembler starts: the reduction and the exchange then run BESIDE the assembler, and the wait for the
     // slowest rank hides behind it.
     cudaStream_t st = h->stream;
-    const bool beside = h->g_ready_valid && dg == h->g_ready_ptr && dJ == h->j_ready_ptr && h->aux_stream && h->ev_g_ready;
+    const bool beside = h->g_ready_valid && dg == h->g_ready_ptr && dJ == h->j_ready_ptr;
     if (beside) {
         CUDA_TRY(h, cudaStreamWaitEvent(h->aux_stream, h->ev_g_ready, 0));
         st = h->aux_stream;

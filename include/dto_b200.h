@@ -35,8 +35,8 @@
  *     finished knot ranges overlap the remaining computation.  For bilinear/derivative problems the structural
  *     zeros of the Hessian (the cross-knot block and every column below the first one a term can touch) do not
  *     cross PCIe: a few host threads of the handle write them into the caller's buffer meanwhile
- *     (DTO_B200_HOST_THREADS, default 4; DTO_B200_SPARSE_D2H=0 delivers the whole array, =2 also leaves the constant
- *     identity/zero head of every Jacobian column to the host threads).  `_dev` entry points take device pointers
+ *     (DTO_B200_HOST_THREADS, default 4; the constant identity/zero head of the Jacobian columns is skipped only for
+ *     arrays given to dto_register_outputs).  `_dev` entry points take device pointers
  *     valid on the handle's device and enqueue on the handle's stream (dto_stream) without synchronising.
  *   - return value: 0 on success, negative dto_status otherwise; no exception crosses the boundary.
  *     dto_last_error() gives the message.  A handle is not thread-safe (matches the reference, whose
@@ -279,10 +279,9 @@ int dto_eval_all(dto_handle* h, const double* Z, double sigma, const double* mu,
  * interval kernels run while the solver goes through its next callbacks, which then wait only for what they deliver
  * (the residual is staged in page-locked memory, the Jacobian goes to a registered array on the side).  Every output is
  * valid when its own callback returns; iterates that are dropped after the objective alone (line searches) pause the
- * early start.  DTO_B200_PREFETCH=0 turns it off.
- * Results are bit-identical to dto_eval_all.  DTO_B200_ITERATE_CACHE=0 disables the cache, =lazy computes only what each
- * callback asks for.  dto_upload makes Z the resident iterate without evaluating anything (and returns after the
- * copy has completed: on knot-range shards, the point after which a neighbour may read this rank's knots). */
+ * early start.  Results are bit-identical to dto_eval_all.  dto_upload makes Z the resident iterate without evaluating
+ * anything (and returns after the copy has completed: on knot-range shards, the point after which a neighbour may read
+ * this rank's knots). */
 int dto_upload(dto_handle* h, const double* Z);
 int dto_cache_stats(const dto_handle* h, int64_t* hits, int64_t* misses);
 /* Optional: tell the handle where the solver keeps its Jacobian / Hessian value arrays (either may be NULL; batch == 1).

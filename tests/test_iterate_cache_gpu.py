@@ -89,24 +89,6 @@ def test_interval_kernel_runs_once_per_iterate():
     ev.close()
 
 
-@pytest.mark.parametrize("mode", ["0", "lazy"])
-def test_cache_modes_agree(monkeypatch, mode):
-    prob = pt.quantum_gate_problem(N=30, levels=16, n_drives=4)
-    Z = prob.trajectory.vec()
-    ev = dto.Evaluator(prob)
-    mu = np.random.default_rng(1).random(ev.n_constraints)
-    ref = _five_calls(ev, Z, 0.9, mu)
-    ev.close()
-    monkeypatch.setenv("DTO_B200_ITERATE_CACHE", mode)
-    ev = dto.Evaluator(prob)
-    got = _five_calls(ev, Z, 0.9, mu)
-    if mode == "0":
-        assert ev.cache_stats() == (0, 5)
-    for a, b in zip(ref, got):
-        assert np.array_equal(np.asarray(a), np.asarray(b))
-    ev.close()
-
-
 @pytest.mark.parametrize("name", ["gate_n32_pipelined", "scaled_n16_octet_long", "gate_n32_persistent"])
 def test_registered_outputs(name):
     """dto_register_outputs: structural constants written once, value-dependent entries per call; speculative delivery of
@@ -166,14 +148,20 @@ def test_eval_all_rejects_bad_buffers():
     ev.close()
 
 
-def test_early_start_of_the_mu_independent_pass(monkeypatch):
+def _objective(ev, Z):
+    """Objective and gradient alone from the fused call."""
+    J, grad = np.empty(1), np.empty(ev.n_vars)
+    ev.eval_all(Z, 1.0, None, J, grad)
+    return J[0], grad
+
+
+def test_early_start_of_the_mu_independent_pass():
     """The first callback on a new iterate (objective or gradient) also starts the residual / Jacobian / jets pass and
-    returns without waiting for it (DTO_B200_PREFETCH=0 turns that off).  Whatever order the callbacks then come in --
-    including iterates that are dropped after the objective alone -- the outputs are those of the plain path, bit for bit."""
+    returns without waiting for it.  Whatever order the callbacks then come in -- including iterates that are dropped
+    after the objective alone -- the outputs are those of the fused call on a second handle (which never starts early),
+    bit for bit."""
     prob = pt.quantum_gate_problem(N=300, levels=16, n_drives=4)
-    monkeypatch.setenv("DTO_B200_PREFETCH", "0")
     ev_ref = dto.Evaluator(prob)
-    monkeypatch.delenv("DTO_B200_PREFETCH")
     ev = dto.Evaluator(prob)
     jac_reg, hess_reg = np.full(ev.nnz_jacobian, np.nan), np.full(ev.nnz_hessian, np.nan)
     rng = np.random.default_rng(11)
@@ -185,29 +173,29 @@ def test_early_start_of_the_mu_independent_pass(monkeypatch):
             ev.register_outputs(jac_reg, hess_reg)
         # A: the solver's order
         Z, mu = new(), rng.random(ev.n_constraints)
-        ref = _five_calls(ev_ref, Z, 1.2, mu)
+        ref = _fused(ev_ref, Z, 1.2, mu)
         got = _five_calls(ev, Z, 1.2, mu)
         for a, b in zip(ref, got):
             assert np.array_equal(np.asarray(a), np.asarray(b))
         # B: line-search style -- objective / gradient alone on iterates that are then dropped, then a full sequence
         for _ in range(3):
             Zt = new()
-            grad_r, grad_g = buf(ev.n_vars), buf(ev.n_vars)
-            assert ev.eval_objective(Zt) == ev_ref.eval_objective(Zt)
+            J_r, grad_r = _objective(ev_ref, Zt)
+            grad_g = buf(ev.n_vars)
+            assert ev.eval_objective(Zt) == J_r
             ev.eval_objective_gradient(grad_g, Zt)
-            ev_ref.eval_objective_gradient(grad_r, Zt)
             assert np.array_equal(grad_g, grad_r)
         for _ in range(6):  # the early start pauses after unused ones and comes back once the pass is asked for again
             Z, mu = new(), rng.random(ev.n_constraints)
-            for a, b in zip(_five_calls(ev_ref, Z, 0.7, mu), _five_calls(ev, Z, 0.7, mu)):
+            for a, b in zip(_fused(ev_ref, Z, 0.7, mu), _five_calls(ev, Z, 0.7, mu)):
                 assert np.array_equal(np.asarray(a), np.asarray(b))
         # C: objective twice, then the Hessian straight away (its jets come from the early-started pass)
         Z, mu = new(), rng.random(ev.n_constraints)
-        assert ev.eval_objective(Z) == ev.eval_objective(Z) == ev_ref.eval_objective(Z)
-        Hg, Hr = buf(ev.nnz_hessian), buf(ev.nnz_hessian)
+        ref = _fused(ev_ref, Z, 1.0, mu)
+        assert ev.eval_objective(Z) == ev.eval_objective(Z) == ref[0]
+        Hg = buf(ev.nnz_hessian)
         ev.eval_hessian_lagrangian(Hg, Z, 1.0, mu)
-        ev_ref.eval_hessian_lagrangian(Hr, Z, 1.0, mu)
-        assert np.array_equal(Hg, Hr)
+        assert np.array_equal(Hg, ref[4])
         # D: objective, then the fused call on the same iterate
         Z, mu = new(), rng.random(ev.n_constraints)
         ev.eval_objective(Z)
@@ -215,16 +203,14 @@ def test_early_start_of_the_mu_independent_pass(monkeypatch):
             assert np.array_equal(np.asarray(a), np.asarray(b))
         # E: gradient first, then the Jacobian into an unregistered buffer, then the residual
         Z = new()
-        gr, gg = buf(ev.n_vars), buf(ev.n_vars)
+        ref = _fused(ev_ref, Z, 1.0, rng.random(ev.n_constraints))
+        gg = buf(ev.n_vars)
         ev.eval_objective_gradient(gg, Z)
-        ev_ref.eval_objective_gradient(gr, Z)
-        jg, jr = buf(ev.nnz_jacobian), buf(ev.nnz_jacobian)
+        jg = buf(ev.nnz_jacobian)
         ev.eval_constraint_jacobian(jg, Z)
-        ev_ref.eval_constraint_jacobian(jr, Z)
-        cg, cr = buf(ev.n_constraints), buf(ev.n_constraints)
+        cg = buf(ev.n_constraints)
         ev.eval_constraint(cg, Z)
-        ev_ref.eval_constraint(cr, Z)
-        assert np.array_equal(gg, gr) and np.array_equal(jg, jr) and np.array_equal(cg, cr)
+        assert np.array_equal(gg, ref[1]) and np.array_equal(jg, ref[3]) and np.array_equal(cg, ref[2])
     ev.unregister_outputs()
     ev.close()
     ev_ref.close()

@@ -290,11 +290,9 @@ def test_knot_range_shards_reassemble_the_whole_problem(peer_halo):
 
 
 # ---- host-pointer callbacks ---------------------------------------------------------------------------------------------
-@pytest.mark.parametrize("cache", ["1", "0", "lazy"])
-def test_callbacks_equal_eval_all(cache, monkeypatch):
+def test_callbacks_equal_eval_all():
     """the five callbacks in the order Ipopt calls them (objective first: early start on a new iterate) against one fused
     pass on another handle, bit for bit; Jacobian products against the materialised Jacobian"""
-    monkeypatch.setenv("DTO_B200_ITERATE_CACHE", cache)
     prob = _shard_problem()
     ev, ref = dto.Evaluator(prob), dto.Evaluator(prob)
     rng = np.random.default_rng(6)

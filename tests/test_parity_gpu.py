@@ -504,58 +504,77 @@ def test_series_plan_matches_norm_based_series(monkeypatch):
             assert relerr(a, b) <= 1e-13
 
 
-def test_host_pipeline_matches_single_pass(monkeypatch):
+def _eval_dev(ev, Z, sigma, mu):
+    """dto_eval_all_dev into device buffers, read back with torch: one pass over the whole trajectory, never cut into
+    knot ranges"""
+    import torch
+
+    dev = torch.device("cuda", torch.cuda.current_device())
+    dZ, dmu = torch.from_numpy(np.ascontiguousarray(Z)).to(dev), torch.from_numpy(np.ascontiguousarray(mu)).to(dev)
+    outs = [torch.full((n,), float("nan"), dtype=torch.float64, device=dev)
+            for n in (1, ev.n_vars, ev.n_constraints, ev.nnz_jacobian, ev.nnz_hessian)]
+    torch.cuda.synchronize()
+    ev.eval_all_dev(dZ.data_ptr(), sigma, dmu.data_ptr(), *[o.data_ptr() for o in outs])
+    ev.synchronize()
+    return [o.cpu().numpy() for o in outs]
+
+
+def test_host_pipeline_matches_single_pass():
     """dto_eval_all with host buffers cuts large problems into knot ranges whose Jacobian columns and Hessian
     blocks leave over PCIe while later ranges are computed; the result must be bit-identical to the
-    single-pass evaluation, whatever the chunk plan (and with knot constraints + a derivative integrator)."""
-    prob = pt.scaled_problem(N=700, state_dim=32, n_controls=2, generator_scale=0.3)
-    Z = prob.trajectory.vec()
-    outs = {}
-    for plan in ("0", "0.12,0.55", "0.05,0.2,0.5,0.9"):
-        monkeypatch.setenv("DTO_B200_PIPELINE", plan)
+    single-pass device-pointer evaluation (also with knot constraints and derivative integrators), for every
+    interval kernel with its own cut plan."""
+    cases = [  # (kernel variant, problem, knot ranges of the host-pointer call)
+        ("persistent", pt.scaled_problem(N=700, state_dim=32, n_controls=2, generator_scale=0.3), 2),
+        ("octet", pt.scaled_problem(N=1000, state_dim=16, n_controls=2, generator_scale=0.25), 4),
+        # 599 intervals: one cut at two rounds of one CTA per SM (296 on a 148-SM B200)
+        ("gbs-dmma", pt.carrier_problem(N=600, state_dim=64, n_drives=2), 2),
+    ]
+    for variant, prob, ranges in cases:
+        Z = prob.trajectory.vec()
         ev = dto.Evaluator(prob)
+        assert ev.kernel_variant(0) == variant
         mu = np.random.default_rng(5).random(ev.n_constraints)
+        ref = _eval_dev(ev, Z, 1.7, mu)
         bufs = [np.full(1, np.nan), np.full(ev.n_vars, np.nan), np.full(ev.n_constraints, np.nan),
                 np.full(ev.nnz_jacobian, np.nan), np.full(ev.nnz_hessian, np.nan)]
+        assert 8 * (ev.nnz_jacobian + ev.nnz_hessian) >= 8 << 20, variant
+        ev.kernel_timing(True)
         ev.eval_all(Z, 1.7, mu, *bufs)
-        assert all(np.isfinite(b).all() for b in bufs), plan
-        outs[plan] = bufs
+        _, launches = ev.kernel_time_ms()  # one per knot range (one interval kernel per range)
+        ev.kernel_timing(False)
+        assert launches == ranges, variant
+        assert all(np.isfinite(b).all() for b in bufs), variant
+        for a, b in zip(ref, bufs):
+            assert np.array_equal(a, b), variant
         ev.close()
-    ref = outs["0"]
-    for plan, got in outs.items():
-        for a, b in zip(ref, got):
-            assert np.array_equal(np.asarray(a), np.asarray(b)), plan
 
 
-def test_structural_zero_hessian_delivery(monkeypatch):
+def test_structural_zero_hessian_delivery():
     """Host-pointer path of bilinear/derivative problems: only the Hessian columns a term can touch cross PCIe (one 2-D
     copy per run of equal knots), host threads write the structural zeros of the caller's buffer meanwhile.  Must be
-    bit-identical to delivering the whole array, including knots where an objective reaches into the x block."""
+    bit-identical to the whole array of the device-pointer evaluation, including knots where an objective reaches into
+    the x block."""
     prob = pt.quantum_gate_problem(N=640, levels=16, n_drives=4)
     t = prob.trajectory
     J = prob.objective + dto.KnotPointObjective(dto.SqDist(np.linspace(-1, 1, 32)), "x", t, times=[5, 6, 300], Qs=[1.0, 2.0, 3.0])
     prob2 = dto.DirectTrajOptProblem(t, J, prob.integrators)
     for pr in (prob, prob2, pt.scaled_problem(N=700, state_dim=32, n_controls=2, generator_scale=0.3)):
         Z = pr.trajectory.vec()
-        outs = {}
-        for mode in ("1", "0", "2"):  # 2: also the constant heads of the Jacobian columns (opt-in)
-            monkeypatch.setenv("DTO_B200_SPARSE_D2H", mode)
-            ev = dto.Evaluator(pr)
-            mu = np.random.default_rng(5).random(ev.n_constraints)
-            for rep in range(2):  # the second call reuses the handle's worker threads
-                bufs = [np.full(1, np.nan), np.full(ev.n_vars, np.nan), np.full(ev.n_constraints, np.nan),
-                        np.full(ev.nnz_jacobian, np.nan), np.full(ev.nnz_hessian, np.nan)]
-                ev.eval_all(Z, 1.7, mu, *bufs)
-                assert all(np.isfinite(b).all() for b in bufs), mode
-            H = np.full(ev.nnz_hessian, np.nan)
-            ev.eval_hessian_lagrangian(H, Z, 1.7, mu)
-            assert np.array_equal(H, bufs[4])
-            outs[mode] = bufs
-            ev.close()
-        for mode in ("1", "2"):
-            for a, b in zip(outs[mode], outs["0"]):
-                assert np.array_equal(a, b)
-
+        ev = dto.Evaluator(pr)
+        mu = np.random.default_rng(5).random(ev.n_constraints)
+        ref = _eval_dev(ev, Z, 1.7, mu)
+        for rep in range(2):  # the second call reuses the handle's worker threads
+            bufs = [np.full(1, np.nan), np.full(ev.n_vars, np.nan), np.full(ev.n_constraints, np.nan),
+                    np.full(ev.nnz_jacobian, np.nan), np.full(ev.nnz_hessian, np.nan)]
+            ev.eval_all(Z, 1.7, mu, *bufs)
+            assert all(np.isfinite(b).all() for b in bufs), rep
+            for a, b in zip(ref, bufs):
+                assert np.array_equal(a, b), rep
+        H = np.full(ev.nnz_hessian, np.nan)
+        ev.eval_hessian_lagrangian(H, Z, 1.7, mu)
+        assert np.array_equal(H, bufs[4])
+        ev.close()
 
 
 @pytest.mark.parametrize("kind", ["persistent", "octet", "generic", "dmma", "tdb"])

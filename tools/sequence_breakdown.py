@@ -1,5 +1,5 @@
 """Wall time of each of the five callbacks on a new iterate (c2 by default), registered and plain output buffers, and of the
-fused call under several pipeline plans.  Usage: python tools/sequence_breakdown.py [c2|c4]"""
+fused call.  Usage: python tools/sequence_breakdown.py [c2|c4]"""
 import os
 import sys
 import time
@@ -17,11 +17,7 @@ prob = bench.build_problem(wl, 42)
 rng = np.random.default_rng(0)
 
 
-def run(register, plan=None, reps=30):
-    if plan is None:
-        os.environ.pop("DTO_B200_PIPELINE", None)
-    else:
-        os.environ["DTO_B200_PIPELINE"] = plan
+def run(register, reps=30):
     ev = dto.Evaluator(prob)
     Z = prob.trajectory.vec()
     pin = lambda a: torch.from_numpy(a).pin_memory().numpy()
@@ -49,11 +45,10 @@ def run(register, plan=None, reps=30):
     for i in range(reps):
         ev.eval_all(Zs[i % 3], 1.0, mus[i % 3], J, grad, g, jac, hess)
     fused = (time.perf_counter() - t0) * 1e3 / reps
-    print(f"{wl} register={int(register)} plan={plan or 'default':14s} sequence {acc.sum():.3f} ms = " +
+    print(f"{wl} register={int(register)} sequence {acc.sum():.3f} ms = " +
           " + ".join(f"{n} {v:.3f}" for n, v in zip(names, acc)) + f" | fused {fused:.3f} ms, d2h {ev.last_d2h_bytes / 1e6:.1f} MB", flush=True)
     ev.close()
 
 
 for reg in (True, False):
-    for plan in (None, "0", "0.5", "0.4", "0.3", "0.3,0.65", "0.2,0.6", "0.15,0.5,0.8"):
-        run(reg, plan)
+    run(reg)

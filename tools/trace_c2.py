@@ -1,8 +1,6 @@
 """Device timeline (DTO_B200_TRACE=1) of the fused host-pointer call and of the callback sequence at c2, registered outputs."""
 import os, sys, time
 os.environ["DTO_B200_TRACE"] = "1"
-if len(sys.argv) > 1:
-    os.environ["DTO_B200_PIPELINE"] = sys.argv[1]
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import numpy as np, torch
 import bench, dto_b200 as dto
