@@ -95,6 +95,7 @@ struct dto_handle {
     int device = 0;
     cudaStream_t stream = nullptr;
     DProb P;
+    DGlobKG kg{};                   // order of the (knot variable, global) Hessian sums (global_terms.cu)
     dto_size_info sizes_global{};  // of the WHOLE problem (one batch member)
     dto_size_info sizes_local{};
     int eval_hessian = 1;
@@ -1021,7 +1022,7 @@ extern "C" int dto_create(const dto_problem_desc* d, dto_handle** out) {
             Q.batch = 1;
             double* dZ0 = dev_upload(h, d->Z0, (size_t)N * z + G);
             double* dprobe = dev_upload<double>(h, nullptr, kg_probe.size());
-            launch_global_hessian(Q, dZ0, 1.0, nullptr, nullptr, dprobe, h->stream, &h->launches);
+            launch_global_hessian(Q, h->kg, dZ0, 1.0, nullptr, nullptr, dprobe, h->stream, &h->launches);
             gg_probe.resize((size_t)L.S * gtri);
             if (cudaMemcpyAsync(kg_probe.data(), dprobe, sizeof(double) * kg_probe.size(), cudaMemcpyDeviceToHost, h->stream) != cudaSuccess ||
                 cudaMemcpyAsync(gg_probe.data(), L.scratchH, sizeof(double) * gg_probe.size(), cudaMemcpyDeviceToHost, h->stream) != cudaSuccess ||
@@ -1068,6 +1069,29 @@ extern "C" int dto_create(const dto_problem_desc* d, dto_handle** out) {
         L.kg_pos = dev_upload(h, kg_pos.data(), kg_pos.size());
         L.gg_pos = dev_upload(h, gg_pos.data(), gg_pos.size());
         L.n_hess_tail = (long long)tail.size();
+        // contributors of every (knot variable, global) tail entry in ascending slot order (e is slot-major): summed in
+        // this fixed order by kg_sum_kernel
+        std::vector<std::vector<long long>> contrib(tail.size());
+        for (size_t e = 0; e < (size_t)L.S * KV * G; ++e)
+            if (kg_pos[e] >= 0) contrib[(size_t)kg_pos[e]].push_back((long long)e);
+        std::vector<long long> kg_dst, kg_src;
+        std::vector<int> kg_ptr{0};
+        for (size_t p = 0; p < contrib.size(); ++p)
+            if (!contrib[p].empty()) {
+                kg_dst.push_back((long long)p);
+                kg_src.insert(kg_src.end(), contrib[p].begin(), contrib[p].end());
+                kg_ptr.push_back((int)kg_src.size());
+            }
+        DGlobKG& kg = h->kg;
+        kg.n = (int)kg_dst.size();
+        if (kg.n > 0) {
+            kg.dst = dev_upload(h, kg_dst.data(), kg_dst.size());
+            kg.ptr = dev_upload(h, kg_ptr.data(), kg_ptr.size());
+            kg.src = dev_upload(h, kg_src.data(), kg_src.size());
+            kg.scratch = dev_upload<double>(h, nullptr, (size_t)P.batch * L.S * KV * G);
+            if (!kg.dst || !kg.ptr || !kg.src || !kg.scratch)
+                return fail_create(h, DTO_ERR_ALLOC, "device allocation failed (global terms)");
+        }
     }
 
     // ---- sizes -----------------------------------------------------------------------------------
@@ -1542,7 +1566,7 @@ static int eval_range(dto_handle* h, const DProb& P, const double* dZ, double si
         return DTO_OK;  // knot-range shards have no global variables
     }
     if (f.want_hess) launch_hessian_assemble(P, dZ, sigma, dmu, dhess, h->stream, &h->launches);
-    if (f.want_hess) launch_global_hessian(P, dZ, sigma, dmu, dhess, nullptr, h->stream, &h->launches);
+    if (f.want_hess) launch_global_hessian(P, h->kg, dZ, sigma, dmu, dhess, nullptr, h->stream, &h->launches);
     return DTO_OK;
 }
 

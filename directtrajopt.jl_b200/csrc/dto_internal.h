@@ -109,6 +109,17 @@ struct DGlob {
     long long n_hess_tail;
 };
 
+// The (knot variable, global) Hessian entries of the terms with global variables, summed in a fixed order: every slot
+// writes its contribution to the scratch, kg_sum_kernel adds each entry's contributors in ascending slot order.  Kept
+// beside DProb, not in it: the kernels that never read it keep their parameter block.
+struct DGlobKG {
+    double* scratch;       // [batch][S][KV][G] per-slot (knot variable a, global g) entries
+    int n;                 // Hessian tail entries of (knot variable, global) pairs
+    const long long* dst;  // [n] their positions inside the Hessian tail
+    const int* ptr;        // [n + 1]: the contributors of entry i are src[ptr[i] .. ptr[i+1])
+    const long long* src;  // index (s KV + a) G + g into a problem's scratch rows, ascending slot s
+};
+
 struct DProb {
     int N;          // global knots
     int z, dt_off, batch;
@@ -315,7 +326,7 @@ void launch_objective(const DProb& P, const double* Z, double* J, double* grad, 
 void launch_violation(const DProb& P, const double* g, const int* row_is_eq, double* viol, cudaStream_t st, long long* launches);
 // terms with global variables: global part of the gradient, (knot, global) and (global, global) Hessian entries
 void launch_global_gradient(const DProb& P, const double* Z, double* grad, cudaStream_t st, long long* launches);
-void launch_global_hessian(const DProb& P, const double* Z, double sigma, const double* mu, double* hess, double* kg_probe,
+void launch_global_hessian(const DProb& P, const DGlobKG& kg, const double* Z, double sigma, const double* mu, double* hess, double* kg_probe,
                            cudaStream_t st, long long* launches);
 void launch_jac_product(const DProb& P, const double* jac, const long long* rows0, const long long* cols0, const double* w,
                         double* y, bool transpose, cudaStream_t st, long long* launches);

@@ -9,10 +9,12 @@
 //   global part of the gradient      g[zN + gi]   = sum_slots w Q dl/dg_gi            (global_objectives.jl:262-266)
 //   (global, global) Hessian entries H[gi, gj]    = sum_slots factor d2/(dg_gi dg_gj)  (global_objectives.jl:334-337,
 //                                                                                       global_knot_point_constraint.jl:243-245)
-//   (knot, global) Hessian entries   H[(k,a), gi] = factor d2/(dv_a dg_gi)             (one slot each)
+//   (knot, global) Hessian entries   H[(k,a), gi] = sum_slots factor d2/(dv_a dg_gi)   (the slots of the terms that
+//                                                                                       list knot k and read v_a, gi)
 // One "slot" = (term, listed time).  Each slot writes its contribution to a slot-major scratch row; a second kernel sums
-// the columns in a fixed order (bit-reproducible).  All of them live in the tail of the Hessian value array: the global
-// columns come after every knot column in the column-major upper triangle (evaluator.jl:199-203).
+// every entry's contributors in ascending slot order (bit-reproducible, whatever the schedule).  All of them live in the
+// tail of the Hessian value array: the global columns come after every knot column in the column-major upper triangle
+// (evaluator.jl:199-203).
 #include "dto_internal.h"
 #include "knotfun.cuh"
 
@@ -50,7 +52,7 @@ __global__ void global_grad_kernel(DProb P, const double* __restrict__ Z, long l
 // thread per (problem, slot, item): item < Gtri -> (gi <= gj) pair into the scratch; then (knot variable a, global gi)
 template <bool Prog>
 __global__ void global_hess_kernel(DProb P, const double* __restrict__ Z, double sigma, const double* __restrict__ mu,
-                                   double* __restrict__ hess, double* __restrict__ kg_probe, long long total) {
+                                   double* __restrict__ kg_scratch, double* __restrict__ kg_probe, long long total) {
     const long long t = (long long)blockIdx.x * blockDim.x + threadIdx.x;
     if (t >= total) return;
     const DGlob& L = P.gl;
@@ -111,12 +113,23 @@ __global__ void global_hess_kernel(DProb P, const double* __restrict__ Z, double
         const long long e = ((long long)s * L.KV + a) * G + gi;
         if (kg_probe != nullptr) {
             if (b == 0) kg_probe[e] = val;
-        } else {
-            const long long pos = L.kg_pos[e];
-            // several terms may couple the same (knot variable, global) pair: at most a handful of adds per entry
-            if (pos >= 0) atomicAdd(hess + (long long)b * P.nnz_hess_local + L.hess_tail_off + pos, val);
+        } else if (L.kg_pos[e] >= 0) {
+            // several terms may couple the same (knot variable, global) pair: kg_sum_kernel adds them in slot order
+            kg_scratch[(long long)b * L.S * L.KV * G + e] = val;
         }
     }
+}
+
+// hess[tail + kg.dst[i]] = sum of entry i's contributors in ascending slot order; thread per (problem, entry)
+__global__ void kg_sum_kernel(DProb P, DGlobKG kg, double* __restrict__ hess, long long total) {
+    const long long t = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (t >= total) return;
+    const DGlob& L = P.gl;
+    const int i = (int)(t % kg.n), b = (int)(t / kg.n);
+    const double* sc = kg.scratch + (long long)b * L.S * L.KV * L.G;
+    double acc = 0.0;
+    for (int p = kg.ptr[i]; p < kg.ptr[i + 1]; ++p) acc += sc[kg.src[p]];
+    hess[(long long)b * P.nnz_hess_local + L.hess_tail_off + kg.dst[i]] = acc;
 }
 
 // out[b*out_stride + out_off + pos[w]] = sum_s scratch[b][s][w]; one warp per (problem, column), fixed order
@@ -159,25 +172,29 @@ void launch_global_gradient(const DProb& P, const double* Z, double* grad, cudaS
     ++*launches;
 }
 
-void launch_global_hessian(const DProb& P, const double* Z, double sigma, const double* mu, double* hess, double* kg_probe,
+void launch_global_hessian(const DProb& P, const DGlobKG& kg, const double* Z, double sigma, const double* mu, double* hess, double* kg_probe,
                            cudaStream_t st, long long* launches) {
     const DGlob& L = P.gl;
     if (L.G == 0 || L.S == 0) return;
     const int gtri = L.G * (L.G + 1) / 2;
-    if (kg_probe == nullptr) {
-        if (L.n_hess_tail == 0) return;
-        cudaMemset2DAsync(hess + L.hess_tail_off, sizeof(double) * P.nnz_hess_local, 0, sizeof(double) * L.n_hess_tail, P.batch, st);
-    }
+    if (kg_probe == nullptr && L.n_hess_tail == 0) return;
     const long long total = (long long)P.batch * L.S * (gtri + L.KV * L.G);
     if (global_programs(P, true) || global_programs(P, false))
-        global_hess_kernel<true><<<(unsigned)((total + 127) / 128), 128, 0, st>>>(P, Z, sigma, mu, hess, kg_probe, total);
+        global_hess_kernel<true><<<(unsigned)((total + 127) / 128), 128, 0, st>>>(P, Z, sigma, mu, kg.scratch, kg_probe, total);
     else
-        global_hess_kernel<false><<<(unsigned)((total + 127) / 128), 128, 0, st>>>(P, Z, sigma, mu, hess, kg_probe, total);
+        global_hess_kernel<false><<<(unsigned)((total + 127) / 128), 128, 0, st>>>(P, Z, sigma, mu, kg.scratch, kg_probe, total);
     ++*launches;
     if (kg_probe == nullptr) {
+        // every tail entry is either a (global, global) pair or has at least one (knot, global) contributor: the two sums
+        // assign the whole tail
         const long long cols = (long long)P.batch * gtri;
         column_sum_kernel<<<(unsigned)((cols + 3) / 4), 128, 0, st>>>(P.batch, L.S, gtri, L.scratchH, L.gg_pos, hess, P.nnz_hess_local,
                                                                       L.hess_tail_off);
         ++*launches;
+        if (kg.n > 0) {
+            const long long items = (long long)P.batch * kg.n;
+            kg_sum_kernel<<<(unsigned)((items + 127) / 128), 128, 0, st>>>(P, kg, hess, items);
+            ++*launches;
+        }
     }
 }
