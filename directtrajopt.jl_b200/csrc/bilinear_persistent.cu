@@ -1293,16 +1293,6 @@ bool launch_variant(const DProb& P, int ii, const double* Z, const double* mu, d
 
 }  // namespace
 
-// the swizzled shared-memory image of the (m+1) row-major generators (what the kernel's prologue stages)
-void bilinear_persistent_swizzled(int n, int m, const double* Grm, double* out) {
-    const int NT = n / 8;
-    const size_t nn = (size_t)n * n;
-    for (int i = 0; i <= m; ++i)
-        for (int s = 0; s < n; ++s)
-            for (int k = 0; k < n; ++k) out[i * nn + (size_t)s * n + ((NT % 2 == 0) ? (k ^ ((s & 1) << 3)) : k)] = Grm[i * nn + (size_t)s * n + k];
-}
-
-
 bool bilinear_persistent_supported(int n, int m) {
     if (m < 0 || m > kMaxDrives) return false;
     return n == 8 || n == 16 || n == 24 || n == 32 || n == 48 || n == 64;

@@ -23,9 +23,7 @@ static thread_local std::string g_create_error;
 struct ConEntry {
     long long col_local;  // local column
     long long grow;       // global 0-based row
-    long long lrow;       // local 0-based row
-    long long e;          // index into the constraint's dense [j][a][i] table
-    int ci;
+    long long e;          // local position
 };
 
 // Host threads that write structural zeros into the caller's Hessian buffer while the GPU computes and the copy
@@ -102,11 +100,9 @@ struct dto_handle {
     int sharded = 0;
     int k0 = 1, k1 = 1;
     std::vector<void*> allocs;
-    // host copies of the descriptor
-    std::vector<dto_integrator_desc> ints;
-    std::vector<dto_objective_desc> objs;
-    std::vector<dto_constraint_desc> cons;
-    std::vector<std::vector<int>> obj_var_offs, obj_times, con_var_offs, con_times;
+    bool upload_failed = false;  // a required dev_upload failed during construction
+    // host copies of the constraints' variable offsets (knot, then global) and listed times
+    std::vector<std::vector<int>> con_var_offs, con_times;
     std::vector<std::vector<int>> con_own_ti;  // owned entries per constraint
     std::vector<long long> int_goff;           // global row offset of each integrator
     std::vector<long long> con_goff;           // global row offset of each constraint (after dynamics)
@@ -114,7 +110,6 @@ struct dto_handle {
     std::vector<ConEntry> con_entries;         // stored constraint Jacobian entries (owned), sorted by (col, row)
     std::vector<std::vector<unsigned char>> con_stored_all;  // per constraint: stored mask over ALL times [ti][a][i]
     std::vector<int> row_is_eq;
-    int G = 0;                                             // traj.global_dim
     std::vector<std::pair<long long, long long>> hess_tail;  // (global column gi, 0-based row) of the Hessian's global columns
     // device buffers
     double *dZ = nullptr, *dmu = nullptr, *dg = nullptr, *djac = nullptr, *dhess = nullptr, *dgrad = nullptr, *dJ = nullptr,
@@ -214,20 +209,26 @@ struct dto_handle {
         }                                                                                        \
     } while (0)
 
+// A device copy of `count` elements of src (zeros when src is null), freed with the handle; nullptr when count is 0 or
+// the allocation, copy or memset fails.  A failure of a required upload sets h->upload_failed, which dto_create checks;
+// an optional one (the caller has a fall-back) clears the CUDA error state instead.
 template <class T>
-static T* dev_upload(dto_handle* h, const T* src, size_t count) {
+static T* dev_upload(dto_handle* h, const T* src, size_t count, bool optional = false) {
     if (count == 0) return nullptr;
     void* p = nullptr;
-    if (cudaMalloc(&p, count * sizeof(T)) != cudaSuccess) return nullptr;
-    h->allocs.push_back(p);
-    if (src) cudaMemcpy(p, src, count * sizeof(T), cudaMemcpyHostToDevice);
-    else cudaMemset(p, 0, count * sizeof(T));
-    return (T*)p;
+    if (cudaMalloc(&p, count * sizeof(T)) == cudaSuccess) {
+        h->allocs.push_back(p);
+        if ((src ? cudaMemcpy(p, src, count * sizeof(T), cudaMemcpyHostToDevice) : cudaMemset(p, 0, count * sizeof(T))) == cudaSuccess)
+            return (T*)p;
+    }
+    if (optional) cudaGetLastError();
+    else h->upload_failed = true;
+    return nullptr;
 }
 
-static int fail_create(dto_handle* h, int code, const std::string& msg) {
+// records why dto_create fails; dto_create destroys the handle
+static int reject(int code, const std::string& msg) {
     g_create_error = msg;
-    if (h) dto_destroy(h);
     return code;
 }
 
@@ -394,11 +395,10 @@ static int upload_knot_program(dto_handle* h, const dto_problem_desc* d, int ind
     std::vector<int4> words;
     std::string msg;
     const int rc = compile_knot_program(d, index, n_vars, n_params, n_out, words, msg);
-    if (rc != DTO_OK) return fail_create(h, rc, msg);
+    if (rc != DTO_OK) return reject(rc, msg);
     const int cw = (d->programs[index].n_consts + 1) / 2;
     pg.n_code = (int)words.size() - cw;
     pg.code = dev_upload(h, words.data(), words.size());
-    if (!pg.code) return fail_create(h, DTO_ERR_ALLOC, "device allocation failed (knot program)");
     return DTO_OK;
 }
 
@@ -434,28 +434,27 @@ extern "C" void dto_destroy(dto_handle* h) {
 }
 
 
-extern "C" int dto_create(const dto_problem_desc* d, dto_handle** out) {
-    if (!d || !out) return fail_create(nullptr, DTO_ERR_INVALID, "null descriptor");
-    *out = nullptr;
+// ---- construction ----------------------------------------------------------------------------------
+// dto_create runs the stages below in order.  A stage that fails records the message (reject) and returns its code;
+// dto_create then destroys the handle.
+
+static int check_header(const dto_problem_desc* d) {
     // version 3 descriptors (no knot programs) end before n_programs: those fields are read only at version 4
-    if (d->abi_version != DTO_B200_ABI_VERSION && d->abi_version != 3) return fail_create(nullptr, DTO_ERR_INVALID, "ABI version mismatch");
-    const bool with_programs = d->abi_version >= 4;
-    if (with_programs && (d->n_programs < 0 || (d->n_programs > 0 && !d->programs)))
-        return fail_create(nullptr, DTO_ERR_INVALID, "bad knot program table");
-    if (d->N < 2 || d->z < 1 || d->batch < 1) return fail_create(nullptr, DTO_ERR_INVALID, "need N >= 2, z >= 1, batch >= 1");
-    if (d->dt_off < 0 || d->dt_off >= d->z) return fail_create(nullptr, DTO_ERR_INVALID, "timestep component outside the knot");
+    if (d->abi_version != DTO_B200_ABI_VERSION && d->abi_version != 3) return reject(DTO_ERR_INVALID, "ABI version mismatch");
+    if (d->abi_version >= 4 && (d->n_programs < 0 || (d->n_programs > 0 && !d->programs)))
+        return reject(DTO_ERR_INVALID, "bad knot program table");
+    if (d->N < 2 || d->z < 1 || d->batch < 1) return reject(DTO_ERR_INVALID, "need N >= 2, z >= 1, batch >= 1");
+    if (d->dt_off < 0 || d->dt_off >= d->z) return reject(DTO_ERR_INVALID, "timestep component outside the knot");
     if (d->n_integrators < 1)
-        return fail_create(nullptr, DTO_ERR_UNSUPPORTED, "at least one integrator is required (dense block Hessian structure)");
+        return reject(DTO_ERR_UNSUPPORTED, "at least one integrator is required (dense block Hessian structure)");
     if (d->n_integrators > DTO_MAX_INT || d->n_objectives > DTO_MAX_OBJ || d->n_constraints > DTO_MAX_CON)
-        return fail_create(nullptr, DTO_ERR_UNSUPPORTED, "too many integrators / objective terms / constraints");
-    int ndev = 0;
-    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0)
-        return fail_create(nullptr, DTO_ERR_CUDA, "no CUDA device: libdto_b200 has no CPU fallback");
-    cudaGetLastError();  // do not inherit a stale error from an earlier, unrelated call
-    dto_handle* h = new (std::nothrow) dto_handle();
-    if (!h) return fail_create(nullptr, DTO_ERR_ALLOC, "out of host memory");
+        return reject(DTO_ERR_UNSUPPORTED, "too many integrators / objective terms / constraints");
+    return DTO_OK;
+}
+
+static int open_device(dto_handle* h, const dto_problem_desc* d, int& smem_optin) {
     if (d->device >= 0) {
-        if (cudaSetDevice(d->device) != cudaSuccess) return fail_create(h, DTO_ERR_CUDA, "cudaSetDevice failed");
+        if (cudaSetDevice(d->device) != cudaSuccess) return reject(DTO_ERR_CUDA, "cudaSetDevice failed");
         h->device = d->device;
     } else {
         cudaGetDevice(&h->device);
@@ -463,40 +462,41 @@ extern "C" int dto_create(const dto_problem_desc* d, dto_handle** out) {
     if (cudaStreamCreateWithFlags(&h->stream, cudaStreamNonBlocking) != cudaSuccess ||
         cudaStreamCreateWithFlags(&h->aux_stream, cudaStreamNonBlocking) != cudaSuccess ||
         cudaStreamCreateWithFlags(&h->copy_stream, cudaStreamNonBlocking) != cudaSuccess)
-        return fail_create(h, DTO_ERR_CUDA, "cudaStreamCreate failed");
+        return reject(DTO_ERR_CUDA, "cudaStreamCreate failed");
     for (cudaEvent_t* e : {&h->ev_fork, &h->ev_join, &h->ev_side_fork, &h->ev_side, &h->ev_g_ready, &h->ev_scal_done, &h->ev_small, &h->ev_g})
-        if (cudaEventCreateWithFlags(e, cudaEventDisableTiming) != cudaSuccess) return fail_create(h, DTO_ERR_CUDA, "cudaEventCreate failed");
-    // the kernels whose shared memory grows with the shape are checked against it here, so that a shape no kernel can
+        if (cudaEventCreateWithFlags(e, cudaEventDisableTiming) != cudaSuccess) return reject(DTO_ERR_CUDA, "cudaEventCreate failed");
+    // the kernels whose shared memory grows with the shape are checked against it, so that a shape no kernel can
     // launch is rejected at construction instead of failing at its first evaluation
-    int smem_optin = 0;
     if (cudaDeviceGetAttribute(&smem_optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, h->device) != cudaSuccess)
-        return fail_create(h, DTO_ERR_CUDA, "cudaDeviceGetAttribute(MaxSharedMemoryPerBlockOptin) failed");
-    auto smem_msg = [&](const std::string& what, size_t need) {
-        return what + " needs " + std::to_string(need) + " bytes of shared memory per block, above the device's limit of " +
-               std::to_string(smem_optin) + " bytes";
-    };
+        return reject(DTO_ERR_CUDA, "cudaDeviceGetAttribute(MaxSharedMemoryPerBlockOptin) failed");
+    return DTO_OK;
+}
 
-    const int N = d->N, z = d->z;
+static std::string smem_msg(const std::string& what, size_t need, int smem_optin) {
+    return what + " needs " + std::to_string(need) + " bytes of shared memory per block, above the device's limit of " +
+           std::to_string(smem_optin) + " bytes";
+}
+
+// the knot window of this handle (a shard owns knots k0..k1 and reads the halo knot k1 + 1)
+static int init_problem(dto_handle* h, const dto_problem_desc* d) {
     h->eval_hessian = d->eval_hessian;
     h->sharded = d->shard_k0 > 0;
     h->k0 = h->sharded ? d->shard_k0 : 1;
-    h->k1 = h->sharded ? d->shard_k1 : N;
-    if (h->k0 < 1 || h->k1 > N || h->k0 > h->k1) return fail_create(h, DTO_ERR_INVALID, "bad shard range");
-    if (h->sharded && d->batch != 1) return fail_create(h, DTO_ERR_UNSUPPORTED, "knot-range shards require batch == 1");
+    h->k1 = h->sharded ? d->shard_k1 : d->N;
+    if (h->k0 < 1 || h->k1 > d->N || h->k0 > h->k1) return reject(DTO_ERR_INVALID, "bad shard range");
+    if (h->sharded && d->batch != 1) return reject(DTO_ERR_UNSUPPORTED, "knot-range shards require batch == 1");
+    if (d->global_dim < 0 || d->global_dim > 1024) return reject(DTO_ERR_INVALID, "global_dim outside 0..1024");
+    if (d->global_dim > 0 && h->sharded) return reject(DTO_ERR_UNSUPPORTED, "knot-range shards do not support global variables");
     const int G = d->global_dim;
-    if (G < 0 || G > 1024) return fail_create(h, DTO_ERR_INVALID, "global_dim outside 0..1024");
-    if (G > 0 && h->sharded) return fail_create(h, DTO_ERR_UNSUPPORTED, "knot-range shards do not support global variables");
-    h->G = G;
-
     DProb& P = h->P;
     memset(&P, 0, sizeof(P));
-    P.N = N;
-    P.z = z;
+    P.N = d->N;
+    P.z = d->z;
     P.dt_off = d->dt_off;
     P.batch = d->batch;
     P.kb = h->k0;
     P.nOwn = h->k1 - h->k0 + 1;
-    P.nK = P.nOwn + (h->k1 < N ? 1 : 0);
+    P.nK = P.nOwn + (h->k1 < d->N ? 1 : 0);
     P.nI = P.nK - 1;
     P.kc0 = 0;
     P.kc1 = P.nK;
@@ -504,16 +504,142 @@ extern "C" int dto_create(const dto_problem_desc* d, dto_handle** out) {
     P.n_int = d->n_integrators;
     P.n_obj = d->n_objectives;
     P.n_con = d->n_constraints;
-    P.n_vars_local = (long long)P.nK * z + G;
-    P.n_grad_local = (long long)P.nOwn * z + G;
-    P.gl.G = G;
+    P.n_vars_local = (long long)P.nK * d->z + G;
+    P.n_grad_local = (long long)P.nOwn * d->z + G;
+    P.gl.G = G;  // traj.global_dim
+    return DTO_OK;
+}
 
-    // ---- integrators -------------------------------------------------------------------------
+// pin: DTO_B200_KERNEL (see build_integrators)
+static int bilinear_variant(int n, int m, bool shared_G, const std::string& pin) {
+    if (pin == "generic") return DTO_VAR_GENERIC;
+    // small states: eight intervals per warp, one tile per jet component (bilinear_octet.cu)
+    const bool octet = bilinear_octet_supported(n, m);
+    if (shared_G && bilinear_persistent_supported(n, m) && pin != "dmma") return octet && pin != "persistent" ? DTO_VAR_OCTET : DTO_VAR_PERSISTENT;
+    if (!shared_G && octet && pin != "dmma" && pin != "persistent") return DTO_VAR_OCTET;  // per-problem generators: fragment-ordered copies
+    return bilinear_dmma_supported(n, m) ? DTO_VAR_DMMA : DTO_VAR_GENERIC;
+}
+
+// Row-major copies of `count` column-major n x n matrices.  With `swizzle` and n / 8 even, column c of row r sits at
+// c ^ ((r & 1) << 3): the shared-memory layout of the tensor-core tiles (dmma_tiles.cuh, the persistent kernel's prologue).
+static std::vector<double> row_major(const double* src, int n, size_t count, bool swizzle) {
+    const size_t nn = (size_t)n * n;
+    const bool x = swizzle && (n / 8) % 2 == 0;
+    std::vector<double> out(count * nn);
+    for (size_t q = 0; q < count; ++q)
+        for (int r = 0; r < n; ++r)
+            for (int c = 0; c < n; ++c) out[q * nn + (size_t)r * n + (x ? (c ^ ((r & 1) << 3)) : c)] = src[q * nn + (size_t)c * n + r];
+    return out;
+}
+
+static int build_bilinear(dto_handle* h, const dto_problem_desc* d, const dto_integrator_desc& s, DInt& I, const std::string& pin, int smem_optin) {
+    const int n = s.x_dim;
+    if (s.u_dim < 0 || s.u_off < 0 || s.u_off + s.u_dim > d->z || !s.G)
+        return reject(DTO_ERR_INVALID, "bilinear integrator: bad drive component or missing generators");
+    const size_t nn = (size_t)n * n, per = (size_t)(s.u_dim + 1) * nn;
+    const size_t cnt = s.G_batch_stride ? (size_t)s.G_batch_stride * (d->batch - 1) + per : per;
+    I.G = dev_upload(h, s.G, cnt);
+    I.G_stride = s.G_batch_stride;
+    std::vector<double> rm = row_major(s.G, n, cnt / nn, false);
+    rm.resize(cnt);
+    I.Grm = dev_upload(h, rm.data(), cnt);
+    if (s.G_batch_stride == 0 && n % 8 == 0) I.Gsw = dev_upload(h, row_major(s.G, n, s.u_dim + 1, true).data(), per);
+    I.hs_stride = (s.u_dim + 1) * n + (s.u_dim + 1) * (s.u_dim + 1);
+    I.variant = bilinear_variant(n, s.u_dim, s.G_batch_stride == 0, pin);
+    if (I.variant >= DTO_VAR_PERSISTENT && s.G_batch_stride == 0) I.wq = dev_upload<unsigned long long>(h, nullptr, 4);
+    if (I.variant == DTO_VAR_OCTET && s.G_batch_stride != 0) {
+        const size_t fd = bilinear_octet_fragment_doubles(n, s.u_dim);
+        std::vector<double> frag(fd * (size_t)d->batch);
+        for (int b = 0; b < d->batch; ++b)
+            bilinear_octet_fragments(n, s.u_dim, s.G + (size_t)b * s.G_batch_stride, frag.data() + (size_t)b * fd);
+        I.bfrag = dev_upload(h, frag.data(), frag.size());
+    }
+    if (n > 96) return reject(DTO_ERR_UNSUPPORTED, "bilinear integrator: state dimension > 96 not supported");
+    if (I.variant == DTO_VAR_GENERIC) {  // one block per interval holds the generator and every jet column
+        const size_t need = generic_smem_bytes(n, s.u_dim, true, d->eval_hessian);
+        if (need > (size_t)smem_optin)
+            return reject(DTO_ERR_UNSUPPORTED, smem_msg("bilinear integrator: the generic kernel at state dimension " + std::to_string(n) + " with " +
+                                                            std::to_string(s.u_dim) + " drives" + (d->eval_hessian ? " and the Hessian" : ""), need, smem_optin));
+    }
+    return DTO_OK;
+}
+
+static int build_tdbilinear(dto_handle* h, const dto_problem_desc* d, const dto_integrator_desc& s, DInt& I, const std::string& pin, int smem_optin) {
+    const int n = s.x_dim;
+    if (s.u_dim < 0 || s.u_off < 0 || s.u_off + s.u_dim > d->z || s.t_off < 0 || s.t_off >= d->z || !s.G)
+        return reject(DTO_ERR_INVALID, "tdbilinear integrator: bad components");
+    if (s.spline_order != 0 && s.spline_order != 1) return reject(DTO_ERR_UNSUPPORTED, "Unsupported spline order");
+    const size_t nn = (size_t)n * n;
+    I.G = dev_upload(h, s.G, nn);
+    I.A = dev_upload(h, s.A, nn * s.u_dim);
+    I.B = dev_upload(h, s.B, nn * s.u_dim);
+    I.omega = dev_upload(h, s.omega, s.u_dim);
+    I.phi = dev_upload(h, s.phi, s.u_dim);
+    I.D = dev_upload(h, s.D, nn * s.n_carrier);
+    I.omega_d = dev_upload(h, s.omega_d, s.n_carrier);
+    I.phi_d = dev_upload(h, s.phi_d, s.n_carrier);
+    // 1-norms that bound ||G(u, t)||_1 for the per-interval macro-step count (tdb_item_steps)
+    auto norm1 = [&](const double* M) {
+        double best = 0.0;
+        for (int c = 0; c < n; ++c) {
+            double sum = 0.0;
+            for (int r = 0; r < n; ++r) sum += fabs(M[(size_t)c * n + r]);
+            best = std::max(best, sum);
+        }
+        return best;
+    };
+    std::vector<double> bn((size_t)std::max(s.u_dim, 1), 0.0);
+    I.tdb_gnorm = norm1(s.G);
+    I.tdb_wmax = 0.0;
+    // DTO_B200_TDB_TOL=0: eight extrapolation columns everywhere (round 1); default: sized per interval
+    const char* tl = getenv("DTO_B200_TDB_TOL");
+    I.tdb_tol = tl ? atof(tl) : 1e-14;
+    for (int i = 0; i < s.u_dim; ++i) {
+        bn[i] = norm1(s.A + (size_t)i * nn) + norm1(s.B + (size_t)i * nn);
+        I.tdb_wmax = std::max(I.tdb_wmax, fabs(s.omega[i]));
+    }
+    for (int j = 0; j < s.n_carrier; ++j) {
+        I.tdb_gnorm += norm1(s.D + (size_t)j * nn);
+        I.tdb_wmax = std::max(I.tdb_wmax, fabs(s.omega_d[j]));
+    }
+    I.tdb_bnorm = dev_upload(h, bn.data(), bn.size());
+    if (n % 8 == 0 && n <= 64) {  // swizzled row-major copies for the tensor-core variant
+        I.Grm = dev_upload(h, row_major(s.G, n, 1, true).data(), nn);
+        if (s.u_dim > 0) {
+            I.Asw = dev_upload(h, row_major(s.A, n, s.u_dim, true).data(), nn * s.u_dim);
+            I.Bsw = dev_upload(h, row_major(s.B, n, s.u_dim, true).data(), nn * s.u_dim);
+        }
+        if (s.n_carrier > 0) I.Dsw = dev_upload(h, row_major(s.D, n, s.n_carrier, true).data(), nn * s.n_carrier);
+        int sms = 148;
+        cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, h->device);
+        I.tdb_scratch_ctas = 2 * sms;
+        // [CTA][16 warps][accumulator, start][one tile in fragment order]
+        I.tdb_scratch = dev_upload<double>(h, nullptr, (size_t)I.tdb_scratch_ctas * 16 * 2 * (n / 8) * 64);
+    }
+    const int np = (s.spline_order == 1 ? 2 * s.u_dim : s.u_dim) + 2;
+    I.hs_stride = np * n + np * np;
+    if (s.spline_order == 1) {
+        h->P.any_cross = 1;
+        h->hblk_len += I.hs_stride;
+        if (h->k0 > 1) h->hs_left = 1;
+    }
+    I.variant = (I.Asw != nullptr && tdb_dmma_supported(I) && pin != "generic") ? DTO_VAR_DMMA : DTO_VAR_GENERIC;
+    if (!tdb_fits(I, (size_t)smem_optin))
+        return reject(DTO_ERR_UNSUPPORTED, "tdbilinear integrator: more than 4 drives or 4 carriers, or a state too large for the device's " +
+                                               std::to_string(smem_optin) + " bytes of shared memory per block");
+    if (n > 96) return reject(DTO_ERR_UNSUPPORTED, "tdbilinear integrator: state dimension > 96 not supported");
+    return DTO_OK;
+}
+
+static int build_integrators(dto_handle* h, const dto_problem_desc* d, int smem_optin, long long& n_dyn_global, long long& n_dyn_local) {
+    DProb& P = h->P;
+    // DTO_B200_KERNEL=generic|dmma|persistent pins an older variant (A/B measurements, parity tests of every variant)
+    const char* pin_env = getenv("DTO_B200_KERNEL");
+    const std::string pin = pin_env ? pin_env : "";
     long long goff = 0, loff = 0;
     int doff = 0;
     for (int i = 0; i < d->n_integrators; ++i) {
         const dto_integrator_desc& s = d->integrators[i];
-        h->ints.push_back(s);
         DInt& I = P.in[i];
         I.kind = s.kind;
         I.x_off = s.x_off;
@@ -526,176 +652,85 @@ extern "C" int dto_create(const dto_problem_desc* d, dto_handle** out) {
         I.doff = doff;
         I.row_off = loff;
         I.steps = s.tdb_steps > 0 ? s.tdb_steps : 1;
-        if (s.x_dim < 1 || s.x_off < 0 || s.x_off + s.x_dim > z) return fail_create(h, DTO_ERR_INVALID, "integrator state component outside the knot");
-        const size_t nn = (size_t)s.x_dim * s.x_dim;
-        if (s.kind == DTO_INT_BILINEAR) {
-            if (s.u_dim < 0 || s.u_off < 0 || s.u_off + s.u_dim > z || !s.G) return fail_create(h, DTO_ERR_INVALID, "bilinear integrator: bad drive component or missing generators");
-            const size_t per = (size_t)(s.u_dim + 1) * nn;
-            const size_t cnt = s.G_batch_stride ? (size_t)s.G_batch_stride * (d->batch - 1) + per : per;
-            I.G = dev_upload(h, s.G, cnt);
-            I.G_stride = s.G_batch_stride;
-            {
-                std::vector<double> rm(cnt);
-                const size_t nmat = cnt / nn;
-                for (size_t q = 0; q < nmat; ++q)
-                    for (int r = 0; r < s.x_dim; ++r)
-                        for (int c = 0; c < s.x_dim; ++c) rm[q * nn + (size_t)r * s.x_dim + c] = s.G[q * nn + (size_t)c * s.x_dim + r];
-                I.Grm = dev_upload(h, rm.data(), cnt);
-                if (s.G_batch_stride == 0 && s.x_dim % 8 == 0) {  // what the persistent kernel's prologue stages
-                    std::vector<double> swz(per);
-                    bilinear_persistent_swizzled(s.x_dim, s.u_dim, rm.data(), swz.data());
-                    I.Gsw = dev_upload(h, swz.data(), per);
-                }
-            }
-            I.hs_stride = (s.u_dim + 1) * s.x_dim + (s.u_dim + 1) * (s.u_dim + 1);
-            I.variant = bilinear_dmma_supported(s.x_dim, s.u_dim) ? DTO_VAR_DMMA : DTO_VAR_GENERIC;
-            // DTO_B200_KERNEL=generic|dmma pins an older variant (A/B measurements, parity tests of every variant)
-            const char* pin = getenv("DTO_B200_KERNEL");
-            const bool pin_generic = pin && strcmp(pin, "generic") == 0, pin_dmma = pin && strcmp(pin, "dmma") == 0;
-            const bool pin_persistent = pin && strcmp(pin, "persistent") == 0;
-            if (bilinear_persistent_supported(s.x_dim, s.u_dim) && s.G_batch_stride == 0 && !pin_dmma && !pin_generic) {
-                I.variant = DTO_VAR_PERSISTENT;
-                I.wq = dev_upload<unsigned long long>(h, nullptr, 4);
-                if (!I.wq) return fail_create(h, DTO_ERR_ALLOC, "device allocation failed (work queue)");
-                // small states: eight intervals per warp, one tile per jet component (bilinear_octet.cu)
-                if (bilinear_octet_supported(s.x_dim, s.u_dim) && !pin_persistent) I.variant = DTO_VAR_OCTET;
-            }
-            if (s.G_batch_stride != 0 && bilinear_octet_supported(s.x_dim, s.u_dim) && !pin_dmma && !pin_generic && !pin_persistent) {
-                // per-problem generators at small n: the octet kernel reads each problem's fragment-ordered copy
-                const size_t fd = bilinear_octet_fragment_doubles(s.x_dim, s.u_dim);
-                std::vector<double> frag(fd * (size_t)d->batch);
-                for (int b = 0; b < d->batch; ++b)
-                    bilinear_octet_fragments(s.x_dim, s.u_dim, s.G + (size_t)b * s.G_batch_stride, frag.data() + (size_t)b * fd);
-                I.bfrag = dev_upload(h, frag.data(), frag.size());
-                if (!I.bfrag) return fail_create(h, DTO_ERR_ALLOC, "device allocation failed (generator fragments)");
-                I.variant = DTO_VAR_OCTET;
-            }
-            if (pin_generic) I.variant = DTO_VAR_GENERIC;
-            if (s.x_dim > 96) return fail_create(h, DTO_ERR_UNSUPPORTED, "bilinear integrator: state dimension > 96 not supported");
-            if (I.variant == DTO_VAR_GENERIC) {  // one block per interval holds the generator and every jet column
-                const size_t need = generic_smem_bytes(s.x_dim, s.u_dim, true, d->eval_hessian);
-                if (need > (size_t)smem_optin)
-                    return fail_create(h, DTO_ERR_UNSUPPORTED, smem_msg("bilinear integrator: the generic kernel at state dimension " +
-                                                                        std::to_string(s.x_dim) + " with " + std::to_string(s.u_dim) +
-                                                                        " drives" + (d->eval_hessian ? " and the Hessian" : ""), need));
-            }
-        } else if (s.kind == DTO_INT_DERIVATIVE) {
-            if (s.u_dim != s.x_dim || s.u_off < 0 || s.u_off + s.u_dim > z) return fail_create(h, DTO_ERR_INVALID, "derivative integrator: derivative component must match the variable's dimension");
-        } else if (s.kind == DTO_INT_TDBILINEAR) {
-            if (s.u_dim < 0 || s.u_off < 0 || s.u_off + s.u_dim > z || s.t_off < 0 || s.t_off >= z || !s.G)
-                return fail_create(h, DTO_ERR_INVALID, "tdbilinear integrator: bad components");
-            if (!tdb_available()) return fail_create(h, DTO_ERR_UNSUPPORTED, "tdbilinear integrator kernel is not built into this library");
-            if (s.spline_order != 0 && s.spline_order != 1) return fail_create(h, DTO_ERR_UNSUPPORTED, "Unsupported spline order");
-            I.G = dev_upload(h, s.G, nn);
-            I.A = dev_upload(h, s.A, nn * s.u_dim);
-            I.B = dev_upload(h, s.B, nn * s.u_dim);
-            I.omega = dev_upload(h, s.omega, s.u_dim);
-            I.phi = dev_upload(h, s.phi, s.u_dim);
-            I.D = dev_upload(h, s.D, nn * s.n_carrier);
-            I.omega_d = dev_upload(h, s.omega_d, s.n_carrier);
-            I.phi_d = dev_upload(h, s.phi_d, s.n_carrier);
-            {
-                // 1-norms that bound ||G(u, t)||_1 for the per-interval macro-step count (tdb_item_steps)
-                auto norm1 = [&](const double* M) {
-                    double best = 0.0;
-                    for (int c = 0; c < s.x_dim; ++c) {
-                        double sum = 0.0;
-                        for (int r = 0; r < s.x_dim; ++r) sum += fabs(M[(size_t)c * s.x_dim + r]);
-                        best = std::max(best, sum);
-                    }
-                    return best;
-                };
-                std::vector<double> bn((size_t)std::max(s.u_dim, 1), 0.0);
-                I.tdb_gnorm = norm1(s.G);
-                I.tdb_wmax = 0.0;
-                {   // DTO_B200_TDB_TOL=0: eight extrapolation columns everywhere (round 1); default: sized per interval
-                    const char* tl = getenv("DTO_B200_TDB_TOL");
-                    I.tdb_tol = tl ? atof(tl) : 1e-14;
-                }
-                for (int i = 0; i < s.u_dim; ++i) {
-                    bn[i] = norm1(s.A + (size_t)i * nn) + norm1(s.B + (size_t)i * nn);
-                    I.tdb_wmax = std::max(I.tdb_wmax, fabs(s.omega[i]));
-                }
-                for (int j = 0; j < s.n_carrier; ++j) {
-                    I.tdb_gnorm += norm1(s.D + (size_t)j * nn);
-                    I.tdb_wmax = std::max(I.tdb_wmax, fabs(s.omega_d[j]));
-                }
-                I.tdb_bnorm = dev_upload(h, bn.data(), bn.size());
-            }
-            if (s.x_dim % 8 == 0 && s.x_dim <= 64) {
-                // swizzled row-major copies for the tensor-core variant (layout of dmma_tiles.cuh)
-                const int nd = s.x_dim;
-                const bool swz = (nd / 8) % 2 == 0;
-                auto swizzled = [&](const double* src, int count) {
-                    std::vector<double> out((size_t)count * nn);
-                    for (int qm = 0; qm < count; ++qm)
-                        for (int r = 0; r < nd; ++r)
-                            for (int c = 0; c < nd; ++c)
-                                out[(size_t)qm * nn + (size_t)r * nd + (swz ? (c ^ ((r & 1) << 3)) : c)] = src[(size_t)qm * nn + (size_t)c * nd + r];
-                    return out;
-                };
-                I.Grm = dev_upload(h, swizzled(s.G, 1).data(), nn);
-                if (s.u_dim > 0) {
-                    I.Asw = dev_upload(h, swizzled(s.A, s.u_dim).data(), nn * s.u_dim);
-                    I.Bsw = dev_upload(h, swizzled(s.B, s.u_dim).data(), nn * s.u_dim);
-                }
-                if (s.n_carrier > 0) I.Dsw = dev_upload(h, swizzled(s.D, s.n_carrier).data(), nn * s.n_carrier);
-                int sms = 148;
-                cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, h->device);
-                I.tdb_scratch_ctas = 2 * sms;
-                // [CTA][16 warps][accumulator, start][one tile in fragment order]
-                I.tdb_scratch = dev_upload<double>(h, nullptr, (size_t)I.tdb_scratch_ctas * 16 * 2 * (nd / 8) * 64);
-            }
-            const int np = (s.spline_order == 1 ? 2 * s.u_dim : s.u_dim) + 2;
-            I.hs_stride = np * s.x_dim + np * np;
-            if (s.spline_order == 1) {
-                P.any_cross = 1;
-                h->hblk_len += I.hs_stride;
-                if (h->k0 > 1) h->hs_left = 1;
-            }
-            {
-                const char* pin = getenv("DTO_B200_KERNEL");
-                I.variant = (I.Asw != nullptr && tdb_dmma_supported(I) && !(pin && strcmp(pin, "generic") == 0)) ? DTO_VAR_DMMA : DTO_VAR_GENERIC;
-            }
-            if (!tdb_fits(I, (size_t)smem_optin))
-                return fail_create(h, DTO_ERR_UNSUPPORTED, "tdbilinear integrator: more than 4 drives or 4 carriers, or a state too large for the device's " +
-                                                           std::to_string(smem_optin) + " bytes of shared memory per block");
-            if (s.x_dim > 96) return fail_create(h, DTO_ERR_UNSUPPORTED, "tdbilinear integrator: state dimension > 96 not supported");
-        } else {
-            return fail_create(h, DTO_ERR_UNSUPPORTED, "unknown integrator kind");
-        }
+        if (s.x_dim < 1 || s.x_off < 0 || s.x_off + s.x_dim > d->z) return reject(DTO_ERR_INVALID, "integrator state component outside the knot");
+        int rc;
+        if (s.kind == DTO_INT_BILINEAR) rc = build_bilinear(h, d, s, I, pin, smem_optin);
+        else if (s.kind == DTO_INT_TDBILINEAR) rc = build_tdbilinear(h, d, s, I, pin, smem_optin);
+        else if (s.kind != DTO_INT_DERIVATIVE) rc = reject(DTO_ERR_UNSUPPORTED, "unknown integrator kind");
+        else if (s.u_dim != s.x_dim || s.u_off < 0 || s.u_off + s.u_dim > d->z)
+            rc = reject(DTO_ERR_INVALID, "derivative integrator: derivative component must match the variable's dimension");
+        else rc = DTO_OK;
+        if (rc != DTO_OK) return rc;
         if (I.hs_stride > 0 && d->eval_hessian) {
             // a shard whose first knot receives the previous interval's block (linear-spline tdbilinear) keeps it in a
             // leading row: the assembler reads row kl - 1 = -1
             const int lead = (s.kind == DTO_INT_TDBILINEAR && s.spline_order == 1 && h->k0 > 1) ? 1 : 0;
             I.hs = dev_upload<double>(h, nullptr, (size_t)P.batch * (std::max(P.nI, 1) + lead) * I.hs_stride);
-            if (!I.hs) return fail_create(h, DTO_ERR_ALLOC, "device allocation failed (Hessian scratch)");
-            I.hs += (size_t)lead * I.hs_stride;
+            if (I.hs) I.hs += (size_t)lead * I.hs_stride;
         }
         h->int_goff.push_back(goff);
-        goff += (long long)s.x_dim * (N - 1);
+        goff += (long long)s.x_dim * (d->N - 1);
         loff += (long long)s.x_dim * P.nI;
         doff += s.x_dim;
         h->variants.push_back(s.kind == DTO_INT_BILINEAR ? (I.variant == DTO_VAR_OCTET ? "octet" : I.variant == DTO_VAR_PERSISTENT ? "persistent" : I.variant == DTO_VAR_DMMA ? "dmma" : "generic")
                                                          : (s.kind == DTO_INT_DERIVATIVE ? "analytic" : (I.variant == DTO_VAR_DMMA ? "gbs-dmma" : "gbs")));
     }
     P.Dsum = doff;
-    const long long n_dyn_global = goff, n_dyn_local = loff;
-    {
-        // small-state bilinear kernel + derivative integrators: one kernel writes whole Jacobian columns
-        bool any_deriv = false;
-        for (int i = 0; i < P.n_int; ++i) any_deriv |= P.in[i].kind == DTO_INT_DERIVATIVE;
-        if (any_deriv)
-            for (int i = 0; i < P.n_int && !P.analytic_fused; ++i)
-                if (P.in[i].kind == DTO_INT_BILINEAR && P.in[i].variant == DTO_VAR_OCTET) P.analytic_fused = i + 1;
-    }
+    n_dyn_global = goff;
+    n_dyn_local = loff;
+    // small-state bilinear kernel + derivative integrators: one kernel writes whole Jacobian columns
+    bool any_deriv = false;
+    for (int i = 0; i < P.n_int; ++i) any_deriv |= P.in[i].kind == DTO_INT_DERIVATIVE;
+    if (any_deriv)
+        for (int i = 0; i < P.n_int && !P.analytic_fused; ++i)
+            if (P.in[i].kind == DTO_INT_BILINEAR && P.in[i].variant == DTO_VAR_OCTET) P.analytic_fused = i + 1;
+    return DTO_OK;
+}
 
-    // ---- objectives --------------------------------------------------------------------------
-    h->obj_var_offs.resize(d->n_objectives);
-    h->obj_times.resize(d->n_objectives);
+// A knot term's variables and times, mapped to this handle's knots
+struct KnotTerm {
+    std::vector<int> all_offs;  // knot variable offsets, then global offsets
+    std::vector<int> g2l;       // global -> position in all_offs (-1: not read)
+    std::vector<int> own_ti;    // owned entries: position in the term's `times`
+    std::vector<int> own_knot;  //   and local knot
+    std::vector<int> k2o;       // local knot -> owned entry (-1: none)
+};
+
+// Validates the knot variables, global variables and listed times of a term.  `who` starts the messages about knot
+// variables and times, `gwho` those about global variables.
+static int parse_knot_term(const dto_handle* h, const dto_problem_desc* d, int n_vars, const int* var_offs, int n_gvars, const int* gvar_offs,
+                           int n_times, const int* times, const std::string& who, const std::string& gwho, KnotTerm& t) {
+    t.all_offs.assign(var_offs, var_offs + n_vars);
+    t.g2l.assign(h->P.gl.G, -1);
+    for (int v = 0; v < n_gvars; ++v) {
+        const int go = gvar_offs[v];
+        if (go < 0 || go >= h->P.gl.G) return reject(DTO_ERR_INVALID, gwho + ": variable outside global_data");
+        if (t.g2l[go] >= 0) return reject(DTO_ERR_UNSUPPORTED, gwho + ": repeated global variable");
+        t.g2l[go] = n_vars + v;
+        t.all_offs.push_back(go);
+    }
+    for (int v = 0; v < n_vars; ++v) {
+        if (var_offs[v] < 0 || var_offs[v] >= d->z) return reject(DTO_ERR_INVALID, who + ": variable outside the knot");
+        for (int v2 = 0; v2 < v; ++v2)
+            if (var_offs[v2] == var_offs[v]) return reject(DTO_ERR_UNSUPPORTED, who + ": repeated variable");
+    }
+    t.k2o.assign(h->P.nK, -1);
+    for (int j = 0; j < n_times; ++j) {
+        const int k = times[j];
+        if (k < 1 || k > d->N) return reject(DTO_ERR_INVALID, who + ": time index outside 1..N");
+        if (k < h->k0 || k > h->k1) continue;
+        if (t.k2o[k - h->k0] >= 0) return reject(DTO_ERR_UNSUPPORTED, who + ": repeated time index");
+        t.k2o[k - h->k0] = (int)t.own_ti.size();
+        t.own_ti.push_back(j);
+        t.own_knot.push_back(k - h->k0);
+    }
+    return DTO_OK;
+}
+
+static int build_objectives(dto_handle* h, const dto_problem_desc* d) {
+    DProb& P = h->P;
     for (int i = 0; i < d->n_objectives; ++i) {
         const dto_objective_desc& s = d->objectives[i];
-        h->objs.push_back(s);
         DObj& O = P.ob[i];
         O.kind = s.kind;
         O.fn = s.fn;
@@ -707,71 +742,53 @@ extern "C" int dto_create(const dto_problem_desc* d, dto_handle** out) {
         O.D = s.D;
         if (s.kind == DTO_OBJ_MINTIME || s.kind == DTO_OBJ_NULL) continue;
         if (s.kind != DTO_OBJ_QUADREG && s.kind != DTO_OBJ_KNOT && s.kind != DTO_OBJ_LINREG && s.kind != DTO_OBJ_GLOBAL_KNOT)
-            return fail_create(h, DTO_ERR_UNSUPPORTED, "unknown objective kind");
+            return reject(DTO_ERR_UNSUPPORTED, "unknown objective kind");
         const bool with_globals = s.kind == DTO_OBJ_GLOBAL_KNOT;
-        const bool program = with_programs && s.fn == DTO_L_PROGRAM;
+        const bool program = d->abi_version >= 4 && s.fn == DTO_L_PROGRAM;
         if ((s.kind == DTO_OBJ_KNOT || with_globals) && !knot_lfun_known(s.fn) && !program)
-            return fail_create(h, DTO_ERR_UNSUPPORTED, "knot objective function is not in the device catalogue");
+            return reject(DTO_ERR_UNSUPPORTED, "knot objective function is not in the device catalogue");
         const int ngv = with_globals ? s.n_gvars : 0;
         if (s.n_vars < (with_globals ? 0 : 1) || s.n_vars + ngv > DTO_MAX_KNOTFN_VARS || (s.n_vars > 0 && !s.var_offs))
-            return fail_create(h, DTO_ERR_INVALID, "objective: bad variable list");
-        if (with_globals && (ngv < 1 || !s.gvar_offs)) return fail_create(h, DTO_ERR_INVALID, "global objective: missing global variable list");
-        std::vector<int> all_offs(s.var_offs, s.var_offs + s.n_vars), g2l(G, -1);
-        for (int v = 0; v < ngv; ++v) {
-            const int go = s.gvar_offs[v];
-            if (go < 0 || go >= G) return fail_create(h, DTO_ERR_INVALID, "global objective: variable outside global_data");
-            if (g2l[go] >= 0) return fail_create(h, DTO_ERR_UNSUPPORTED, "global objective: repeated global variable");
-            g2l[go] = s.n_vars + v;
-            all_offs.push_back(go);
-        }
+            return reject(DTO_ERR_INVALID, "objective: bad variable list");
+        if (with_globals && (ngv < 1 || !s.gvar_offs)) return reject(DTO_ERR_INVALID, "global objective: missing global variable list");
+        KnotTerm t;
+        const int rc = parse_knot_term(h, d, s.n_vars, s.var_offs, ngv, s.gvar_offs, s.n_times, s.times, "objective", "global objective", t);
+        if (rc != DTO_OK) return rc;
         O.nv = s.n_vars + ngv;
-        for (int v = 0; v < s.n_vars; ++v) {
-            if (s.var_offs[v] < 0 || s.var_offs[v] >= z) return fail_create(h, DTO_ERR_INVALID, "objective: variable outside the knot");
-            for (int v2 = 0; v2 < v; ++v2)
-                if (s.var_offs[v2] == s.var_offs[v]) return fail_create(h, DTO_ERR_UNSUPPORTED, "objective: repeated variable");
-        }
-        std::vector<int> k2o(P.nK, -1), own, ownk;
-        for (int t = 0; t < s.n_times; ++t) {
-            const int k = s.times[t];
-            if (k < 1 || k > N) return fail_create(h, DTO_ERR_INVALID, "objective: time index outside 1..N");
-            if (k >= h->k0 && k <= h->k1) {
-                if (k2o[k - h->k0] >= 0) return fail_create(h, DTO_ERR_UNSUPPORTED, "objective: repeated time index");
-                k2o[k - h->k0] = (int)own.size();
-                own.push_back(t);
-                ownk.push_back(k - h->k0);
-            }
-        }
-        O.var_offs = dev_upload(h, all_offs.data(), all_offs.size());
-        O.g2l = with_globals ? dev_upload(h, g2l.data(), g2l.size()) : nullptr;
-        O.own_ti = dev_upload(h, own.data(), own.size());
-        O.own_knot = dev_upload(h, ownk.data(), ownk.size());
-        O.nt_own = (int)own.size();
-        O.own_kmin = ownk.empty() ? 0 : *std::min_element(ownk.begin(), ownk.end());
-        O.own_kmax = ownk.empty() ? -1 : *std::max_element(ownk.begin(), ownk.end());
-        O.knot_to_own = dev_upload(h, k2o.data(), k2o.size());
+        O.var_offs = dev_upload(h, t.all_offs.data(), t.all_offs.size());
+        O.g2l = with_globals ? dev_upload(h, t.g2l.data(), t.g2l.size()) : nullptr;
+        O.own_ti = dev_upload(h, t.own_ti.data(), t.own_ti.size());
+        O.own_knot = dev_upload(h, t.own_knot.data(), t.own_knot.size());
+        O.nt_own = (int)t.own_ti.size();
+        O.own_kmin = t.own_knot.empty() ? 0 : *std::min_element(t.own_knot.begin(), t.own_knot.end());
+        O.own_kmax = t.own_knot.empty() ? -1 : *std::max_element(t.own_knot.begin(), t.own_knot.end());
+        O.knot_to_own = dev_upload(h, t.k2o.data(), t.k2o.size());
         if (s.kind == DTO_OBJ_QUADREG || s.kind == DTO_OBJ_LINREG) {
-            if (!s.R) return fail_create(h, DTO_ERR_INVALID, "regularizer: missing R");
+            if (!s.R) return reject(DTO_ERR_INVALID, "regularizer: missing R");
             for (int v = 0; v < s.n_vars; ++v)
-                if (s.var_offs[v] == d->dt_off) return fail_create(h, DTO_ERR_UNSUPPORTED, "regularizer on the timestep component itself is not supported");
+                if (s.var_offs[v] == d->dt_off) return reject(DTO_ERR_UNSUPPORTED, "regularizer on the timestep component itself is not supported");
             O.R = dev_upload(h, s.R, s.n_vars);
-            O.baseline = (s.kind == DTO_OBJ_QUADREG && s.baseline) ? dev_upload(h, s.baseline, (size_t)s.n_vars * N) : nullptr;
+            O.baseline = (s.kind == DTO_OBJ_QUADREG && s.baseline) ? dev_upload(h, s.baseline, (size_t)s.n_vars * d->N) : nullptr;
         } else {
-            if (!s.Qs || (s.n_params > 0 && !s.params)) return fail_create(h, DTO_ERR_INVALID, "knot objective: missing Qs/params");
+            if (!s.Qs || (s.n_params > 0 && !s.params)) return reject(DTO_ERR_INVALID, "knot objective: missing Qs/params");
             O.params = dev_upload(h, s.params, (size_t)std::max(1, s.n_params) * s.n_times);
             O.Qs = dev_upload(h, s.Qs, s.n_times);
             if (program) {
-                const int rc = upload_knot_program(h, d, s.program, O.nv, s.n_params, 1, O.prog);
-                if (rc != DTO_OK) return rc;
+                const int prc = upload_knot_program(h, d, s.program, O.nv, s.n_params, 1, O.prog);
+                if (prc != DTO_OK) return prc;
             }
         }
     }
+    return DTO_OK;
+}
 
-    P.hess_tab = nullptr;
+static int build_hessian_tables(dto_handle* h, const dto_problem_desc* d, int smem_optin) {
+    DProb& P = h->P;
     if (d->eval_hessian) {  // stream-out gather table of the Hessian assembler (assemble.cu), knots with cross rows
         const size_t need = hessian_assemble_smem_bytes(P);
         if (need > (size_t)smem_optin)
-            return fail_create(h, DTO_ERR_UNSUPPORTED, smem_msg("Hessian assembly of a knot of " + std::to_string(P.z) + " variables" +
-                                                                (P.any_cross ? " coupled to its neighbour" : ""), need));
+            return reject(DTO_ERR_UNSUPPORTED, smem_msg("Hessian assembly of a knot of " + std::to_string(P.z) + " variables" +
+                                                            (P.any_cross ? " coupled to its neighbour" : ""), need, smem_optin));
         const int zz = P.z;
         std::vector<unsigned int> tab((size_t)zz * zz + (size_t)zz * (zz + 1) / 2);
         size_t e = 0;
@@ -781,320 +798,302 @@ extern "C" int dto_create(const dto_problem_desc* d, dto_handle** out) {
         }
         P.hess_tab = dev_upload(h, tab.data(), tab.size());
     }
-    {   // knot objectives: room for their Hessian pairs (assemble.cu: knot_objective_pairs_kernel)
-        long long off = 0;
-        for (int i = 0; i < d->n_objectives; ++i) {
-            DObj& O = P.ob[i];
-            O.side_off = off;
-            if ((O.kind == DTO_OBJ_KNOT || O.kind == DTO_OBJ_GLOBAL_KNOT) && O.nvk > 0) off += (long long)O.nt_own * (O.nvk * (O.nvk + 1) / 2);
-        }
-        P.side_stride = off;
-        P.knot_side = nullptr;
-        if (off > 0 && d->eval_hessian) {
-            P.knot_side = dev_upload<double>(h, nullptr, (size_t)off * (size_t)std::max(1, d->batch));
-            if (!P.knot_side) return fail_create(h, DTO_ERR_CUDA, "out of device memory (knot objective pairs)");
-        }
+    // knot objectives: room for their Hessian pairs (assemble.cu: knot_objective_pairs_kernel)
+    long long off = 0;
+    for (int i = 0; i < d->n_objectives; ++i) {
+        DObj& O = P.ob[i];
+        O.side_off = off;
+        if ((O.kind == DTO_OBJ_KNOT || O.kind == DTO_OBJ_GLOBAL_KNOT) && O.nvk > 0) off += (long long)O.nt_own * (O.nvk * (O.nvk + 1) / 2);
     }
+    P.side_stride = off;
+    if (off > 0 && d->eval_hessian) P.knot_side = dev_upload<double>(h, nullptr, (size_t)off * (size_t)std::max(1, d->batch));
+    return DTO_OK;
+}
 
-    // ---- knot constraints ----------------------------------------------------------------------
+static int build_constraints(dto_handle* h, const dto_problem_desc* d, long long n_dyn_local, std::vector<std::vector<int>>& con_own_knot,
+                             long long& n_nl_global) {
+    DProb& P = h->P;
     h->con_own_ti.resize(d->n_constraints);
+    h->con_times.resize(d->n_constraints);
+    con_own_knot.resize(d->n_constraints);
     long long cgoff = 0, cloff = n_dyn_local;
-    std::vector<std::vector<int>> con_own_knot(d->n_constraints);
     for (int i = 0; i < d->n_constraints; ++i) {
         const dto_constraint_desc& s = d->constraints[i];
-        h->cons.push_back(s);
-        const bool program = with_programs && s.fn == DTO_G_PROGRAM;
-        if (!knot_cfun_known(s.fn) && !program)
-            return fail_create(h, DTO_ERR_UNSUPPORTED, "knot constraint function is not in the device catalogue");
+        const bool program = d->abi_version >= 4 && s.fn == DTO_G_PROGRAM;
+        if (!knot_cfun_known(s.fn) && !program) return reject(DTO_ERR_UNSUPPORTED, "knot constraint function is not in the device catalogue");
         const int ngv = s.n_gvars;
         if (ngv < 0 || s.n_vars < 0 || s.n_vars + ngv < 1 || s.n_vars + ngv > DTO_MAX_KNOTFN_VARS || s.g_dim < 1 || s.g_dim > 16 ||
             (s.n_vars > 0 && !s.var_offs) || (ngv > 0 && !s.gvar_offs))
-            return fail_create(h, DTO_ERR_INVALID, "constraint: bad variable list or g_dim");
+            return reject(DTO_ERR_INVALID, "constraint: bad variable list or g_dim");
         if (s.fn == DTO_G_NORM_PRODUCT) {
-            if (s.g_dim != 2 || s.n_params < 3) return fail_create(h, DTO_ERR_INVALID, "constraint: norm_product has g_dim 2 and 3 parameters");
+            if (s.g_dim != 2 || s.n_params < 3) return reject(DTO_ERR_INVALID, "constraint: norm_product has g_dim 2 and 3 parameters");
         } else if (s.fn != DTO_G_LINEAR && !program && s.g_dim != 1)
-            return fail_create(h, DTO_ERR_INVALID, "constraint: g_dim must be 1 for this function");
-        std::vector<int> all_offs(s.var_offs, s.var_offs + s.n_vars), g2l(G, -1);
-        for (int v = 0; v < ngv; ++v) {
-            const int go = s.gvar_offs[v];
-            if (go < 0 || go >= G) return fail_create(h, DTO_ERR_INVALID, "constraint: variable outside global_data");
-            if (g2l[go] >= 0) return fail_create(h, DTO_ERR_UNSUPPORTED, "constraint: repeated global variable");
-            g2l[go] = s.n_vars + v;
-            all_offs.push_back(go);
-        }
-        h->con_var_offs.push_back(all_offs);
-        if (!d->Z0) return fail_create(h, DTO_ERR_INVALID, "knot constraints need the initial trajectory Z0 (stored Jacobian pattern)");
-        for (int v = 0; v < s.n_vars; ++v) {
-            if (s.var_offs[v] < 0 || s.var_offs[v] >= z) return fail_create(h, DTO_ERR_INVALID, "constraint: variable outside the knot");
-            for (int v2 = 0; v2 < v; ++v2)
-                if (s.var_offs[v2] == s.var_offs[v]) return fail_create(h, DTO_ERR_UNSUPPORTED, "constraint: repeated variable");
-        }
+            return reject(DTO_ERR_INVALID, "constraint: g_dim must be 1 for this function");
+        if (!d->Z0) return reject(DTO_ERR_INVALID, "knot constraints need the initial trajectory Z0 (stored Jacobian pattern)");
+        KnotTerm t;
+        const int rc = parse_knot_term(h, d, s.n_vars, s.var_offs, ngv, s.gvar_offs, s.n_times, s.times, "constraint", "constraint", t);
+        if (rc != DTO_OK) return rc;
         DCon& C = P.co[i];
         C.fn = s.fn;
         C.nv = s.n_vars + ngv;
         C.nvk = s.n_vars;
         C.gd = s.g_dim;
         C.np = s.n_params;
-        std::vector<int> k2o(P.nK, -1);
-        for (int t = 0; t < s.n_times; ++t) {
-            const int k = s.times[t];
-            if (k < 1 || k > N) return fail_create(h, DTO_ERR_INVALID, "constraint: time index outside 1..N");
-            if (k >= h->k0 && k <= h->k1) {
-                if (k2o[k - h->k0] >= 0) return fail_create(h, DTO_ERR_UNSUPPORTED, "constraint: repeated time index");
-                k2o[k - h->k0] = (int)h->con_own_ti[i].size();
-                h->con_own_ti[i].push_back(t);
-                con_own_knot[i].push_back(k - h->k0);
-            }
-        }
-        C.nt_own = (int)h->con_own_ti[i].size();
+        C.nt_own = (int)t.own_ti.size();
         C.row_off = cloff;
-        C.var_offs = dev_upload(h, all_offs.data(), all_offs.size());
-        C.g2l = ngv > 0 ? dev_upload(h, g2l.data(), g2l.size()) : nullptr;
-        C.own_ti = dev_upload(h, h->con_own_ti[i].data(), h->con_own_ti[i].size());
-        C.own_knot = dev_upload(h, con_own_knot[i].data(), con_own_knot[i].size());
-        C.knot_to_own = dev_upload(h, k2o.data(), k2o.size());
+        C.var_offs = dev_upload(h, t.all_offs.data(), t.all_offs.size());
+        C.g2l = ngv > 0 ? dev_upload(h, t.g2l.data(), t.g2l.size()) : nullptr;
+        C.own_ti = dev_upload(h, t.own_ti.data(), t.own_ti.size());
+        C.own_knot = dev_upload(h, t.own_knot.data(), t.own_knot.size());
+        C.knot_to_own = dev_upload(h, t.k2o.data(), t.k2o.size());
         C.params = dev_upload(h, s.params, (size_t)std::max(1, s.n_params) * s.n_times);
         if (program) {
-            if (s.n_params > 0 && !s.params) return fail_create(h, DTO_ERR_INVALID, "constraint: missing params");
-            const int rc = upload_knot_program(h, d, s.program, C.nv, s.n_params, s.g_dim, C.prog);
-            if (rc != DTO_OK) return rc;
+            if (s.n_params > 0 && !s.params) return reject(DTO_ERR_INVALID, "constraint: missing params");
+            const int prc = upload_knot_program(h, d, s.program, C.nv, s.n_params, s.g_dim, C.prog);
+            if (prc != DTO_OK) return prc;
         }
+        h->con_var_offs.push_back(std::move(t.all_offs));
+        h->con_own_ti[i] = std::move(t.own_ti);
+        con_own_knot[i] = std::move(t.own_knot);
+        h->con_times[i].assign(s.times, s.times + s.n_times);
         h->con_goff.push_back(cgoff);
         cgoff += (long long)s.g_dim * s.n_times;
         cloff += (long long)s.g_dim * C.nt_own;
     }
-    const long long n_nl_global = cgoff;
+    n_nl_global = cgoff;
     P.n_cons_local = cloff;
+    return DTO_OK;
+}
 
-    // ---- stored pattern of the knot-constraint Jacobians at Z0 (problem 0) ---------------------
-    // Evaluated over ALL times (a shard needs the whole pattern to know global positions) with the
-    // same device templates that later produce the values.
+// every listed time of constraint i: positions 0.. in its `times` and their 0-based knots
+static void all_times(const dto_handle* h, int i, std::vector<int>& ti, std::vector<int>& knot) {
+    const std::vector<int>& times = h->con_times[i];
+    ti.resize(times.size());
+    knot.resize(times.size());
+    for (size_t t = 0; t < times.size(); ++t) {
+        ti[t] = (int)t;
+        knot[t] = times[t] - 1;
+    }
+}
+
+// ---- stored pattern of the knot-constraint Jacobians at Z0 (problem 0) ---------------------
+// Evaluated over ALL times (a shard needs the whole pattern to know global positions) with the same device templates
+// that later produce the values.
+static int probe_constraint_pattern(dto_handle* h, const dto_problem_desc* d) {
+    const DProb& P = h->P;
+    const int N = d->N;
     h->con_stored_all.resize(d->n_constraints);
-    if (d->n_constraints > 0) {
-        DProb Q = P;  // whole-trajectory view for the probe
-        Q.batch = 1;
-        Q.kb = 1;
-        Q.nK = N;
-        Q.nOwn = N;
-        Q.nI = N - 1;
-        Q.n_vars_local = (long long)N * z + G;
-        Q.halo = nullptr;
-        double* dZ0 = dev_upload(h, d->Z0, (size_t)N * z + G);
-        long long total = 0;
-        std::vector<void*> tmp;
-        for (int i = 0; i < d->n_constraints; ++i) {
-            const dto_constraint_desc& s = d->constraints[i];
-            std::vector<int> all_ti(s.n_times), all_k(s.n_times);
-            for (int t = 0; t < s.n_times; ++t) {
-                all_ti[t] = t;
-                all_k[t] = s.times[t] - 1;
-            }
-            DCon& C = Q.co[i];
-            C.nt_own = s.n_times;
-            C.own_ti = dev_upload(h, all_ti.data(), all_ti.size());
-            C.own_knot = dev_upload(h, all_k.data(), all_k.size());
-            total += (long long)s.n_times * s.g_dim * (s.n_vars + s.n_gvars);
-        }
-        double* dprobe = dev_upload<double>(h, nullptr, (size_t)std::max<long long>(total, 1));
-        launch_constraint_pattern_probe(Q, dZ0, dprobe, h->stream, &h->launches);
-        std::vector<double> probe((size_t)total);
-        if (cudaMemcpyAsync(probe.data(), dprobe, sizeof(double) * total, cudaMemcpyDeviceToHost, h->stream) != cudaSuccess ||
-            cudaStreamSynchronize(h->stream) != cudaSuccess)
-            return fail_create(h, DTO_ERR_CUDA, std::string("constraint pattern probe failed: ") + cudaGetErrorString(cudaGetLastError()));
-        long long off = 0;
-        for (int i = 0; i < d->n_constraints; ++i) {
-            const dto_constraint_desc& s = d->constraints[i];
-            const long long cnt = (long long)s.n_times * s.g_dim * (s.n_vars + s.n_gvars);
-            h->con_stored_all[i].resize((size_t)cnt);
-            // SparseArrays' scalar setindex! does not store a zero value (either sign)
-            for (long long e = 0; e < cnt; ++e) h->con_stored_all[i][(size_t)e] = probe[(size_t)(off + e)] != 0.0 ? 1 : 0;
-            off += cnt;
-        }
-    }
-
-    // ---- local Jacobian column pointers and constraint scatter maps ----------------------------
-    // local column of variable v of constraint i at local knot kl: a knot column, or one of the G columns after them
-    auto con_col = [&](int i, int v, int kl) -> size_t {
-        return v < P.co[i].nvk ? (size_t)kl * z + h->con_var_offs[i][v] : (size_t)P.nK * z + h->con_var_offs[i][v];
-    };
-    std::vector<long long> ccount((size_t)P.nK * z + G, 0);
+    if (d->n_constraints == 0) return DTO_OK;
+    DProb Q = P;  // whole-trajectory view for the probe
+    Q.batch = 1;
+    Q.kb = 1;
+    Q.nK = N;
+    Q.nOwn = N;
+    Q.nI = N - 1;
+    Q.n_vars_local = (long long)N * d->z + h->P.gl.G;
+    Q.halo = nullptr;
+    double* dZ0 = dev_upload(h, d->Z0, (size_t)N * d->z + h->P.gl.G);
+    long long total = 0;
     for (int i = 0; i < d->n_constraints; ++i) {
-        const dto_constraint_desc& s = d->constraints[i];
-        const int nv = P.co[i].nv;
-        for (size_t j = 0; j < h->con_own_ti[i].size(); ++j) {
-            const int ti = h->con_own_ti[i][j], kl = con_own_knot[i][j];
-            for (int v = 0; v < nv; ++v)
-                for (int a = 0; a < s.g_dim; ++a)
-                    if (h->con_stored_all[i][((size_t)ti * s.g_dim + a) * nv + v]) ccount[con_col(i, v, kl)]++;
-        }
+        std::vector<int> all_ti, all_k;
+        all_times(h, i, all_ti, all_k);
+        DCon& C = Q.co[i];
+        C.nt_own = (int)all_ti.size();
+        C.own_ti = dev_upload(h, all_ti.data(), all_ti.size());
+        C.own_knot = dev_upload(h, all_k.data(), all_k.size());
+        total += (long long)C.nt_own * C.gd * C.nv;
     }
-    h->jac_colptr.assign((size_t)P.nK * z + G + 1, 0);
-    for (int kl = 0; kl < P.nK; ++kl) {
-        const long long per_col_int = (long long)P.Dsum * ((kl >= 1 ? 1 : 0) + (kl < P.nI ? 1 : 0));
-        for (int l = 0; l < z; ++l) {
-            const size_t c = (size_t)kl * z + l;
-            h->jac_colptr[c + 1] = h->jac_colptr[c] + per_col_int + ccount[c];
-        }
+    double* dprobe = dev_upload<double>(h, nullptr, (size_t)std::max<long long>(total, 1));
+    if (h->upload_failed) return reject(DTO_ERR_ALLOC, "device allocation failed (constraint pattern probe)");
+    launch_constraint_pattern_probe(Q, dZ0, dprobe, h->stream, &h->launches);
+    std::vector<double> probe((size_t)total);
+    if (cudaMemcpyAsync(probe.data(), dprobe, sizeof(double) * total, cudaMemcpyDeviceToHost, h->stream) != cudaSuccess ||
+        cudaStreamSynchronize(h->stream) != cudaSuccess)
+        return reject(DTO_ERR_CUDA, std::string("constraint pattern probe failed: ") + cudaGetErrorString(cudaGetLastError()));
+    long long off = 0;
+    for (int i = 0; i < d->n_constraints; ++i) {
+        const long long cnt = (long long)Q.co[i].nt_own * Q.co[i].gd * Q.co[i].nv;
+        h->con_stored_all[i].resize((size_t)cnt);
+        // SparseArrays' scalar setindex! does not store a zero value (either sign)
+        for (long long e = 0; e < cnt; ++e) h->con_stored_all[i][(size_t)e] = probe[(size_t)(off + e)] != 0.0 ? 1 : 0;
+        off += cnt;
     }
-    // global columns hold constraint entries only (integrators do not read globals: _integrators.jl:54-58)
-    for (int gi = 0; gi < G; ++gi) {
-        const size_t c = (size_t)P.nK * z + gi;
-        h->jac_colptr[c + 1] = h->jac_colptr[c] + ccount[c];
-    }
+    return DTO_OK;
+}
+
+// Jacobian rows of the integrators in a knot column: Dsum per adjacent interval (knots 0..n_own - 1 begin one)
+static long long interval_rows(const DProb& P, int k, int n_own) { return (long long)P.Dsum * ((k >= 1 ? 1 : 0) + (k < n_own ? 1 : 0)); }
+
+// f(j, a, v, column) for the stored Jacobian entries of constraint i at its entries ti[j] on knots knot[j] of a window of
+// nk knots, in position order; a knot variable's column is knot * z + offset, global gi's nk * z + gi
+template <class F>
+static void for_each_stored(const dto_handle* h, int i, const std::vector<int>& ti, const std::vector<int>& knot, int nk, F&& f) {
+    const DCon& C = h->P.co[i];
+    const std::vector<int>& offs = h->con_var_offs[i];
+    const std::vector<unsigned char>& stored = h->con_stored_all[i];
+    for (size_t j = 0; j < ti.size(); ++j)
+        for (int v = 0; v < C.nv; ++v)
+            for (int a = 0; a < C.gd; ++a)
+                if (stored[((size_t)ti[j] * C.gd + a) * C.nv + v])
+                    f(j, a, v, v < C.nvk ? (size_t)knot[j] * h->P.z + offs[v] : (size_t)nk * h->P.z + offs[v]);
+}
+
+// Jacobian column pointers over a window of nk knots (the first n_own begin an interval), then the global columns, which
+// hold constraint entries only (integrators do not read globals: _integrators.jl:54-58)
+static std::vector<long long> jac_column_pointers(const dto_handle* h, const std::vector<std::vector<int>>& ti,
+                                                  const std::vector<std::vector<int>>& knot, int nk, int n_own) {
+    const DProb& P = h->P;
+    const size_t knot_cols = (size_t)nk * P.z, cols = knot_cols + h->P.gl.G;
+    std::vector<long long> ptr(cols + 1, 0);
+    for (int i = 0; i < P.n_con; ++i) for_each_stored(h, i, ti[i], knot[i], nk, [&](size_t, int, int, size_t c) { ptr[c + 1]++; });
+    for (size_t c = 0; c < cols; ++c) ptr[c + 1] += ptr[c] + (c < knot_cols ? interval_rows(P, (int)(c / P.z), n_own) : 0);
+    return ptr;
+}
+
+// local Jacobian column pointers and the constraint scatter maps
+static void build_jacobian_layout(dto_handle* h, const std::vector<std::vector<int>>& con_own_knot, long long n_dyn_global) {
+    DProb& P = h->P;
+    const size_t knot_cols = (size_t)P.nK * P.z;
+    h->jac_colptr = jac_column_pointers(h, h->con_own_ti, con_own_knot, P.nK, P.nI);
     P.nnz_jac_local = h->jac_colptr.back();
     P.jac_colptr = dev_upload(h, h->jac_colptr.data(), h->jac_colptr.size());
-    P.jac_closed = h->con_entries.empty() && d->n_constraints == 0 ? 1 : 0;
-    {
-        std::vector<long long> fill((size_t)P.nK * z + G, 0);
-        for (int i = 0; i < d->n_constraints; ++i) {
+    P.jac_closed = P.n_con == 0 ? 1 : 0;
+    std::vector<long long> next(h->jac_colptr.size() - 1);  // position of the next constraint entry of each column
+    for (size_t c = 0; c < next.size(); ++c) next[c] = h->jac_colptr[c] + (c < knot_cols ? interval_rows(P, (int)(c / P.z), P.nI) : 0);
+    for (int i = 0; i < P.n_con; ++i) {
+        DCon& C = P.co[i];
+        std::vector<long long> pos((size_t)C.nt_own * C.gd * C.nv, -1);
+        for_each_stored(h, i, h->con_own_ti[i], con_own_knot[i], P.nK, [&](size_t j, int a, int v, size_t c) {
+            const long long p = next[c]++;
+            pos[(j * C.gd + a) * C.nv + v] = p;
+            const long long ti = h->con_own_ti[i][j];
+            h->con_entries.push_back(ConEntry{(long long)c, n_dyn_global + h->con_goff[i] + ti * C.gd + a, p});
+        });
+        C.jac_pos = dev_upload(h, pos.data(), pos.size());
+    }
+    std::stable_sort(h->con_entries.begin(), h->con_entries.end(), [](const ConEntry& a, const ConEntry& b) { return a.e < b.e; });
+}
+
+// one listed time of a term with global variables: objective or constraint index, entry of its `times`, 0-based knot,
+// knot variables, knot + global variables, knot and global offsets
+struct GlobSlot {
+    int term, j, kl, nvk, nv;
+    const int *koffs, *goffs;
+};
+
+// ---- terms with global variables: slots, Hessian tail (the global columns) -----------------------
+// Pattern: objective terms mark the dense [knot vars; globals]^2 block of every listed time
+// (global_objectives.jl:268-291); constraint terms store what their Hessian at Z0 with mu = ones holds
+// (evaluator.jl:168-171, global_knot_point_constraint.jl:205-249).  Upper triangle: a global column holds the
+// coupled knot rows in ascending order, then the coupled global rows up to its own.
+static int build_global_terms(dto_handle* h, const dto_problem_desc* d) {
+    DProb& P = h->P;
+    const int G = h->P.gl.G, N = d->N, z = d->z;
+    if (G == 0) return DTO_OK;
+    DGlob& L = P.gl;
+    std::vector<GlobSlot> slots;
+    int KV = 0;
+    for (int i = 0; i < d->n_objectives; ++i)
+        if (P.ob[i].kind == DTO_OBJ_GLOBAL_KNOT) {
+            const dto_objective_desc& s = d->objectives[i];
+            KV = std::max(KV, P.ob[i].nvk);
+            for (int t = 0; t < s.n_times; ++t)  // not sharded: owned entry == position in `times`
+                slots.push_back(GlobSlot{i, t, s.times[t] - 1, P.ob[i].nvk, P.ob[i].nv, s.var_offs, s.gvar_offs});
+        }
+    L.S_obj = (int)slots.size();
+    for (int i = 0; i < d->n_constraints; ++i)
+        if (P.co[i].nv > P.co[i].nvk) {
             const dto_constraint_desc& s = d->constraints[i];
-            DCon& C = P.co[i];
-            const int nv = C.nv;
-            std::vector<long long> pos((size_t)C.nt_own * s.g_dim * nv, -1);
-            for (size_t j = 0; j < h->con_own_ti[i].size(); ++j) {
-                const int ti = h->con_own_ti[i][j], kl = con_own_knot[i][j];
-                for (int v = 0; v < nv; ++v)
-                    for (int a = 0; a < s.g_dim; ++a) {
-                        if (!h->con_stored_all[i][((size_t)ti * s.g_dim + a) * nv + v]) continue;
-                        const size_t c = con_col(i, v, kl);
-                        const long long per_col_int = v < C.nvk ? (long long)P.Dsum * ((kl >= 1 ? 1 : 0) + (kl < P.nI ? 1 : 0)) : 0;
-                        const long long e = ((long long)j * s.g_dim + a) * nv + v;
-                        const long long p = h->jac_colptr[c] + per_col_int + fill[c]++;
-                        pos[(size_t)e] = p;
-                        ConEntry ce;
-                        ce.col_local = (long long)c;
-                        ce.grow = n_dyn_global + h->con_goff[i] + (long long)ti * s.g_dim + a;
-                        ce.lrow = C.row_off + (long long)j * s.g_dim + a;
-                        ce.e = p;  // local position
-                        ce.ci = i;
-                        h->con_entries.push_back(ce);
-                    }
-            }
-            C.jac_pos = dev_upload(h, pos.data(), pos.size());
+            KV = std::max(KV, P.co[i].nvk);
+            for (int t = 0; t < s.n_times; ++t) slots.push_back(GlobSlot{i, t, s.times[t] - 1, P.co[i].nvk, P.co[i].nv, s.var_offs, s.gvar_offs});
         }
-        std::stable_sort(h->con_entries.begin(), h->con_entries.end(),
-                         [](const ConEntry& a, const ConEntry& b) { return a.e < b.e; });
+    L.S = (int)slots.size();
+    L.KV = KV;
+    const int gtri = G * (G + 1) / 2;
+    if (L.S > 0) {
+        std::vector<int> slot_term, slot_j;
+        for (const GlobSlot& s : slots) {
+            slot_term.push_back(s.term);
+            slot_j.push_back(s.j);
+        }
+        L.slot_term = dev_upload(h, slot_term.data(), slot_term.size());
+        L.slot_j = dev_upload(h, slot_j.data(), slot_j.size());
+        if (L.S_obj > 0) L.scratchG = dev_upload<double>(h, nullptr, (size_t)P.batch * L.S_obj * G);
+        L.scratchH = dev_upload<double>(h, nullptr, (size_t)P.batch * L.S * gtri);
     }
-
-    // ---- terms with global variables: slots, Hessian tail (the global columns) -----------------------
-    // Pattern: objective terms mark the dense [knot vars; globals]^2 block of every listed time
-    // (global_objectives.jl:268-291); constraint terms store what their Hessian at Z0 with mu = ones holds
-    // (evaluator.jl:168-171, global_knot_point_constraint.jl:205-249).  Upper triangle: a global column holds the
-    // coupled knot rows in ascending order, then the coupled global rows up to its own.
-    if (G > 0) {
-        DGlob& L = P.gl;
-        std::vector<int> slot_term, slot_j, slot_kl;
-        int KV = 0;
-        for (int i = 0; i < d->n_objectives; ++i)
-            if (P.ob[i].kind == DTO_OBJ_GLOBAL_KNOT) {
-                KV = std::max(KV, P.ob[i].nvk);
-                for (int t = 0; t < d->objectives[i].n_times; ++t) {  // not sharded: owned entry == position in `times`
-                    slot_term.push_back(i);
-                    slot_j.push_back(t);
-                    slot_kl.push_back(d->objectives[i].times[t] - 1);
-                }
+    std::vector<double> kg_probe((size_t)L.S * std::max(KV, 1) * G, 0.0), gg_probe;
+    if (L.S > L.S_obj) {  // constraint Hessians at Z0, mu = ones, through the same device templates
+        DProb Q = P;
+        Q.batch = 1;
+        double* dZ0 = dev_upload(h, d->Z0, (size_t)N * z + G);
+        double* dprobe = dev_upload<double>(h, nullptr, kg_probe.size());
+        if (h->upload_failed) return reject(DTO_ERR_ALLOC, "device allocation failed (global Hessian pattern probe)");
+        launch_global_hessian(Q, h->kg, dZ0, 1.0, nullptr, nullptr, dprobe, h->stream, &h->launches);
+        gg_probe.resize((size_t)L.S * gtri);
+        if (cudaMemcpyAsync(kg_probe.data(), dprobe, sizeof(double) * kg_probe.size(), cudaMemcpyDeviceToHost, h->stream) != cudaSuccess ||
+            cudaMemcpyAsync(gg_probe.data(), L.scratchH, sizeof(double) * gg_probe.size(), cudaMemcpyDeviceToHost, h->stream) != cudaSuccess ||
+            cudaStreamSynchronize(h->stream) != cudaSuccess)
+            return reject(DTO_ERR_CUDA, std::string("global Hessian pattern probe failed: ") + cudaGetErrorString(cudaGetLastError()));
+    }
+    auto pair_index = [&](int gi, int gj) { return gi * G - gi * (gi - 1) / 2 + (gj - gi); };  // gi <= gj
+    std::vector<std::pair<long long, long long>>& tail = h->hess_tail;
+    for (int sl = 0; sl < L.S; ++sl) {
+        const GlobSlot& s = slots[sl];
+        const bool dense = sl < L.S_obj;  // objective terms: the whole block
+        for (int v = s.nvk; v < s.nv; ++v) {
+            const int gi = s.goffs[v - s.nvk];
+            for (int a = 0; a < s.nvk; ++a)
+                if (dense || kg_probe[((size_t)sl * KV + a) * G + gi] != 0.0) tail.emplace_back((long long)gi, (long long)s.kl * z + s.koffs[a]);
+            for (int v2 = s.nvk; v2 < s.nv; ++v2) {
+                const int g2 = s.goffs[v2 - s.nvk];
+                if (g2 > gi) continue;
+                if (dense || gg_probe[(size_t)sl * gtri + pair_index(g2, gi)] != 0.0) tail.emplace_back((long long)gi, (long long)N * z + g2);
             }
-        L.S_obj = (int)slot_term.size();
-        for (int i = 0; i < d->n_constraints; ++i)
-            if (P.co[i].nv > P.co[i].nvk) {
-                KV = std::max(KV, P.co[i].nvk);
-                for (int t = 0; t < d->constraints[i].n_times; ++t) {
-                    slot_term.push_back(i);
-                    slot_j.push_back(t);
-                    slot_kl.push_back(d->constraints[i].times[t] - 1);
-                }
-            }
-        L.S = (int)slot_term.size();
-        L.KV = KV;
-        const int gtri = G * (G + 1) / 2;
-        if (L.S > 0) {
-            L.slot_term = dev_upload(h, slot_term.data(), slot_term.size());
-            L.slot_j = dev_upload(h, slot_j.data(), slot_j.size());
-            if (L.S_obj > 0) L.scratchG = dev_upload<double>(h, nullptr, (size_t)P.batch * L.S_obj * G);
-            L.scratchH = dev_upload<double>(h, nullptr, (size_t)P.batch * L.S * gtri);
-            if (!L.slot_term || !L.slot_j || !L.scratchH || (L.S_obj > 0 && !L.scratchG))
-                return fail_create(h, DTO_ERR_ALLOC, "device allocation failed (global terms)");
-        }
-        std::vector<double> kg_probe((size_t)L.S * std::max(KV, 1) * G, 0.0), gg_probe;
-        if (L.S > L.S_obj) {  // constraint Hessians at Z0, mu = ones, through the same device templates
-            if (!d->Z0) return fail_create(h, DTO_ERR_INVALID, "constraints need the initial trajectory Z0 (stored pattern)");
-            DProb Q = P;
-            Q.batch = 1;
-            double* dZ0 = dev_upload(h, d->Z0, (size_t)N * z + G);
-            double* dprobe = dev_upload<double>(h, nullptr, kg_probe.size());
-            launch_global_hessian(Q, h->kg, dZ0, 1.0, nullptr, nullptr, dprobe, h->stream, &h->launches);
-            gg_probe.resize((size_t)L.S * gtri);
-            if (cudaMemcpyAsync(kg_probe.data(), dprobe, sizeof(double) * kg_probe.size(), cudaMemcpyDeviceToHost, h->stream) != cudaSuccess ||
-                cudaMemcpyAsync(gg_probe.data(), L.scratchH, sizeof(double) * gg_probe.size(), cudaMemcpyDeviceToHost, h->stream) != cudaSuccess ||
-                cudaStreamSynchronize(h->stream) != cudaSuccess)
-                return fail_create(h, DTO_ERR_CUDA, std::string("global Hessian pattern probe failed: ") + cudaGetErrorString(cudaGetLastError()));
-        }
-        auto pair_index = [&](int gi, int gj) { return gi * G - gi * (gi - 1) / 2 + (gj - gi); };  // gi <= gj
-        std::vector<std::pair<long long, long long>>& tail = h->hess_tail;
-        for (int sl = 0; sl < L.S; ++sl) {
-            const bool is_obj = sl < L.S_obj;
-            const int ti = slot_term[sl];
-            const int nvk = is_obj ? P.ob[ti].nvk : P.co[ti].nvk, nv = is_obj ? P.ob[ti].nv : P.co[ti].nv;
-            const int* koffs = is_obj ? d->objectives[ti].var_offs : d->constraints[ti].var_offs;
-            const int* goffs = is_obj ? d->objectives[ti].gvar_offs : d->constraints[ti].gvar_offs;
-            for (int v = nvk; v < nv; ++v) {
-                const int gi = goffs[v - nvk];
-                for (int a = 0; a < nvk; ++a)
-                    if (is_obj || kg_probe[((size_t)sl * KV + a) * G + gi] != 0.0)
-                        tail.emplace_back((long long)gi, (long long)slot_kl[sl] * z + koffs[a]);
-                for (int v2 = nvk; v2 < nv; ++v2) {
-                    const int g2 = goffs[v2 - nvk];
-                    if (g2 > gi) continue;
-                    if (is_obj || gg_probe[(size_t)sl * gtri + pair_index(g2, gi)] != 0.0) tail.emplace_back((long long)gi, (long long)N * z + g2);
-                }
-            }
-        }
-        std::sort(tail.begin(), tail.end());
-        tail.erase(std::unique(tail.begin(), tail.end()), tail.end());
-        auto find_pos = [&](long long gi, long long row) -> long long {
-            auto it = std::lower_bound(tail.begin(), tail.end(), std::make_pair(gi, row));
-            return (it != tail.end() && it->first == gi && it->second == row) ? (long long)(it - tail.begin()) : -1;
-        };
-        std::vector<long long> kg_pos((size_t)L.S * std::max(KV, 1) * G, -1), gg_pos((size_t)gtri, -1);
-        for (int sl = 0; sl < L.S; ++sl) {
-            const bool is_obj = sl < L.S_obj;
-            const int ti = slot_term[sl];
-            const int nvk = is_obj ? P.ob[ti].nvk : P.co[ti].nvk;
-            const int* koffs = is_obj ? d->objectives[ti].var_offs : d->constraints[ti].var_offs;
-            for (int a = 0; a < nvk; ++a)
-                for (int gi = 0; gi < G; ++gi) kg_pos[((size_t)sl * KV + a) * G + gi] = find_pos(gi, (long long)slot_kl[sl] * z + koffs[a]);
-        }
-        for (int gi = 0; gi < G; ++gi)
-            for (int gj = gi; gj < G; ++gj) gg_pos[(size_t)pair_index(gi, gj)] = find_pos(gj, (long long)N * z + gi);
-        L.kg_pos = dev_upload(h, kg_pos.data(), kg_pos.size());
-        L.gg_pos = dev_upload(h, gg_pos.data(), gg_pos.size());
-        L.n_hess_tail = (long long)tail.size();
-        // contributors of every (knot variable, global) tail entry in ascending slot order (e is slot-major): summed in
-        // this fixed order by kg_sum_kernel
-        std::vector<std::vector<long long>> contrib(tail.size());
-        for (size_t e = 0; e < (size_t)L.S * KV * G; ++e)
-            if (kg_pos[e] >= 0) contrib[(size_t)kg_pos[e]].push_back((long long)e);
-        std::vector<long long> kg_dst, kg_src;
-        std::vector<int> kg_ptr{0};
-        for (size_t p = 0; p < contrib.size(); ++p)
-            if (!contrib[p].empty()) {
-                kg_dst.push_back((long long)p);
-                kg_src.insert(kg_src.end(), contrib[p].begin(), contrib[p].end());
-                kg_ptr.push_back((int)kg_src.size());
-            }
-        DGlobKG& kg = h->kg;
-        kg.n = (int)kg_dst.size();
-        if (kg.n > 0) {
-            kg.dst = dev_upload(h, kg_dst.data(), kg_dst.size());
-            kg.ptr = dev_upload(h, kg_ptr.data(), kg_ptr.size());
-            kg.src = dev_upload(h, kg_src.data(), kg_src.size());
-            kg.scratch = dev_upload<double>(h, nullptr, (size_t)P.batch * L.S * KV * G);
-            if (!kg.dst || !kg.ptr || !kg.src || !kg.scratch)
-                return fail_create(h, DTO_ERR_ALLOC, "device allocation failed (global terms)");
         }
     }
+    std::sort(tail.begin(), tail.end());
+    tail.erase(std::unique(tail.begin(), tail.end()), tail.end());
+    auto find_pos = [&](long long gi, long long row) -> long long {
+        auto it = std::lower_bound(tail.begin(), tail.end(), std::make_pair(gi, row));
+        return (it != tail.end() && it->first == gi && it->second == row) ? (long long)(it - tail.begin()) : -1;
+    };
+    std::vector<long long> kg_pos((size_t)L.S * std::max(KV, 1) * G, -1), gg_pos((size_t)gtri, -1);
+    for (int sl = 0; sl < L.S; ++sl)
+        for (int a = 0; a < slots[sl].nvk; ++a)
+            for (int gi = 0; gi < G; ++gi) kg_pos[((size_t)sl * KV + a) * G + gi] = find_pos(gi, (long long)slots[sl].kl * z + slots[sl].koffs[a]);
+    for (int gi = 0; gi < G; ++gi)
+        for (int gj = gi; gj < G; ++gj) gg_pos[(size_t)pair_index(gi, gj)] = find_pos(gj, (long long)N * z + gi);
+    L.kg_pos = dev_upload(h, kg_pos.data(), kg_pos.size());
+    L.gg_pos = dev_upload(h, gg_pos.data(), gg_pos.size());
+    L.n_hess_tail = (long long)tail.size();
+    // contributors of every (knot variable, global) tail entry in ascending slot order (e is slot-major): summed in
+    // this fixed order by kg_sum_kernel
+    std::vector<std::vector<long long>> contrib(tail.size());
+    for (size_t e = 0; e < (size_t)L.S * KV * G; ++e)
+        if (kg_pos[e] >= 0) contrib[(size_t)kg_pos[e]].push_back((long long)e);
+    std::vector<long long> kg_dst, kg_src;
+    std::vector<int> kg_ptr{0};
+    for (size_t p = 0; p < contrib.size(); ++p)
+        if (!contrib[p].empty()) {
+            kg_dst.push_back((long long)p);
+            kg_src.insert(kg_src.end(), contrib[p].begin(), contrib[p].end());
+            kg_ptr.push_back((int)kg_src.size());
+        }
+    DGlobKG& kg = h->kg;
+    kg.n = (int)kg_dst.size();
+    if (kg.n > 0) {
+        kg.dst = dev_upload(h, kg_dst.data(), kg_dst.size());
+        kg.ptr = dev_upload(h, kg_ptr.data(), kg_ptr.size());
+        kg.src = dev_upload(h, kg_src.data(), kg_src.size());
+        kg.scratch = dev_upload<double>(h, nullptr, (size_t)P.batch * L.S * KV * G);
+    }
+    return DTO_OK;
+}
 
-    // ---- sizes -----------------------------------------------------------------------------------
+// sizes of this shard and of the whole problem, and the equality flags of the local rows
+static void set_sizes(dto_handle* h, const dto_problem_desc* d, long long n_dyn_global, long long n_dyn_local, long long n_nl_global) {
+    DProb& P = h->P;
+    const int N = d->N, z = d->z, G = h->P.gl.G;
     const long long tri = (long long)z * (z + 1) / 2;
     P.gl.hess_tail_off = hess_knot_base(P, P.nOwn);  // base of the knot after the last owned one
     P.nnz_hess_local = P.gl.hess_tail_off + P.gl.n_hess_tail;
@@ -1108,28 +1107,22 @@ extern "C" int dto_create(const dto_problem_desc* d, dto_handle** out) {
     h->sizes_global.n_dynamics_cons = n_dyn_global;
     h->sizes_global.n_nonlinear_cons = n_nl_global;
     h->sizes_global.n_cons = n_dyn_global + n_nl_global;
-    {
-        long long stored = 0;
-        for (auto& m : h->con_stored_all)
-            for (unsigned char c : m) stored += c;
-        h->sizes_global.nnz_jac = (long long)(N - 1) * P.Dsum * 2 * z + stored;
-        h->sizes_global.nnz_hess = (long long)N * tri + (long long)(N - 1) * z * z + P.gl.n_hess_tail;
-    }
-
-    // equality flags of the local rows
+    long long stored = 0;
+    for (auto& m : h->con_stored_all)
+        for (unsigned char c : m) stored += c;
+    h->sizes_global.nnz_jac = (long long)(N - 1) * P.Dsum * 2 * z + stored;
+    h->sizes_global.nnz_hess = (long long)N * tri + (long long)(N - 1) * z * z + P.gl.n_hess_tail;
     h->row_is_eq.assign((size_t)P.n_cons_local, 1);
     for (int i = 0; i < d->n_constraints; ++i)
         if (!d->constraints[i].equality)
             for (long long r = 0; r < (long long)P.co[i].nt_own * P.co[i].gd; ++r) h->row_is_eq[(size_t)(P.co[i].row_off + r)] = 0;
     h->d_row_is_eq = dev_upload(h, h->row_is_eq.data(), h->row_is_eq.size());
+}
 
-    // keep host copies of small arrays the structure queries need
-    h->con_times.resize(d->n_constraints);
-    for (int i = 0; i < d->n_constraints; ++i) {
-        h->con_times[i].assign(d->constraints[i].times, d->constraints[i].times + d->constraints[i].n_times);
-    }
-
-    // ---- work buffers --------------------------------------------------------------------------
+// work buffers, the iterate cache, and the optional series plans and jets (without them the kernels size the series
+// from ||dt G(u)||_1 and recompute the jets)
+static int build_work_buffers(dto_handle* h, const dto_problem_desc* d) {
+    DProb& P = h->P;
     const size_t B = (size_t)P.batch;
     h->dZ = dev_upload<double>(h, nullptr, B * (size_t)P.n_vars_local);
     h->dmu = dev_upload<double>(h, nullptr, B * (size_t)std::max<long long>(P.n_cons_local, 1));
@@ -1140,155 +1133,183 @@ extern "C" int dto_create(const dto_problem_desc* d, dto_handle** out) {
     h->dviol = dev_upload<double>(h, nullptr, B);
     h->dpartials = dev_upload<double>(h, nullptr, B * ((size_t)P.nOwn + (size_t)(P.nOwn + 2047) / 2048));
     if (d->eval_hessian) h->dhess = dev_upload<double>(h, nullptr, B * (size_t)std::max<long long>(P.nnz_hess_local, 1));
-    if (!h->dZ || !h->dmu || !h->dg || !h->djac || !h->dgrad || !h->dJ || !h->dpartials || (d->eval_hessian && !h->dhess))
-        return fail_create(h, DTO_ERR_ALLOC, "device allocation failed (work buffers)");
-    {
-        // iterate cache: the page-locked host copy of the resident iterate
-        if (const char* tr = getenv("DTO_B200_TRACE")) h->trace = atoi(tr);
-        if (cudaHostAlloc((void**)&h->hZpin, sizeof(double) * B * (size_t)P.n_vars_local, cudaHostAllocDefault) != cudaSuccess) {
-            h->hZpin = nullptr;
-            return fail_create(h, DTO_ERR_ALLOC, "page-locked host allocation failed (iterate cache)");
-        }
-        bool ok = d->eval_hessian;
-        bool any = false;
+    if (const char* tr = getenv("DTO_B200_TRACE")) h->trace = atoi(tr);
+    // iterate cache: the page-locked host copy of the resident iterate
+    if (cudaHostAlloc((void**)&h->hZpin, sizeof(double) * B * (size_t)P.n_vars_local, cudaHostAllocDefault) != cudaSuccess) {
+        h->hZpin = nullptr;
+        return reject(DTO_ERR_ALLOC, "page-locked host allocation failed (iterate cache)");
+    }
+    // per-interval series plans of the bilinear interval kernels (series_plan.cu); DTO_B200_SERIES_PLAN=0: size the
+    // series from ||dt G(u)||_1 as round 1 did
+    const char* sp = getenv("DTO_B200_SERIES_PLAN");
+    if (!(sp && strcmp(sp, "0") == 0))
         for (int i = 0; i < P.n_int; ++i) {
-            if (P.in[i].kind == DTO_INT_DERIVATIVE) continue;
-            any = true;
-            ok = ok && P.in[i].kind == DTO_INT_BILINEAR && P.in[i].variant >= DTO_VAR_PERSISTENT;
+            DInt& I = P.in[i];
+            if (I.kind != DTO_INT_BILINEAR || I.variant < DTO_VAR_PERSISTENT) continue;
+            if (I.variant == DTO_VAR_OCTET) continue;  // n = 8 / 16: see DESIGN.md section 3
+            const dto_integrator_desc& sd = d->integrators[i];
+            if (sd.G_batch_stride != 0 || series_plan_smem(I.n, I.m) == 0) continue;  // shared sets that fit shared memory
+            std::vector<float> pm;
+            series_plan_matrices(I.n, I.m, sd.G, pm);
+            I.planmat = dev_upload(h, pm.data(), pm.size(), true);
+            I.plan = (const double2*)dev_upload<double>(h, nullptr, 2 * B * (size_t)std::max(P.nI, 1), true);
+            if (!I.plan || !I.planmat) I.plan = nullptr;
         }
-        {
-            // per-interval series plans of the bilinear interval kernels (series_plan.cu); DTO_B200_SERIES_PLAN=0: size the
-            // series from ||dt G(u)||_1 as round 1 did
-            const char* sp = getenv("DTO_B200_SERIES_PLAN");
-            if (!(sp && strcmp(sp, "0") == 0))
-                for (int i = 0; i < P.n_int; ++i) {
-                    DInt& I = P.in[i];
-                    if (I.kind != DTO_INT_BILINEAR || I.variant < DTO_VAR_PERSISTENT) continue;
-                    if (I.variant == DTO_VAR_OCTET) continue;  // n = 8 / 16: see DESIGN.md section 3
-                    const dto_integrator_desc& sd = d->integrators[i];
-                    if (sd.G_batch_stride != 0 || series_plan_smem(I.n, I.m) == 0) continue;  // shared sets that fit shared memory
-                    std::vector<float> pm;
-                    series_plan_matrices(I.n, I.m, sd.G, pm);
-                    I.planmat = dev_upload(h, pm.data(), pm.size());
-                    I.plan = (const double2*)dev_upload<double>(h, nullptr, 2 * B * (size_t)std::max(P.nI, 1));
-                    if (!I.plan || !I.planmat) {
-                        cudaGetLastError();
-                        I.plan = nullptr;
-                    }
-                }
-        }
-        if (ok && any) {
-            for (int i = 0; i < P.n_int && ok; ++i) {
-                DInt& I = P.in[i];
-                if (I.kind != DTO_INT_BILINEAR) continue;
-                I.jet_stride = (I.m * (I.m + 1) / 2 + 1 + 2 * I.m) * I.n;
-                I.jets = dev_upload<double>(h, nullptr, B * (size_t)std::max(P.nI, 1) * I.jet_stride);
-                ok = I.jets != nullptr;
-            }
-            if (!ok) cudaGetLastError();
-            h->jets_ok = ok;
-        }
+    bool ok = d->eval_hessian, any = false;
+    for (int i = 0; i < P.n_int; ++i) {
+        if (P.in[i].kind == DTO_INT_DERIVATIVE) continue;
+        any = true;
+        ok = ok && P.in[i].kind == DTO_INT_BILINEAR && P.in[i].variant >= DTO_VAR_PERSISTENT;
     }
-    {
-        // chunk boundaries of the host-pointer pipeline as cumulative fractions of the intervals.  The persistent interval
-        // kernel needs many items per warp to fill the FP64 pipe (one forward item alone takes ~100 us): two ranges; the
-        // octet kernel's items are small: four
-        bool persistent = false;
-        for (int i = 0; i < P.n_int; ++i) persistent |= P.in[i].kind == DTO_INT_BILINEAR && P.in[i].variant == DTO_VAR_PERSISTENT;
-        bool tdbi = false;
-        for (int i = 0; i < P.n_int; ++i) tdbi |= P.in[i].kind == DTO_INT_TDBILINEAR;
-        if (tdbi) {
-            // one CTA per SM works through the intervals of a range in rounds (~1 ms each at n = 64): boundaries at
-            // multiples of two full rounds, so that cutting costs no partial round (c3: 296 / 592 / 888 of 999)
-            int sms = 148;
-            cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, h->device);
-            for (int k = 2 * sms; k + sms / 2 < P.nI; k += 2 * sms) h->pipeline_fracs.push_back((k + 0.5) / (double)std::max(P.nI, 1));
-        } else if (persistent) h->pipeline_fracs = {0.5};
-        else h->pipeline_fracs = {0.1, 0.4, 0.7};
+    if (ok && any) {
+        for (int i = 0; i < P.n_int && ok; ++i) {
+            DInt& I = P.in[i];
+            if (I.kind != DTO_INT_BILINEAR) continue;
+            I.jet_stride = (I.m * (I.m + 1) / 2 + 1 + 2 * I.m) * I.n;
+            I.jets = dev_upload<double>(h, nullptr, B * (size_t)std::max(P.nI, 1) * I.jet_stride, true);
+            ok = I.jets != nullptr;
+        }
+        h->jets_ok = ok;
     }
+    return DTO_OK;
+}
+
+// the host-pointer path: pipeline cuts, structural-zero runs of the Hessian, constant heads of the Jacobian columns
+static void plan_host_path(dto_handle* h, const dto_problem_desc* d) {
+    DProb& P = h->P;
+    const int z = d->z;
+    // chunk boundaries of the host-pointer pipeline as cumulative fractions of the intervals.  The persistent interval
+    // kernel needs many items per warp to fill the FP64 pipe (one forward item alone takes ~100 us): two ranges; the
+    // octet kernel's items are small: four
+    bool persistent = false, tdbi = false;
+    for (int i = 0; i < P.n_int; ++i) persistent |= P.in[i].kind == DTO_INT_BILINEAR && P.in[i].variant == DTO_VAR_PERSISTENT;
+    for (int i = 0; i < P.n_int; ++i) tdbi |= P.in[i].kind == DTO_INT_TDBILINEAR;
+    if (tdbi) {
+        // one CTA per SM works through the intervals of a range in rounds (~1 ms each at n = 64): boundaries at
+        // multiples of two full rounds, so that cutting costs no partial round (c3: 296 / 592 / 888 of 999)
+        int sms = 148;
+        cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, h->device);
+        for (int k = 2 * sms; k + sms / 2 < P.nI; k += 2 * sms) h->pipeline_fracs.push_back((k + 0.5) / (double)std::max(P.nI, 1));
+    } else if (persistent) h->pipeline_fracs = {0.5};
+    else h->pipeline_fracs = {0.1, 0.4, 0.7};
     // ---- structural zeros of the Hessian (host-pointer path) -------------------------------------------------------
     // For bilinear/derivative problems every entry of a knot's region in a column below l0(k) is identically zero
     // (x enters the dynamics linearly: the cross block and the (x, x) block carry no term; SURVEY.md section 8a).
     // l0(k) = smallest column any term of the problem can write at knot k (column of a pair = its larger component).
-    {
-        bool ok = d->eval_hessian && d->batch == 1 && !P.any_cross && G == 0;
-        for (int i = 0; i < P.n_int; ++i) ok = ok && (P.in[i].kind == DTO_INT_BILINEAR || P.in[i].kind == DTO_INT_DERIVATIVE);
-        if (ok) {
-            int l_int = z;  // knots that own an interval
-            for (int i = 0; i < P.n_int; ++i) {
-                const dto_integrator_desc& s = d->integrators[i];
-                if (s.kind == DTO_INT_BILINEAR) {
-                    for (int p = 0; p <= s.u_dim; ++p) {
-                        const int c = p < s.u_dim ? s.u_off + p : d->dt_off;
-                        l_int = std::min(l_int, std::max(s.x_off, c));  // (x_a, param): smallest with a = 0
-                        l_int = std::min(l_int, c);                     // (param, param)
-                    }
-                } else {
-                    l_int = std::min(l_int, std::max(s.u_off, d->dt_off));  // (xdot_a, dt)
+    bool ok = d->eval_hessian && d->batch == 1 && !P.any_cross && h->P.gl.G == 0;
+    for (int i = 0; i < P.n_int; ++i) ok = ok && (P.in[i].kind == DTO_INT_BILINEAR || P.in[i].kind == DTO_INT_DERIVATIVE);
+    if (ok) {
+        int l_int = z;  // knots that own an interval
+        for (int i = 0; i < P.n_int; ++i) {
+            const dto_integrator_desc& s = d->integrators[i];
+            if (s.kind == DTO_INT_BILINEAR) {
+                for (int p = 0; p <= s.u_dim; ++p) {
+                    const int c = p < s.u_dim ? s.u_off + p : d->dt_off;
+                    l_int = std::min(l_int, std::max(s.x_off, c));  // (x_a, param): smallest with a = 0
+                    l_int = std::min(l_int, c);                     // (param, param)
                 }
-            }
-            std::vector<int> l0((size_t)P.nOwn, z);
-            for (int kl = 0; kl < P.nOwn; ++kl)
-                if (kl < P.nI) l0[kl] = l_int;
-            auto touch = [&](const int* times, int nt, int lmin) {
-                for (int t = 0; t < nt; ++t) {
-                    const int k = times[t];
-                    if (k >= h->k0 && k <= h->k1) l0[k - h->k0] = std::min(l0[k - h->k0], lmin);
-                }
-            };
-            for (int i = 0; i < d->n_objectives; ++i) {
-                const dto_objective_desc& s = d->objectives[i];
-                if (s.kind == DTO_OBJ_MINTIME || s.kind == DTO_OBJ_NULL) continue;
-                int lmin = z;
-                for (int v = 0; v < s.n_vars; ++v) lmin = std::min(lmin, s.var_offs[v]);
-                if (s.kind == DTO_OBJ_QUADREG || s.kind == DTO_OBJ_LINREG) lmin = std::min(lmin, d->dt_off);
-                touch(s.times, s.n_times, lmin);
-            }
-            for (int i = 0; i < d->n_constraints; ++i) {
-                const dto_constraint_desc& s = d->constraints[i];
-                int lmin = z;
-                for (int v = 0; v < s.n_vars; ++v) lmin = std::min(lmin, s.var_offs[v]);
-                touch(s.times, s.n_times, lmin);
-            }
-            long long zeros = 0;
-            for (int kl = 0; kl < P.nOwn; ++kl) {
-                const long long nc = hess_knot_has_cross(P, kl) ? z : 0;
-                const long long skip = (long long)l0[kl] * nc + (long long)l0[kl] * (l0[kl] + 1) / 2;
-                if (skip > 0) h->hess_zero_segs.emplace_back(hess_knot_base(P, kl), skip);
-                zeros += skip;
-                if (!h->hess_runs.empty() && h->hess_runs.back().l0 == l0[kl] &&
-                    hess_knot_has_cross(P, h->hess_runs.back().k0) == hess_knot_has_cross(P, kl))
-                    h->hess_runs.back().cnt++;
-                else
-                    h->hess_runs.push_back(HRun{kl, 1, l0[kl]});
-            }
-            // worth it only when most of the array is structural and the runs are long (few copies)
-            // host threads for the zero fill: at most 4, at most half the cores; with fewer than 3 the fill would be slower
-            // than the bus it relieves (one thread writes ~10 GB/s), so the whole array is delivered instead
-            int nth = (int)std::min<unsigned>(4, std::max(1u, std::thread::hardware_concurrency() / 2));
-            if (const char* e2 = getenv("DTO_B200_HOST_THREADS")) nth = std::max(1, std::min(32, atoi(e2)));
-            if (zeros * 2 < P.nnz_hess_local || h->hess_runs.size() > 64) {
-                h->hess_runs.clear();
-                h->hess_zero_segs.clear();
-            } else if (nth >= 3) {  // unregistered buffers need the fill threads; registered ones have their zeros in place
-                h->zero_fill = new (std::nothrow) ZeroFill();
-                if (h->zero_fill) h->zero_fill->start(nth);
+            } else {
+                l_int = std::min(l_int, std::max(s.u_off, d->dt_off));  // (xdot_a, dt)
             }
         }
+        std::vector<int> l0((size_t)P.nOwn, z);
+        for (int kl = 0; kl < P.nOwn; ++kl)
+            if (kl < P.nI) l0[kl] = l_int;
+        auto touch = [&](const int* times, int nt, int lmin) {
+            for (int t = 0; t < nt; ++t) {
+                const int k = times[t];
+                if (k >= h->k0 && k <= h->k1) l0[k - h->k0] = std::min(l0[k - h->k0], lmin);
+            }
+        };
+        for (int i = 0; i < d->n_objectives; ++i) {
+            const dto_objective_desc& s = d->objectives[i];
+            if (s.kind == DTO_OBJ_MINTIME || s.kind == DTO_OBJ_NULL) continue;
+            int lmin = z;
+            for (int v = 0; v < s.n_vars; ++v) lmin = std::min(lmin, s.var_offs[v]);
+            if (s.kind == DTO_OBJ_QUADREG || s.kind == DTO_OBJ_LINREG) lmin = std::min(lmin, d->dt_off);
+            touch(s.times, s.n_times, lmin);
+        }
+        for (int i = 0; i < d->n_constraints; ++i) {
+            const dto_constraint_desc& s = d->constraints[i];
+            int lmin = z;
+            for (int v = 0; v < s.n_vars; ++v) lmin = std::min(lmin, s.var_offs[v]);
+            touch(s.times, s.n_times, lmin);
+        }
+        long long zeros = 0;
+        for (int kl = 0; kl < P.nOwn; ++kl) {
+            const long long nc = hess_knot_has_cross(P, kl) ? z : 0;
+            const long long skip = (long long)l0[kl] * nc + (long long)l0[kl] * (l0[kl] + 1) / 2;
+            if (skip > 0) h->hess_zero_segs.emplace_back(hess_knot_base(P, kl), skip);
+            zeros += skip;
+            if (!h->hess_runs.empty() && h->hess_runs.back().l0 == l0[kl] &&
+                hess_knot_has_cross(P, h->hess_runs.back().k0) == hess_knot_has_cross(P, kl))
+                h->hess_runs.back().cnt++;
+            else
+                h->hess_runs.push_back(HRun{kl, 1, l0[kl]});
+        }
+        // worth it only when most of the array is structural and the runs are long (few copies)
+        // host threads for the zero fill: at most 4, at most half the cores; with fewer than 3 the fill would be slower
+        // than the bus it relieves (one thread writes ~10 GB/s), so the whole array is delivered instead
+        int nth = (int)std::min<unsigned>(4, std::max(1u, std::thread::hardware_concurrency() / 2));
+        if (const char* e2 = getenv("DTO_B200_HOST_THREADS")) nth = std::max(1, std::min(32, atoi(e2)));
+        if (zeros * 2 < P.nnz_hess_local || h->hess_runs.size() > 64) {
+            h->hess_runs.clear();
+            h->hess_zero_segs.clear();
+        } else if (nth >= 3) {  // unregistered buffers need the fill threads; registered ones have their zeros in place
+            h->zero_fill = new (std::nothrow) ZeroFill();
+            if (h->zero_fill) h->zero_fill->start(nth);
+        }
     }
-    {
-        // Jacobian: d r_{k-1} / d z_k of a bilinear or derivative integrator is the constant [0 .. I .. 0] block
-        // (bilinear_integrator.jl:81, derivative_integrator.jl:45: x_{k+1} enters linearly).  With one column layout for
-        // all inner knots (no knot-constraint rows) the rest of every column is one strided copy.  Only registered Jacobian
-        // arrays (dto_register_outputs) skip the heads: they get them once; an unregistered buffer would need them written
-        // on every call (74 000 small memsets at c2).
-        const int k0i = P.in[0].kind;
-        const long long L = 2LL * P.Dsum, d1 = P.in[0].n;
-        if (d->batch == 1 && P.jac_closed && G == 0 && P.nI >= 3 && (k0i == DTO_INT_BILINEAR || k0i == DTO_INT_DERIVATIVE) && 8 * (L - d1) >= 256)
-            h->jac_skip_ok = (int)d1;
+    // Jacobian: d r_{k-1} / d z_k of a bilinear or derivative integrator is the constant [0 .. I .. 0] block
+    // (bilinear_integrator.jl:81, derivative_integrator.jl:45: x_{k+1} enters linearly).  With one column layout for
+    // all inner knots (no knot-constraint rows) the rest of every column is one strided copy.  Only registered Jacobian
+    // arrays (dto_register_outputs) skip the heads: they get them once; an unregistered buffer would need them written
+    // on every call (74 000 small memsets at c2).
+    const int k0i = P.in[0].kind;
+    const long long L = 2LL * P.Dsum, d1 = P.in[0].n;
+    if (d->batch == 1 && P.jac_closed && h->P.gl.G == 0 && P.nI >= 3 && (k0i == DTO_INT_BILINEAR || k0i == DTO_INT_DERIVATIVE) && 8 * (L - d1) >= 256)
+        h->jac_skip_ok = (int)d1;
+}
+
+extern "C" int dto_create(const dto_problem_desc* d, dto_handle** out) {
+    if (!d || !out) return reject(DTO_ERR_INVALID, "null descriptor");
+    *out = nullptr;
+    int rc = check_header(d);
+    if (rc != DTO_OK) return rc;
+    int ndev = 0;
+    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) return reject(DTO_ERR_CUDA, "no CUDA device: libdto_b200 has no CPU fallback");
+    cudaGetLastError();  // do not inherit a stale error from an earlier, unrelated call
+    dto_handle* h = new (std::nothrow) dto_handle();
+    if (!h) return reject(DTO_ERR_ALLOC, "out of host memory");
+
+    int smem_optin = 0;                                            // shared memory per block (opt-in) of the device
+    long long n_dyn_global = 0, n_dyn_local = 0, n_nl_global = 0;  // dynamics rows (whole problem, shard), knot-constraint rows
+    std::vector<std::vector<int>> con_own_knot;                    // local knot of every owned entry of each constraint
+    rc = open_device(h, d, smem_optin);
+    if (rc == DTO_OK) rc = init_problem(h, d);
+    if (rc == DTO_OK) rc = build_integrators(h, d, smem_optin, n_dyn_global, n_dyn_local);
+    if (rc == DTO_OK) rc = build_objectives(h, d);
+    if (rc == DTO_OK) rc = build_hessian_tables(h, d, smem_optin);
+    if (rc == DTO_OK) rc = build_constraints(h, d, n_dyn_local, con_own_knot, n_nl_global);
+    if (rc == DTO_OK) rc = probe_constraint_pattern(h, d);
+    if (rc == DTO_OK) {
+        build_jacobian_layout(h, con_own_knot, n_dyn_global);
+        rc = build_global_terms(h, d);
     }
-    if (cudaStreamSynchronize(h->stream) != cudaSuccess || cudaGetLastError() != cudaSuccess)
-        return fail_create(h, DTO_ERR_CUDA, "CUDA failure during construction");
+    if (rc == DTO_OK) {
+        set_sizes(h, d, n_dyn_global, n_dyn_local, n_nl_global);
+        rc = build_work_buffers(h, d);
+    }
+    if (rc == DTO_OK) {
+        plan_host_path(h, d);
+        if (h->upload_failed) rc = reject(DTO_ERR_ALLOC, "device allocation failed");
+        else if (cudaStreamSynchronize(h->stream) != cudaSuccess || cudaGetLastError() != cudaSuccess)
+            rc = reject(DTO_ERR_CUDA, "CUDA failure during construction");
+    }
+    if (rc != DTO_OK) {
+        dto_destroy(h);
+        return rc;
+    }
     *out = h;
     return DTO_OK;
 }
@@ -1341,7 +1362,7 @@ extern "C" int dto_jac_structure(const dto_handle* h, int64_t* rows, int64_t* co
             }
         }
     }
-    for (int gi = 0; gi < h->G; ++gi)  // global columns: constraint rows only
+    for (int gi = 0; gi < h->P.gl.G; ++gi)  // global columns: constraint rows only
         while (ce < h->con_entries.size() && h->con_entries[ce].col_local == (long long)P.nK * z + gi) {
             rows[w] = h->con_entries[ce].grow + 1;
             cols[w] = (long long)P.N * z + gi + 1;
@@ -1402,27 +1423,16 @@ extern "C" int dto_shard_maps(const dto_handle* h, int64_t* con_rows, int64_t* j
         for (int i = 0; i < P.n_int; ++i)
             for (int kl = 0; kl < P.nI; ++kl)
                 for (int a = 0; a < P.in[i].n; ++a) con_rows[w++] = h->int_goff[i] + ((long long)P.kb - 1 + kl) * P.in[i].n + a;
-        for (size_t i = 0; i < h->cons.size(); ++i)
+        for (int i = 0; i < P.n_con; ++i)
             for (int ti : h->con_own_ti[i])
-                for (int a = 0; a < h->cons[i].g_dim; ++a)
-                    con_rows[w++] = h->sizes_global.n_dynamics_cons + h->con_goff[i] + (long long)ti * h->cons[i].g_dim + a;
+                for (int a = 0; a < P.co[i].gd; ++a)
+                    con_rows[w++] = h->sizes_global.n_dynamics_cons + h->con_goff[i] + (long long)ti * P.co[i].gd + a;
     }
     if (jac_pos) {
         // global column pointers from the all-times stored pattern
-        std::vector<long long> gcount((size_t)N * z, 0);
-        for (size_t i = 0; i < h->cons.size(); ++i) {
-            const dto_constraint_desc& s = h->cons[i];
-            for (int t = 0; t < s.n_times; ++t)
-                for (int v = 0; v < s.n_vars; ++v)
-                    for (int a = 0; a < s.g_dim; ++a)
-                        if (h->con_stored_all[i][((size_t)t * s.g_dim + a) * s.n_vars + v])
-                            gcount[(size_t)(h->con_times[i][t] - 1) * z + h->con_var_offs[i][v]]++;
-        }
-        std::vector<long long> gptr((size_t)N * z + 1, 0);
-        for (int k = 0; k < N; ++k) {
-            const long long per = (long long)P.Dsum * ((k >= 1 ? 1 : 0) + (k < N - 1 ? 1 : 0));
-            for (int l = 0; l < z; ++l) gptr[(size_t)k * z + l + 1] = gptr[(size_t)k * z + l] + per + gcount[(size_t)k * z + l];
-        }
+        std::vector<std::vector<int>> ti(P.n_con), knot(P.n_con);
+        for (int i = 0; i < P.n_con; ++i) all_times(h, i, ti[i], knot[i]);
+        const std::vector<long long> gptr = jac_column_pointers(h, ti, knot, N, N - 1);
         long long w = 0;
         size_t ce = 0;
         for (int kl = 0; kl < P.nK; ++kl) {
@@ -1439,7 +1449,7 @@ extern "C" int dto_shard_maps(const dto_handle* h, int64_t* con_rows, int64_t* j
                     if (kl < P.nI)
                         for (int a = 0; a < dd; ++a) jac_pos[w++] = own_start + a;
                 }
-                const long long per = (long long)P.Dsum * ((gprev ? 1 : 0) + (gown ? 1 : 0));
+                const long long per = interval_rows(P, (int)kg, N - 1);
                 long long r = 0;
                 while (ce < h->con_entries.size() && h->con_entries[ce].col_local == (long long)kl * z + l) {
                     jac_pos[w++] = base + per + r++;

@@ -302,11 +302,9 @@ bool launch_bilinear_product(const DProb& P, int ii, const double* Z, const doub
                              long long* launches);
 void launch_analytic_product(const DProb& P, const double* Z, const double* w, double* y, bool transpose, cudaStream_t st,
                              long long* launches);
-void bilinear_persistent_swizzled(int n, int m, const double* Grm, double* out);
 size_t series_plan_smem(int n, int m);
 void series_plan_matrices(int n, int m, const double* Gcm, std::vector<float>& out);
 bool launch_series_plan(const DProb& P, int ii, const double* Z, cudaStream_t st, long long* launches);
-bool tdb_available();
 bool tdb_dmma_supported(const DInt& I);
 bool launch_tdb_dmma(const DProb& P, int ii, const double* Z, const double* mu, double* g, double* jac, EvalFlags f, cudaStream_t st,
                      long long* launches);

@@ -404,7 +404,6 @@ size_t tdb_smem_bytes(const DInt& I, bool want_jac, bool want_hess) {
 
 }  // namespace
 
-bool tdb_available() { return true; }
 
 void launch_tdb(const DProb& P, int ii, const double* Z, const double* mu, double* g, double* jac, EvalFlags f, cudaStream_t st,
                 long long* launches) {
