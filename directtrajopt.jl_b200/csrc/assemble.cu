@@ -764,6 +764,24 @@ size_t hessian_assemble_smem_bytes(const DProb& P) {
     return hessian_assemble_plan(P, W);
 }
 
+template <int GS, bool PROG>
+static bool configure_assemble(bool left_block, std::string& err) {
+    const std::string args = "<" + std::to_string(GS) + (PROG ? ", true>" : ", false>");
+    return opt_in_smem(hessian_assemble_kernel<GS, PROG>, 227 * 1024, "hessian_assemble_kernel" + args, err) &&
+           (!left_block || opt_in_smem(hessian_assemble_left_kernel<GS, PROG>, 227 * 1024, "hessian_assemble_left_kernel" + args, err));
+}
+
+// the form launch_hessian_assemble picks for this problem, and its left-knot form if the handle launches it
+bool hessian_assemble_configure(const DProb& P, bool left_block, std::string& err) {
+    if (hessian_assemble_smem_bytes(P) <= 48 * 1024) return true;
+    const int GS = P.z <= 16 ? 8 : (P.z <= 24 ? 16 : 32);
+    if (any_program_constraint(P))
+        return GS == 8 ? configure_assemble<8, true>(left_block, err)
+                       : (GS == 16 ? configure_assemble<16, true>(left_block, err) : configure_assemble<32, true>(left_block, err));
+    return GS == 8 ? configure_assemble<8, false>(left_block, err)
+                   : (GS == 16 ? configure_assemble<16, false>(left_block, err) : configure_assemble<32, false>(left_block, err));
+}
+
 void launch_hessian_assemble(const DProb& P, const double* Z, double sigma, const double* mu, double* hess, cudaStream_t st,
                              long long* launches, bool left_block) {
     const int nKc = std::min(P.kc1, P.nOwn) - P.kc0;
@@ -771,21 +789,6 @@ void launch_hessian_assemble(const DProb& P, const double* Z, double sigma, cons
     const int GS = P.z <= 16 ? 8 : (P.z <= 24 ? 16 : 32), GPW = 32 / GS;
     int W;
     const size_t smem = hessian_assemble_plan(P, W);
-    static PerDeviceOnce configured;
-    if (smem > 48 * 1024 && configured.first()) {
-        cudaFuncSetAttribute(hessian_assemble_kernel<32, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
-        cudaFuncSetAttribute(hessian_assemble_kernel<16, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
-        cudaFuncSetAttribute(hessian_assemble_kernel<8, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
-        cudaFuncSetAttribute(hessian_assemble_kernel<32, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
-        cudaFuncSetAttribute(hessian_assemble_kernel<16, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
-        cudaFuncSetAttribute(hessian_assemble_kernel<8, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
-        cudaFuncSetAttribute(hessian_assemble_left_kernel<32, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
-        cudaFuncSetAttribute(hessian_assemble_left_kernel<16, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
-        cudaFuncSetAttribute(hessian_assemble_left_kernel<8, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
-        cudaFuncSetAttribute(hessian_assemble_left_kernel<32, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
-        cudaFuncSetAttribute(hessian_assemble_left_kernel<16, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
-        cudaFuncSetAttribute(hessian_assemble_left_kernel<8, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
-    }
     const long long total = (long long)nKc * P.batch;
     const unsigned grid = (unsigned)((total + (long long)W * GPW - 1) / ((long long)W * GPW));
     if (left_block) {  // local knot 0 only (kc0 = 0, kc1 = 1)

@@ -487,7 +487,7 @@ __global__ void __launch_bounds__(128) bilinear_dmma_kernel(DProb P, int ii, con
 }
 
 template <int NT, int MT>
-bool launch_variant(const DProb& P, int ii, const double* Z, const double* mu, double* g, double* jac, EvalFlags f, cudaStream_t st,
+void launch_variant(const DProb& P, int ii, const double* Z, const double* mu, double* g, double* jac, EvalFlags f, cudaStream_t st,
                     long long* launches) {
     const DInt& I = P.in[ii];
     const int n = 8 * NT, ld = dmma_ld(n);
@@ -495,18 +495,12 @@ bool launch_variant(const DProb& P, int ii, const double* Z, const double* mu, d
     const size_t shared_part = sizeof(double) * (size_t)I.m * n * ld;
     int W = 4;
     while (W > 1 && shared_part + W * per_warp > 100 * 1024) W >>= 1;
-    const size_t smem = shared_part + W * per_warp;
-    if (smem > 227 * 1024) return false;
+    const size_t smem = shared_part + W * per_warp;  // at most 182.5 KB (n = 64, m = 4, W = 1)
     auto kern = bilinear_dmma_kernel<NT, MT>;
-    static PerDeviceOnce configured;
-    if (configured.first()) {
-        if (cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024) != cudaSuccess) return false;
-    }
     const int cpp = (P.nI + W - 1) / W;
     dim3 grid((unsigned)(cpp * P.batch), 1 + (f.want_jac ? 1 : 0) + (f.want_hess ? 1 : 0));
     kern<<<grid, W * 32, smem, st>>>(P, ii, Z, mu, f.want_g ? g : nullptr, jac, f.want_jac ? 1 : 0, f.want_hess ? 1 : 0, W, cpp);
     ++*launches;
-    return true;
 }
 
 }  // namespace
@@ -516,26 +510,22 @@ bool bilinear_dmma_supported(int n, int m) {
     return n == 8 || n == 16 || n == 24 || n == 32 || n == 48 || n == 64;
 }
 
-bool launch_bilinear_dmma(const DProb& P, int ii, const double* Z, const double* mu, double* g, double* jac, EvalFlags f,
+bool bilinear_dmma_configure(int n, std::string& err) {
+    return with_nt(n, [&](auto nt) {
+        constexpr int NT = decltype(nt)::value;
+        return opt_in_smem(bilinear_dmma_kernel<NT, 1>, 227 * 1024, "bilinear_dmma_kernel<" + std::to_string(NT) + ", 1>", err) &&
+               opt_in_smem(bilinear_dmma_kernel<NT, 2>, 227 * 1024, "bilinear_dmma_kernel<" + std::to_string(NT) + ", 2>", err);
+    });
+}
+
+void launch_bilinear_dmma(const DProb& P, int ii, const double* Z, const double* mu, double* g, double* jac, EvalFlags f,
                           cudaStream_t st, long long* launches) {
     const DInt& I = P.in[ii];
-    if (P.nI <= 0) return true;
-    if (!bilinear_dmma_supported(I.n, I.m)) return false;
+    if (P.nI <= 0) return;
     const int nrows = f.want_hess ? 1 + I.m + I.m * (I.m + 1) / 2 : 1 + I.m;
-    const bool two = nrows > 8;
     // MT is the number of 8-row tiles of the forward role; the EXP role uses the same MT per chunk
-#define DTO_DISPATCH(NTv)                                                                                      \
-    case NTv:                                                                                                  \
-        return two ? launch_variant<NTv, 2>(P, ii, Z, mu, g, jac, f, st, launches)                             \
-                   : launch_variant<NTv, 1>(P, ii, Z, mu, g, jac, f, st, launches);
-    switch (I.n / 8) {
-        DTO_DISPATCH(1)
-        DTO_DISPATCH(2)
-        DTO_DISPATCH(3)
-        DTO_DISPATCH(4)
-        DTO_DISPATCH(6)
-        DTO_DISPATCH(8)
-    }
-#undef DTO_DISPATCH
-    return false;
+    with_nt(I.n, [&](auto nt) {
+        if (nrows > 8) launch_variant<decltype(nt)::value, 2>(P, ii, Z, mu, g, jac, f, st, launches);
+        else launch_variant<decltype(nt)::value, 1>(P, ii, Z, mu, g, jac, f, st, launches);
+    });
 }

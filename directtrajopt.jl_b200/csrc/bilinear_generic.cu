@@ -247,15 +247,15 @@ size_t generic_smem_bytes(int n, int m, bool want_jac, bool want_hess) {
     return sizeof(double) * ((size_t)(n | 1) * n + 3 * (size_t)ncol * n + 3 * n);
 }
 
+bool bilinear_generic_configure(int n, int m, std::string& err) {
+    return generic_smem_bytes(n, m, true, true) <= 48 * 1024 || opt_in_smem(bilinear_generic_kernel, 227 * 1024, "bilinear_generic_kernel", err);
+}
+
 void launch_bilinear_generic(const DProb& P, int ii, const double* Z, const double* mu, double* g, double* jac, EvalFlags f,
                              cudaStream_t st, long long* launches) {
     const DInt& I = P.in[ii];
     if (P.nI <= 0) return;
     size_t smem = generic_smem_bytes(I.n, I.m, f.want_jac, f.want_hess);
-    static PerDeviceOnce configured;
-    if (smem > 48 * 1024 && configured.first()) {
-        cudaFuncSetAttribute(bilinear_generic_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
-    }
     bilinear_generic_kernel<<<P.nI * P.batch, 32, smem, st>>>(P, ii, Z, mu, f.want_g ? g : nullptr, jac, f.want_jac ? 1 : 0,
                                                                f.want_hess ? 1 : 0);
     ++*launches;

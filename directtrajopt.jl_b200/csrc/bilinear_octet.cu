@@ -656,15 +656,12 @@ __global__ void __launch_bounds__(NT == 1 ? 256 : 128, (NT == 1 && M <= 2) ? 2 :
 }
 
 template <int NT, int M, bool PP>
-bool launch_octet_pp(const DProb& P, int ii, const double* Z, const double* mu, double* g, double* jac, EvalFlags f, cudaStream_t st,
-                     long long* launches) {
+void launch_octet_pp(const DProb& P, int ii, const double* Z, const double* mu, double* g, double* jac, EvalFlags f, int split,
+                     cudaStream_t st, long long* launches) {
     constexpr int n = 8 * NT;
-    const size_t smem = PP ? 0 : sizeof(double) * (size_t)(M + 1) * n * n + sizeof(double2) * (size_t)2 * (M + 1) * NT * NT * 32;
+    constexpr size_t smem = PP ? 0 : sizeof(double) * (size_t)(M + 1) * n * n + sizeof(double2) * (size_t)2 * (M + 1) * NT * NT * 32;
+    static_assert(smem <= 48 * 1024, "the octet kernel is launched without opting into more than 48 KB of shared memory");
     auto kern = bilinear_octet_kernel<NT, M, PP>;
-    static PerDeviceOnce configured;
-    if (smem > 48 * 1024 && configured.first()) {
-        if (cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess) return false;
-    }
     int dev = 0, sms = 148;
     cudaGetDevice(&dev);
     cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
@@ -675,7 +672,6 @@ bool launch_octet_pp(const DProb& P, int ii, const double* Z, const double* mu, 
     const long long octs = PP ? (long long)P.batch * ((nIc + 7) / 8) : (items + 7) / 8, wpc = threads / 32;
     const int nPh = (f.jets != DTO_JETS_USE ? 1 : 0) + (f.want_jac ? 1 : 0) + (f.want_hess ? 1 : 0);
     const long long resident = (long long)std::max(1, sms - P.reserve_sms) * per_sm * wpc;  // warps in flight
-    const char* env = getenv("DTO_B200_OCTET_SPLIT");           // A/B switch: 0 = whole octets only, 1 = every octet in phases
     // Three forms: whole octets only; every octet in phases (a third of the granularity, but ~8 % (n = 16) / ~20 % (n = 8)
     // slower per octet); whole rounds of whole octets and the remainder in phases.  Measured (tools/c4_size_sweep.py,
     // tools/c5_batch_sweep.py): with two or more complete rounds the third form wins or ties everywhere (c5 on one to
@@ -687,7 +683,7 @@ bool launch_octet_pp(const DProb& P, int ii, const double* Z, const double* mu, 
     const long long full = (long long)floor(rounds) * resident;  // octets of the complete rounds
     long long n_whole = octs;
     if (nPh > 1) {
-        if (env) n_whole = env[0] == '1' ? 0 : octs;
+        if (split >= 0) n_whole = split ? 0 : octs;
         else if (rounds >= 2.0) n_whole = full < octs ? full : octs;
         else if (idle(rounds) - idle(rounds * nPh) > 0.1) n_whole = 0;
     }
@@ -695,17 +691,13 @@ bool launch_octet_pp(const DProb& P, int ii, const double* Z, const double* mu, 
     const int grid = (int)std::max<long long>(1, std::min<long long>((long long)std::max(1, sms - P.reserve_sms) * per_sm, (units + wpc - 1) / wpc));
     kern<<<grid, threads, smem, st>>>(P, ii, Z, mu, f.want_g ? g : nullptr, jac, f.want_jac ? 1 : 0, f.want_hess ? 1 : 0, f.jets, n_whole);
     ++*launches;
-    return true;
 }
 
 template <int NT, int M>
-bool launch_octet(const DProb& P, int ii, const double* Z, const double* mu, double* g, double* jac, EvalFlags f, cudaStream_t st,
-                  long long* launches) {
-    if (P.in[ii].G_stride != 0) {
-        if (P.in[ii].bfrag == nullptr) return false;
-        return launch_octet_pp<NT, M, true>(P, ii, Z, mu, g, jac, f, st, launches);
-    }
-    return launch_octet_pp<NT, M, false>(P, ii, Z, mu, g, jac, f, st, launches);
+void launch_octet(const DProb& P, int ii, const double* Z, const double* mu, double* g, double* jac, EvalFlags f, int split,
+                  cudaStream_t st, long long* launches) {
+    if (P.in[ii].G_stride != 0) launch_octet_pp<NT, M, true>(P, ii, Z, mu, g, jac, f, split, st, launches);
+    else launch_octet_pp<NT, M, false>(P, ii, Z, mu, g, jac, f, split, st, launches);
 }
 
 }  // namespace
@@ -731,24 +723,21 @@ bool bilinear_octet_supported(int n, int m) {
     return false;
 }
 
-bool launch_bilinear_octet(const DProb& P, int ii, const double* Z, const double* mu, double* g, double* jac, EvalFlags f,
+void launch_bilinear_octet(const DProb& P, int ii, const double* Z, const double* mu, double* g, double* jac, EvalFlags f, int split,
                            cudaStream_t st, long long* launches) {
     const DInt& I = P.in[ii];
-    if (std::min(P.kc1, P.nI) - P.kc0 <= 0) return true;
-    if (!bilinear_octet_supported(I.n, I.m)) return false;
-    if (f.jets != DTO_JETS_NONE && I.jets == nullptr) return false;
+    if (std::min(P.kc1, P.nI) - P.kc0 <= 0) return;
     if (I.n == 8) {
         switch (I.m) {
-            case 1: return launch_octet<1, 1>(P, ii, Z, mu, g, jac, f, st, launches);
-            case 2: return launch_octet<1, 2>(P, ii, Z, mu, g, jac, f, st, launches);
-            case 3: return launch_octet<1, 3>(P, ii, Z, mu, g, jac, f, st, launches);
-            case 4: return launch_octet<1, 4>(P, ii, Z, mu, g, jac, f, st, launches);
+            case 1: return launch_octet<1, 1>(P, ii, Z, mu, g, jac, f, split, st, launches);
+            case 2: return launch_octet<1, 2>(P, ii, Z, mu, g, jac, f, split, st, launches);
+            case 3: return launch_octet<1, 3>(P, ii, Z, mu, g, jac, f, split, st, launches);
+            case 4: return launch_octet<1, 4>(P, ii, Z, mu, g, jac, f, split, st, launches);
         }
     } else if (I.n == 16) {
         switch (I.m) {
-            case 1: return launch_octet<2, 1>(P, ii, Z, mu, g, jac, f, st, launches);
-            case 2: return launch_octet<2, 2>(P, ii, Z, mu, g, jac, f, st, launches);
+            case 1: return launch_octet<2, 1>(P, ii, Z, mu, g, jac, f, split, st, launches);
+            case 2: return launch_octet<2, 2>(P, ii, Z, mu, g, jac, f, split, st, launches);
         }
     }
-    return false;
 }

@@ -1206,57 +1206,50 @@ __global__ void __launch_bounds__(max_warps<NT>() * 32, 1)
     }
 }
 
+constexpr size_t kSmemBudget = 227 * 1024 - 1024;  // dynamic shared memory the persistent kernel launches with at most
+
 template <int NT>
-bool launch_product_nt(const DProb& P, int ii, const double* Z, const double* w, double* y, bool transpose, cudaStream_t st,
+void launch_product_nt(const DProb& P, int ii, const double* Z, const double* w, double* y, bool transpose, cudaStream_t st,
                        long long* launches) {
     const DInt& I = P.in[ii];
     constexpr int n = 8 * NT;
     const size_t mat = sizeof(double) * (size_t)n * n;
     const size_t slot = 2 * mat + sizeof(double) * (1 + kMaxDrives) * n;
     const size_t shared_part = (size_t)(I.m + 1) * mat;
-    const size_t budget = 227 * 1024 - 1024;
-    if (shared_part + slot > budget) return false;
     int dev = 0, sms = 148;
     cudaGetDevice(&dev);
     cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-    const int W = (int)std::min<size_t>(max_warps<NT>(), (budget - shared_part) / slot);
+    const int W = (int)std::min<size_t>(max_warps<NT>(), (kSmemBudget - shared_part) / slot);
     const size_t smem = shared_part + (size_t)W * slot;
     auto kern = bilinear_product_kernel<NT>;
-    static PerDeviceOnce configured;
-    if (configured.first()) {
-        if (cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024) != cudaSuccess) return false;
-    }
     const long long items = (long long)P.batch * P.nI;
     const int grid = (int)std::max<long long>(1, std::min<long long>(sms, (items + W - 1) / W));
     const long long per_warp = items / ((long long)grid * W);
     const int fetch = (NT <= 2) ? (int)std::max<long long>(1, std::min<long long>(8, per_warp / 8)) : 1;
     kern<<<grid, W * 32, smem, st>>>(P, ii, Z, w, y, transpose ? 1 : 0, I.wq, fetch);
-    if (cudaMemsetAsync(I.wq, 0, 4 * sizeof(unsigned long long), st) != cudaSuccess) return false;  // zero between launches
+    cudaMemsetAsync(I.wq, 0, 4 * sizeof(unsigned long long), st);  // zero between launches
     ++*launches;
-    return true;
 }
 
 template <int NT, int MT>
-bool launch_variant(const DProb& P, int ii, const double* Z, const double* mu, double* g, double* jac, EvalFlags f, cudaStream_t st,
-                    long long* launches) {
+void launch_variant(const DProb& P, int ii, const double* Z, const double* mu, double* g, double* jac, EvalFlags f, int ne_cap,
+                    cudaStream_t st, long long* launches) {
     const DInt& I = P.in[ii];
     constexpr int n = 8 * NT;
     const size_t mat = sizeof(double) * (size_t)n * n;
     const size_t slot = mat + sizeof(double) * (1 + kMaxDrives) * n;
-    const size_t shared_part = (size_t)(I.m + 1) * mat;
-    const size_t budget = 227 * 1024 - 1024;
-    if (shared_part + slot > budget) return false;
+    const size_t shared_part = (size_t)(I.m + 1) * mat;  // with one slot at most 194.5 KB (n = 64, m = 4)
     int dev = 0, sms = 148;
     cudaGetDevice(&dev);
     cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
     // warps per CTA and how many of them carry the two spare matrices: prefer full occupancy, then
     // one Paterson-Stockmeyer warp per three
-    int W = (int)std::min<size_t>(max_warps<NT>(), (budget - shared_part) / slot);
+    int W = (int)std::min<size_t>(max_warps<NT>(), (kSmemBudget - shared_part) / slot);
     int nE = 0;
     if (f.want_jac) {
         int bestW = W, bestE = 0;
         for (int w = W; w >= std::max(2, W - 4); --w) {
-            const size_t left = budget - shared_part - (size_t)w * slot;
+            const size_t left = kSmemBudget - shared_part - (size_t)w * slot;
             const int e = (int)std::min<size_t>((size_t)w, left / (2 * mat));
             if (e >= (w + 2) / 3) {
                 bestW = w;
@@ -1269,15 +1262,10 @@ bool launch_variant(const DProb& P, int ii, const double* Z, const double* mu, d
             }
         }
         W = bestW;
-        nE = bestE;
-        if (const char* env = getenv("DTO_B200_K1_NE")) nE = std::max(0, std::min(nE, atoi(env)));  // experiments
+        nE = std::min(bestE, ne_cap);
     }
     const size_t smem = shared_part + (size_t)W * slot + (size_t)nE * 2 * mat;
     auto kern = bilinear_persistent_kernel<NT, MT>;
-    static PerDeviceOnce configured;
-    if (configured.first()) {
-        if (cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)budget) != cudaSuccess) return false;
-    }
     const long long items = (long long)P.batch * (std::min(P.kc1, P.nI) - P.kc0);
     const long long roles = (f.jets != DTO_JETS_USE ? 1 : 0) + (f.want_jac ? 1 : 0) + (f.want_hess ? 1 : 0);
     const long long want_ctas = (items * roles + W - 1) / W;
@@ -1288,7 +1276,6 @@ bool launch_variant(const DProb& P, int ii, const double* Z, const double* mu, d
     const int fetch = (NT <= 2) ? (int)std::max<long long>(1, std::min<long long>(8, per_warp / 8)) : 1;
     kern<<<grid, W * 32, smem, st>>>(P, ii, Z, mu, f.want_g ? g : nullptr, jac, f.want_jac ? 1 : 0, f.want_hess ? 1 : 0, I.wq, nE, fetch, f.jets);
     ++*launches;
-    return true;
 }
 
 }  // namespace
@@ -1298,44 +1285,37 @@ bool bilinear_persistent_supported(int n, int m) {
     return n == 8 || n == 16 || n == 24 || n == 32 || n == 48 || n == 64;
 }
 
-bool launch_bilinear_persistent(const DProb& P, int ii, const double* Z, const double* mu, double* g, double* jac, EvalFlags f,
-                                cudaStream_t st, long long* launches) {
+// the product kernel's m + 1 generators and one warp's slot: they exceed kSmemBudget at n = 64, m = 4
+bool bilinear_product_supported(int n, int m) {
+    const size_t mat = sizeof(double) * (size_t)n * n;
+    return (size_t)(m + 1) * mat + 2 * mat + sizeof(double) * (1 + kMaxDrives) * n <= kSmemBudget;
+}
+
+bool bilinear_persistent_configure(int n, bool interval, bool product, std::string& err) {
+    return with_nt(n, [&](auto nt) {
+        constexpr int NT = decltype(nt)::value;
+        const std::string s = std::to_string(NT);
+        return (!interval || (opt_in_smem(bilinear_persistent_kernel<NT, 1>, kSmemBudget, "bilinear_persistent_kernel<" + s + ", 1>", err) &&
+                              opt_in_smem(bilinear_persistent_kernel<NT, 2>, kSmemBudget, "bilinear_persistent_kernel<" + s + ", 2>", err))) &&
+               (!product || opt_in_smem(bilinear_product_kernel<NT>, 227 * 1024, "bilinear_product_kernel<" + s + ">", err));
+    });
+}
+
+void launch_bilinear_persistent(const DProb& P, int ii, const double* Z, const double* mu, double* g, double* jac, EvalFlags f,
+                                int ne_cap, cudaStream_t st, long long* launches) {
     const DInt& I = P.in[ii];
-    if (std::min(P.kc1, P.nI) - P.kc0 <= 0) return true;
-    if (!bilinear_persistent_supported(I.n, I.m) || I.G_stride != 0 || I.wq == nullptr) return false;
-    if (f.jets != DTO_JETS_NONE && I.jets == nullptr) return false;
+    if (std::min(P.kc1, P.nI) - P.kc0 <= 0) return;
     const bool second = (f.want_hess && f.jets == DTO_JETS_NONE) || f.jets == DTO_JETS_STORE;  // forward role carries d2/du du
     const int nrows = second ? 1 + I.m + I.m * (I.m + 1) / 2 : 1 + I.m;
-    const bool two = nrows > 8;
-#define DTO_DISPATCH(NTv)                                                                                      \
-    case NTv:                                                                                                  \
-        return two ? launch_variant<NTv, 2>(P, ii, Z, mu, g, jac, f, st, launches)                             \
-                   : launch_variant<NTv, 1>(P, ii, Z, mu, g, jac, f, st, launches);
-    switch (I.n / 8) {
-        DTO_DISPATCH(1)
-        DTO_DISPATCH(2)
-        DTO_DISPATCH(3)
-        DTO_DISPATCH(4)
-        DTO_DISPATCH(6)
-        DTO_DISPATCH(8)
-    }
-#undef DTO_DISPATCH
-    return false;
+    with_nt(I.n, [&](auto nt) {
+        if (nrows > 8) launch_variant<decltype(nt)::value, 2>(P, ii, Z, mu, g, jac, f, ne_cap, st, launches);
+        else launch_variant<decltype(nt)::value, 1>(P, ii, Z, mu, g, jac, f, ne_cap, st, launches);
+    });
 }
 
 // y (+)= the rows / columns of integrator ii in J w (transpose = false: rows are assigned) or J' w (atomically added)
-bool launch_bilinear_product(const DProb& P, int ii, const double* Z, const double* w, double* y, bool transpose, cudaStream_t st,
+void launch_bilinear_product(const DProb& P, int ii, const double* Z, const double* w, double* y, bool transpose, cudaStream_t st,
                              long long* launches) {
-    const DInt& I = P.in[ii];
-    if (P.nI <= 0) return true;
-    if (!bilinear_persistent_supported(I.n, I.m) || I.G_stride != 0 || I.wq == nullptr || P.halo != nullptr) return false;
-    switch (I.n / 8) {
-        case 1: return launch_product_nt<1>(P, ii, Z, w, y, transpose, st, launches);
-        case 2: return launch_product_nt<2>(P, ii, Z, w, y, transpose, st, launches);
-        case 3: return launch_product_nt<3>(P, ii, Z, w, y, transpose, st, launches);
-        case 4: return launch_product_nt<4>(P, ii, Z, w, y, transpose, st, launches);
-        case 6: return launch_product_nt<6>(P, ii, Z, w, y, transpose, st, launches);
-        case 8: return launch_product_nt<8>(P, ii, Z, w, y, transpose, st, launches);
-    }
-    return false;
+    if (P.nI <= 0) return;
+    with_nt(P.in[ii].n, [&](auto nt) { launch_product_nt<decltype(nt)::value>(P, ii, Z, w, y, transpose, st, launches); });
 }

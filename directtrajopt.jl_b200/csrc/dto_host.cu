@@ -178,6 +178,11 @@ struct dto_handle {
     bool have_g = false, have_jac = false;  // dg, djac
     bool have_jets = false;    // DInt::jets of every bilinear integrator
     bool jets_ok = false;      // every interval kernel of the problem can keep / use the jets
+    bool matrix_free = false;  // Jacobian products come from the series, not from the materialised Jacobian (jac_product)
+    // launch forms pinned by test and measurement switches (DESIGN.md section 5), read when the handle is built
+    int k1_ne_cap = std::numeric_limits<int>::max();  // DTO_B200_K1_NE: most Paterson-Stockmeyer warps of the persistent kernel
+    int octet_split = -1;      // DTO_B200_OCTET_SPLIT: 0 whole octets only, 1 every octet in phases, -1 chosen per launch
+    bool tdb_split = true;     // DTO_B200_TDB_SPLIT=0: one 16-warp CTA per interval instead of two kernels
     long long cache_hits = 0, cache_misses = 0;
     // ---- registered outputs (dto_register_outputs): the solver's own value arrays, page-locked, structural constants
     // written once; later callbacks that are handed these pointers move only the value-dependent entries
@@ -636,6 +641,9 @@ static int build_integrators(dto_handle* h, const dto_problem_desc* d, int smem_
     // DTO_B200_KERNEL=generic|dmma|persistent pins an older variant (A/B measurements, parity tests of every variant)
     const char* pin_env = getenv("DTO_B200_KERNEL");
     const std::string pin = pin_env ? pin_env : "";
+    if (const char* e = getenv("DTO_B200_K1_NE")) h->k1_ne_cap = std::max(0, atoi(e));
+    if (const char* e = getenv("DTO_B200_OCTET_SPLIT")) h->octet_split = e[0] == '1' ? 1 : 0;
+    if (const char* e = getenv("DTO_B200_TDB_SPLIT")) h->tdb_split = e[0] != '0';
     long long goff = 0, loff = 0;
     int doff = 0;
     for (int i = 0; i < d->n_integrators; ++i) {
@@ -1174,6 +1182,44 @@ static int build_work_buffers(dto_handle* h, const dto_problem_desc* d) {
     return DTO_OK;
 }
 
+// Products straight from the series for problems made of bilinear integrators whose shared generators the product kernel
+// can stage, derivative integrators and knot constraints; anything else materialises the Jacobian values first, as the
+// reference does (evaluator.jl:406-456).  DTO_B200_JVP=materialize forces the latter.
+static bool matrix_free_products(const dto_handle* h) {
+    const DProb& P = h->P;
+    const char* env = getenv("DTO_B200_JVP");
+    if (h->sharded || P.gl.G > 0 || (env && strcmp(env, "materialize") == 0)) return false;
+    for (int i = 0; i < P.n_int; ++i) {
+        const DInt& I = P.in[i];
+        if (I.kind != DTO_INT_DERIVATIVE &&
+            !(I.kind == DTO_INT_BILINEAR && I.variant >= DTO_VAR_PERSISTENT && I.G_stride == 0 && bilinear_product_supported(I.n, I.m)))
+            return false;
+    }
+    return true;
+}
+
+// Every kernel the handle can launch is opted into the shared memory it launches with here (the attribute is per
+// device), so that a kernel that cannot be configured fails construction instead of an evaluation
+static int configure_kernels(dto_handle* h, const dto_problem_desc* d) {
+    const DProb& P = h->P;
+    h->matrix_free = matrix_free_products(h);
+    std::string err;
+    bool ok = true;
+    for (int i = 0; i < P.n_int && ok; ++i) {
+        const DInt& I = P.in[i];
+        if (I.kind == DTO_INT_BILINEAR) {
+            if (I.variant >= DTO_VAR_PERSISTENT) ok = bilinear_persistent_configure(I.n, I.variant == DTO_VAR_PERSISTENT, h->matrix_free, err);
+            else if (I.variant == DTO_VAR_DMMA) ok = bilinear_dmma_configure(I.n, err);
+            else ok = bilinear_generic_configure(I.n, I.m, err);
+            if (ok && I.plan) ok = series_plan_configure(I.m, err);
+        } else if (I.kind == DTO_INT_TDBILINEAR) {
+            ok = I.variant == DTO_VAR_DMMA ? tdb_dmma_configure(I.n, err) : tdb_configure(err);
+        }
+    }
+    if (ok && d->eval_hessian) ok = hessian_assemble_configure(P, h->hs_left, err);
+    return ok ? DTO_OK : reject(DTO_ERR_CUDA, err);
+}
+
 // the host-pointer path: pipeline cuts, structural-zero runs of the Hessian, constant heads of the Jacobian columns
 static void plan_host_path(dto_handle* h, const dto_problem_desc* d) {
     DProb& P = h->P;
@@ -1300,6 +1346,7 @@ extern "C" int dto_create(const dto_problem_desc* d, dto_handle** out) {
         set_sizes(h, d, n_dyn_global, n_dyn_local, n_nl_global);
         rc = build_work_buffers(h, d);
     }
+    if (rc == DTO_OK) rc = configure_kernels(h, d);
     if (rc == DTO_OK) {
         plan_host_path(h, d);
         if (h->upload_failed) rc = reject(DTO_ERR_ALLOC, "device allocation failed");
@@ -1506,7 +1553,6 @@ static HsRows hs_rows(const DProb& P, bool leading) {
 static int eval_range(dto_handle* h, const DProb& P, const double* dZ, double sigma, const double* dmu, double* dg, double* djac,
                       double* dhess, EvalFlags f) {
     if (!(f.want_g || f.want_jac || f.want_hess)) return DTO_OK;
-    bool fused_missed = false;
     // knot-objective Hessian pairs: they depend on Z only, so they run beside the interval kernels (second stream) and the
     // assembler below waits for them
     bool side_on_aux = false;
@@ -1525,24 +1571,18 @@ static int eval_range(dto_handle* h, const DProb& P, const double* dZ, double si
         const bool timed = h->timing && h->ev_used < h->ev_pool.size();
         if (timed) cudaEventRecord(h->ev_pool[h->ev_used].first, h->stream);
         if (P.in[i].kind == DTO_INT_BILINEAR) {
-            bool done = false;
-            if (P.in[i].variant == DTO_VAR_OCTET) {
-                done = launch_bilinear_octet(P, i, dZ, dmu, dg, djac, f, h->stream, &h->launches);
-                if (!done && P.analytic_fused == i + 1) fused_missed = true;
+            switch (P.in[i].variant) {
+                case DTO_VAR_OCTET: launch_bilinear_octet(P, i, dZ, dmu, dg, djac, f, h->octet_split, h->stream, &h->launches); break;
+                case DTO_VAR_PERSISTENT: launch_bilinear_persistent(P, i, dZ, dmu, dg, djac, f, h->k1_ne_cap, h->stream, &h->launches); break;
+                case DTO_VAR_DMMA: launch_bilinear_dmma(P, i, dZ, dmu, dg, djac, f, h->stream, &h->launches); break;
+                default: launch_bilinear_generic(P, i, dZ, dmu, dg, djac, f, h->stream, &h->launches);
             }
-            if (!done && P.in[i].variant >= DTO_VAR_PERSISTENT && P.in[i].G_stride == 0) done = launch_bilinear_persistent(P, i, dZ, dmu, dg, djac, f, h->stream, &h->launches);
-            if (!done && f.jets != DTO_JETS_NONE) {
-                h->err = "interval kernel cannot keep the forward jets between callbacks (internal)";
-                return DTO_ERR_CUDA;
-            }
-            if (!done && P.in[i].variant >= DTO_VAR_DMMA && bilinear_dmma_supported(P.in[i].n, P.in[i].m))
-                done = launch_bilinear_dmma(P, i, dZ, dmu, dg, djac, f, h->stream, &h->launches);
-            if (!done) launch_bilinear_generic(P, i, dZ, dmu, dg, djac, f, h->stream, &h->launches);
             if (f.jets == DTO_JETS_USE) launch_hpp_contract(P, i, dmu, h->stream, &h->launches);
         } else if (P.in[i].kind == DTO_INT_TDBILINEAR) {
-            bool done = false;
-            if (P.in[i].variant == DTO_VAR_DMMA) done = launch_tdb_dmma(P, i, dZ, dmu, dg, djac, f, h->stream, &h->launches);
-            if (!done) launch_tdb(P, i, dZ, dmu, dg, djac, f, h->stream, &h->launches);
+            switch (P.in[i].variant) {
+                case DTO_VAR_DMMA: launch_tdb_dmma(P, i, dZ, dmu, dg, djac, f, h->tdb_split, h->stream, &h->launches); break;
+                default: launch_tdb(P, i, dZ, dmu, dg, djac, f, h->stream, &h->launches);
+            }
         }
         if (timed) cudaEventRecord(h->ev_pool[h->ev_used++].second, h->stream);
     }
@@ -1550,15 +1590,7 @@ static int eval_range(dto_handle* h, const DProb& P, const double* dZ, double si
     // knot they belong to
     if (f.want_hess && h->hs_push_now && P.nI - 1 >= P.kc0 && P.nI - 1 < P.kc1)
         launch_hs_push(h->xwin, h->peer_win[h->link_rank + 1], hs_rows(P, false), P.z, h->hblk_len, h->hseq, h->stream, &h->launches);
-    if (f.want_g || f.want_jac) {
-        if (fused_missed) {
-            DProb Pn = P;
-            Pn.analytic_fused = 0;
-            launch_analytic(Pn, dZ, dg, djac, f, h->stream, &h->launches);
-        } else {
-            launch_analytic(P, dZ, dg, djac, f, h->stream, &h->launches);
-        }
-    }
+    if (f.want_g || f.want_jac) launch_analytic(P, dZ, dg, djac, f, h->stream, &h->launches);
     if (side_on_aux) CUDA_TRY(h, cudaStreamWaitEvent(h->stream, h->ev_side, 0));
     if (h->want_g_ready) CUDA_TRY(h, cudaEventRecord(h->ev_g_ready, h->stream));  // every residual row is written
     if (f.want_hess && h->hs_recv_now) {
@@ -2227,19 +2259,6 @@ extern "C" int dto_register_outputs(dto_handle* h, double* jac_vals, double* hes
     return DTO_OK;
 }
 
-// Products straight from the series for problems made of persistent-variant bilinear integrators, derivative
-// integrators and knot constraints; anything else materialises the Jacobian values first, as the reference does
-// (evaluator.jl:406-456).  DTO_B200_JVP=materialize forces the latter.
-static bool matrix_free_capable(const dto_handle* h) {
-    const DProb& P = h->P;
-    if (h->sharded || P.gl.G > 0) return false;
-    const char* env = getenv("DTO_B200_JVP");
-    if (env && strcmp(env, "materialize") == 0) return false;
-    for (int i = 0; i < P.n_int; ++i)
-        if (P.in[i].kind != DTO_INT_DERIVATIVE && !(P.in[i].kind == DTO_INT_BILINEAR && P.in[i].variant >= DTO_VAR_PERSISTENT)) return false;
-    return true;
-}
-
 static int jac_product(dto_handle* h, const double* Z, const double* w, double* y, bool transpose) {
     if (!h || !Z || !w || !y) return DTO_ERR_INVALID;
     const DProb& P = h->P;
@@ -2264,15 +2283,12 @@ static int jac_product(dto_handle* h, const double* Z, const double* w, double* 
         if (rc < 0) return rc;
     }
     CUDA_TRY(h, cudaMemcpyAsync(h->dw, w, sizeof(double) * B * nw, cudaMemcpyHostToDevice, h->stream));
-    bool done = false;
-    if (matrix_free_capable(h)) {
+    if (h->matrix_free) {
         CUDA_TRY(h, cudaMemsetAsync(h->dy, 0, sizeof(double) * B * ny, h->stream));
-        done = true;
-        for (int i = 0; i < P.n_int && done; ++i)
-            if (P.in[i].kind == DTO_INT_BILINEAR) done = launch_bilinear_product(P, i, h->dZ, h->dw, h->dy, transpose, h->stream, &h->launches);
-        if (done) launch_analytic_product(P, h->dZ, h->dw, h->dy, transpose, h->stream, &h->launches);
-    }
-    if (!done) {
+        for (int i = 0; i < P.n_int; ++i)
+            if (P.in[i].kind == DTO_INT_BILINEAR) launch_bilinear_product(P, i, h->dZ, h->dw, h->dy, transpose, h->stream, &h->launches);
+        launch_analytic_product(P, h->dZ, h->dw, h->dy, transpose, h->stream, &h->launches);
+    } else {
         if (!h->d_rows0) {
             std::vector<int64_t> r((size_t)P.nnz_jac_local), c((size_t)P.nnz_jac_local);
             int rc = dto_jac_structure(h, r.data(), c.data());

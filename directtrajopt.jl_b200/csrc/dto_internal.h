@@ -5,6 +5,7 @@
 
 #include <algorithm>
 #include <string>
+#include <type_traits>
 #include <vector>
 
 #include "../../include/dto_b200.h"
@@ -259,17 +260,26 @@ void launch_shard_scalars(XWin* own, XWin* const* peers, int rank, int world, un
 // variants of the bilinear kernel
 enum { DTO_VAR_GENERIC = 0, DTO_VAR_DMMA = 1, DTO_VAR_PERSISTENT = 2, DTO_VAR_OCTET = 3 };
 
-// cudaFuncSetAttribute is per device: a launcher opts a kernel into large dynamic shared memory once per device
-struct PerDeviceOnce {
-    bool done[64] = {};
-    bool first() {
-        int d = 0;
-        if (cudaGetDevice(&d) != cudaSuccess || d < 0 || d >= 64) return true;
-        if (done[d]) return false;
-        done[d] = true;
-        return true;
+// Opts `kern` into `bytes` of dynamic shared memory on the current device; a failure names the kernel in `err`
+template <class F>
+bool opt_in_smem(F* kern, size_t bytes, const std::string& name, std::string& err) {
+    const cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes);
+    if (e != cudaSuccess) err = "cannot opt " + name + " into " + std::to_string(bytes) + " bytes of shared memory: " + cudaGetErrorString(e);
+    return e == cudaSuccess;
+}
+
+// f(std::integral_constant<int, n / 8>()) for the states of the tensor-core kernels, n = 8, 16, 24, 32, 48 and 64
+template <class F>
+auto with_nt(int n, F&& f) {
+    switch (n / 8) {
+        case 1: return f(std::integral_constant<int, 1>());
+        case 2: return f(std::integral_constant<int, 2>());
+        case 3: return f(std::integral_constant<int, 3>());
+        case 4: return f(std::integral_constant<int, 4>());
+        case 6: return f(std::integral_constant<int, 6>());
+        default: return f(std::integral_constant<int, 8>());
     }
-};
+}
 
 // ---- kernel launchers (defined in the .cu files) ------------------------------------------------
 // jets: 0 = single pass (the Hessian pass contracts the second-order jet with mu in the interval kernel);
@@ -284,33 +294,43 @@ struct EvalFlags {
 };
 // (parameter, parameter) block of the compact Hessian from stored jets: hpp = -mu' W, same summation order as the kernels
 void launch_hpp_contract(const DProb& P, int ii, const double* mu, cudaStream_t st, long long* launches);
+// The interval-kernel launchers launch the variant dto_create chose (DInt::variant) and never decline: construction
+// accepts only shapes they launch and opts their kernels into shared memory (*_configure).  ne_cap and split carry the
+// switches the handle read when it was built (dto_host.cu).
 void launch_bilinear_generic(const DProb& P, int ii, const double* Z, const double* mu, double* g, double* jac, EvalFlags f,
                              cudaStream_t st, long long* launches);
+bool bilinear_generic_configure(int n, int m, std::string& err);
 size_t generic_smem_bytes(int n, int m, bool want_jac, bool want_hess);  // dynamic shared memory of one generic K1 block
-bool launch_bilinear_dmma(const DProb& P, int ii, const double* Z, const double* mu, double* g, double* jac, EvalFlags f,
+void launch_bilinear_dmma(const DProb& P, int ii, const double* Z, const double* mu, double* g, double* jac, EvalFlags f,
                           cudaStream_t st, long long* launches);
 bool bilinear_dmma_supported(int n, int m);
-bool launch_bilinear_persistent(const DProb& P, int ii, const double* Z, const double* mu, double* g, double* jac, EvalFlags f,
-                                cudaStream_t st, long long* launches);
+bool bilinear_dmma_configure(int n, std::string& err);
+void launch_bilinear_persistent(const DProb& P, int ii, const double* Z, const double* mu, double* g, double* jac, EvalFlags f,
+                                int ne_cap, cudaStream_t st, long long* launches);
 bool bilinear_persistent_supported(int n, int m);
-bool launch_bilinear_octet(const DProb& P, int ii, const double* Z, const double* mu, double* g, double* jac, EvalFlags f,
+bool bilinear_persistent_configure(int n, bool interval, bool product, std::string& err);
+void launch_bilinear_octet(const DProb& P, int ii, const double* Z, const double* mu, double* g, double* jac, EvalFlags f, int split,
                            cudaStream_t st, long long* launches);
 bool bilinear_octet_supported(int n, int m);
 void bilinear_octet_fragments(int n, int m, const double* Gcm, double* out);
 size_t bilinear_octet_fragment_doubles(int n, int m);
-bool launch_bilinear_product(const DProb& P, int ii, const double* Z, const double* w, double* y, bool transpose, cudaStream_t st,
+void launch_bilinear_product(const DProb& P, int ii, const double* Z, const double* w, double* y, bool transpose, cudaStream_t st,
                              long long* launches);
+bool bilinear_product_supported(int n, int m);  // the product kernel's shared memory fits (persistent-supported shapes)
 void launch_analytic_product(const DProb& P, const double* Z, const double* w, double* y, bool transpose, cudaStream_t st,
                              long long* launches);
 size_t series_plan_smem(int n, int m);
 void series_plan_matrices(int n, int m, const double* Gcm, std::vector<float>& out);
-bool launch_series_plan(const DProb& P, int ii, const double* Z, cudaStream_t st, long long* launches);
+void launch_series_plan(const DProb& P, int ii, const double* Z, cudaStream_t st, long long* launches);
+bool series_plan_configure(int m, std::string& err);
 bool tdb_dmma_supported(const DInt& I);
-bool launch_tdb_dmma(const DProb& P, int ii, const double* Z, const double* mu, double* g, double* jac, EvalFlags f, cudaStream_t st,
-                     long long* launches);
+bool tdb_dmma_configure(int n, std::string& err);
+void launch_tdb_dmma(const DProb& P, int ii, const double* Z, const double* mu, double* g, double* jac, EvalFlags f, bool split,
+                     cudaStream_t st, long long* launches);
 bool tdb_fits(const DInt& I, size_t smem_limit);
 void launch_tdb(const DProb& P, int ii, const double* Z, const double* mu, double* g, double* jac, EvalFlags f, cudaStream_t st,
                 long long* launches);
+bool tdb_configure(std::string& err);
 void launch_analytic(const DProb& P, const double* Z, double* g, double* jac, EvalFlags f, cudaStream_t st, long long* launches);
 void launch_constraints(const DProb& P, const double* Z, double* g, double* jac, EvalFlags f, cudaStream_t st, long long* launches);
 bool launch_knot_objective_pairs(const DProb& P, const double* Z, cudaStream_t st, long long* launches);
@@ -319,6 +339,7 @@ bool launch_knot_objective_pairs(const DProb& P, const double* Z, cudaStream_t s
 void launch_hessian_assemble(const DProb& P, const double* Z, double sigma, const double* mu, double* hess, cudaStream_t st,
                              long long* launches, bool left_block = false);
 size_t hessian_assemble_smem_bytes(const DProb& P);  // dynamic shared memory of one assembler block (depends on z, any_cross)
+bool hessian_assemble_configure(const DProb& P, bool left_block, std::string& err);
 void launch_objective(const DProb& P, const double* Z, double* J, double* grad, double* partials, cudaStream_t st,
                       long long* launches);
 void launch_violation(const DProb& P, const double* g, const int* row_is_eq, double* viol, cudaStream_t st, long long* launches);

@@ -183,14 +183,10 @@ void series_plan_matrices(int n, int m, const double* Gcm /* (m+1) column-major 
 }
 
 template <int NM>
-static bool launch_plan_nm(const DProb& P, int ii, const double* Z, double2* out, long long items, int sms, cudaStream_t st) {
+static void launch_plan_nm(const DProb& P, int ii, const double* Z, double2* out, long long items, int sms, cudaStream_t st) {
     constexpr int T = 4;
     const DInt& I = P.in[ii];
     const size_t smem = series_plan_smem(I.n, I.m);
-    static PerDeviceOnce configured;
-    if (configured.first()) {
-        if (cudaFuncSetAttribute(series_plan_kernel<NM, T>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024) != cudaSuccess) return false;
-    }
     const int gs = (I.n <= 32 && 32 % I.n == 0) ? I.n : 32, per_warp = 32 / gs;
     const long long groups = (items + T - 1) / T, tasks = (groups + per_warp - 1) / per_warp;
     // every CTA stages the matrices once: as few warps per CTA as keep all SMs busy
@@ -200,26 +196,28 @@ static bool launch_plan_nm(const DProb& P, int ii, const double* Z, double2* out
     const int per_sm = (int)std::max<size_t>(1, std::min<size_t>(2048 / threads, (220 * 1024) / (smem + 1024)));
     const int grid = (int)std::min<long long>((tasks + wpc - 1) / wpc, (long long)sms * per_sm);
     series_plan_kernel<NM, T><<<grid, threads, smem, st>>>(P, ii, Z, out, gs);
-    return true;
 }
 
-bool launch_series_plan(const DProb& P, int ii, const double* Z, cudaStream_t st, long long* launches) {
+bool series_plan_configure(int m, std::string& err) {
+    void (*const kern[])(DProb, int, const double*, double2*, int) = {series_plan_kernel<1, 4>, series_plan_kernel<2, 4>, series_plan_kernel<3, 4>,
+                                                                     series_plan_kernel<4, 4>, series_plan_kernel<5, 4>};
+    return opt_in_smem(kern[m], 200 * 1024, "series_plan_kernel<" + std::to_string(m + 1) + ", 4>", err);
+}
+
+void launch_series_plan(const DProb& P, int ii, const double* Z, cudaStream_t st, long long* launches) {
     const DInt& I = P.in[ii];
-    if (I.plan == nullptr || I.planmat == nullptr || I.G_stride != 0 || series_plan_smem(I.n, I.m) == 0) return false;
     const long long items = (long long)P.batch * (std::min(P.kc1, P.nI) - P.kc0);
-    if (items <= 0) return true;
+    if (items <= 0) return;
     int dev = 0, sms = 148;
     cudaGetDevice(&dev);
     cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
     double2* out = const_cast<double2*>(I.plan);
-    bool ok = false;
     switch (I.m) {
-        case 0: ok = launch_plan_nm<1>(P, ii, Z, out, items, sms, st); break;
-        case 1: ok = launch_plan_nm<2>(P, ii, Z, out, items, sms, st); break;
-        case 2: ok = launch_plan_nm<3>(P, ii, Z, out, items, sms, st); break;
-        case 3: ok = launch_plan_nm<4>(P, ii, Z, out, items, sms, st); break;
-        case 4: ok = launch_plan_nm<5>(P, ii, Z, out, items, sms, st); break;
+        case 0: launch_plan_nm<1>(P, ii, Z, out, items, sms, st); break;
+        case 1: launch_plan_nm<2>(P, ii, Z, out, items, sms, st); break;
+        case 2: launch_plan_nm<3>(P, ii, Z, out, items, sms, st); break;
+        case 3: launch_plan_nm<4>(P, ii, Z, out, items, sms, st); break;
+        case 4: launch_plan_nm<5>(P, ii, Z, out, items, sms, st); break;
     }
-    if (ok) ++*launches;
-    return ok;
+    ++*launches;
 }

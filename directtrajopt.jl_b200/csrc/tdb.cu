@@ -411,15 +411,13 @@ void launch_tdb(const DProb& P, int ii, const double* Z, const double* mu, doubl
     const int nIc = std::min(P.kc1, P.nI) - P.kc0;
     if (nIc <= 0) return;
     const size_t smem = tdb_smem_bytes(I, f.want_jac, f.want_hess);
-    static PerDeviceOnce configured;
-    if (configured.first()) {
-        cudaFuncSetAttribute(tdb_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
-    }
     const int K = 8;
     dim3 grid((unsigned)(nIc * P.batch), 1 + (f.want_jac ? 1 : 0) + (f.want_hess ? 1 : 0));
     tdb_kernel<<<grid, kThreads, smem, st>>>(P, ii, Z, mu, f.want_g ? g : nullptr, jac, f.want_jac ? 1 : 0, f.want_hess ? 1 : 0, K);
     ++*launches;
 }
+
+bool tdb_configure(std::string& err) { return opt_in_smem(tdb_kernel, 227 * 1024, "tdb_kernel", err); }
 
 bool tdb_fits(const DInt& I, size_t smem_limit) {
     return I.m <= kMaxM && I.n_carrier <= kMaxC && tdb_smem_bytes(I, true, true) <= smem_limit;

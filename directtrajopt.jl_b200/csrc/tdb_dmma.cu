@@ -1168,7 +1168,7 @@ struct Plan {
     size_t smem;
 };
 
-bool make_plan(const DInt& I, bool want_jac, bool want_hess, Plan& pl) {
+bool make_plan(const DInt& I, bool want_jac, bool want_hess, bool allow_split, Plan& pl) {
     const int n = I.n, m = I.m, nc = I.n_carrier;
     if (n % 8 != 0 || n > 64 || (n / 8 == 5) || (n / 8 == 7) || m > kMaxM || nc > kMaxC || I.Asw == nullptr) return false;
     const int np = (I.order == 1 ? 2 * m : m) + 2, npairs = np * (np + 1) / 2;
@@ -1184,10 +1184,8 @@ bool make_plan(const DInt& I, bool want_jac, bool want_hess, Plan& pl) {
     pl.warps = pl.TF + pl.TE + pl.TA;
     if (pl.warps > 8) {
         const int half = std::max(pl.TF + pl.TA, pl.TE);
-        // two kernels of 8-warp CTAs (forward + adjoint tiles / propagator tiles, 255 registers each); DTO_B200_TDB_SPLIT=0 = one
+        // two kernels of 8-warp CTAs (forward + adjoint tiles / propagator tiles, 255 registers each); !allow_split = one
         // 16-warp CTA at 128 registers (measured slower: 11.1 against 9.2 ms at c3)
-        const char* env = getenv("DTO_B200_TDB_SPLIT");
-        const bool allow_split = !(env && env[0] == '0');
         if (half <= 8 && pl.TE > 0 && (allow_split || pl.warps > kMaxWarpsT)) {
             pl.split = 1;
             pl.warps = half;
@@ -1215,11 +1213,6 @@ template <int NT, int MAXW>
 void launch_nt_w(const DProb& P, int ii, const double* Z, const double* mu, double* g, double* jac, EvalFlags f, cudaStream_t st,
                  const Plan& pl) {
     auto kern = tdb_dmma_kernel<NT, MAXW>;
-    static PerDeviceOnce configured;
-    if (configured.first()) {
-        cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
-        cudaFuncSetAttribute(tdb_exp_kernel<NT>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
-    }
     const DInt& I = P.in[ii];
     const int ctas = std::min((std::min(P.kc1, P.nI) - P.kc0) * P.batch, I.tdb_scratch_ctas / 2);  // persistent: one CTA per SM
     if (!pl.split) {
@@ -1237,37 +1230,35 @@ void launch_nt_w(const DProb& P, int ii, const double* Z, const double* mu, doub
                                                                                                        I.tdb_scratch);
 }
 
-template <int NT>
-void launch_nt(const DProb& P, int ii, const double* Z, const double* mu, double* g, double* jac, EvalFlags f, cudaStream_t st,
-               const Plan& pl) {
-    if (pl.warps <= 8) launch_nt_w<NT, 8>(P, ii, Z, mu, g, jac, f, st, pl);
-    else launch_nt_w<NT, 16>(P, ii, Z, mu, g, jac, f, st, pl);
-}
-
 }  // namespace
 
+// the plan of a Jacobian and Hessian pass: every other pass needs fewer tiles and no more shared memory
 bool tdb_dmma_supported(const DInt& I) {
     Plan pl;
-    return make_plan(I, true, true, pl);
+    return make_plan(I, true, true, true, pl);
 }
 
-bool launch_tdb_dmma(const DProb& P, int ii, const double* Z, const double* mu, double* g, double* jac, EvalFlags f, cudaStream_t st,
-                     long long* launches) {
+bool tdb_dmma_configure(int n, std::string& err) {
+    return with_nt(n, [&](auto nt) {
+        constexpr int NT = decltype(nt)::value;
+        const std::string s = std::to_string(NT);
+        return opt_in_smem(tdb_dmma_kernel<NT, 8>, 227 * 1024, "tdb_dmma_kernel<" + s + ", 8>", err) &&
+               opt_in_smem(tdb_dmma_kernel<NT, 16>, 227 * 1024, "tdb_dmma_kernel<" + s + ", 16>", err) &&
+               opt_in_smem(tdb_exp_kernel<NT>, 227 * 1024, "tdb_exp_kernel<" + s + ">", err);
+    });
+}
+
+void launch_tdb_dmma(const DProb& P, int ii, const double* Z, const double* mu, double* g, double* jac, EvalFlags f, bool split,
+                     cudaStream_t st, long long* launches) {
     const DInt& I = P.in[ii];
-    if (std::min(P.kc1, P.nI) - P.kc0 <= 0) return true;
+    if (std::min(P.kc1, P.nI) - P.kc0 <= 0) return;
     Plan pl;
-    if (!make_plan(I, f.want_jac, f.want_hess, pl)) return false;
-    switch (I.n / 8) {
-        case 1: launch_nt<1>(P, ii, Z, mu, g, jac, f, st, pl); break;
-        case 2: launch_nt<2>(P, ii, Z, mu, g, jac, f, st, pl); break;
-        case 3: launch_nt<3>(P, ii, Z, mu, g, jac, f, st, pl); break;
-        case 4: launch_nt<4>(P, ii, Z, mu, g, jac, f, st, pl); break;
-        case 6: launch_nt<6>(P, ii, Z, mu, g, jac, f, st, pl); break;
-        case 8: launch_nt<8>(P, ii, Z, mu, g, jac, f, st, pl); break;
-        default: return false;
-    }
+    make_plan(I, f.want_jac, f.want_hess, split, pl);  // succeeds where tdb_dmma_supported did
+    with_nt(I.n, [&](auto nt) {
+        if (pl.warps <= 8) launch_nt_w<decltype(nt)::value, 8>(P, ii, Z, mu, g, jac, f, st, pl);
+        else launch_nt_w<decltype(nt)::value, 16>(P, ii, Z, mu, g, jac, f, st, pl);
+    });
     ++*launches;
-    return true;
 }
 
 #ifdef DTO_TDB_PROFILE

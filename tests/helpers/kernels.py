@@ -1,7 +1,7 @@
 """Which interval kernels (and which knot-side kernels) a call launched, as the CUDA profiler (CUPTI) reports them.
 
-A handle's reported variant is what construction chose; a launcher may still decline a shape and let the next one in
-the chain run.  Tests that must know which instantiation produced their numbers ask the profiler instead."""
+A handle's reported variant names the kernel family construction chose, and the launchers run exactly that family.  Which
+instantiation of it (template arguments, products, split forms) ran is the profiler's to say."""
 import re
 
 _KERNEL_RE = re.compile(r"(?<![A-Za-z0-9_])(bilinear_(?:persistent|dmma|octet|generic|product)_kernel|tdb_(?:dmma_|exp_)?kernel)(<[^>(]*>)?")

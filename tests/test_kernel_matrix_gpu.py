@@ -2,9 +2,9 @@
 
 K1 is a family of template instantiations: octet (n = 8, 16), persistent and dmma (n = 8..64, NT = n / 8 tiles, MT = 2
 forward tiles once 1 + m + m(m+1)/2 > 8), the per-problem-generator forms of octet and dmma, generic (any other shape),
-and the matrix-free product kernel.  The host picks one at construction and launchers may decline a shape, so the
-variant a handle reports is not proof of which kernel produced the numbers.  Each cell below therefore records the
-interval kernels the CUDA profiler sees and asserts that they are exactly the ones the cell is meant to reach; the
+and the matrix-free product kernel.  The host picks the family at construction, and the variant a handle reports names
+it; the template arguments follow from the shape and the pass.  Each cell asserts the reported family and records the
+interval kernels the CUDA profiler sees, asserting that they are exactly the ones the cell is meant to reach; the
 coverage guard at the end asserts that the cells together reached every instantiation in KERNELS.
 
 Every cell runs on an iterate whose intervals take different code paths: dt = 0, u = 0, and theta = |dt| ||G(u)||_1
@@ -175,6 +175,7 @@ def test_instantiation_matches_oracle(cell, monkeypatch):
     hr, hc = ev.hessian_lagrangian_structure()
     assert np.array_equal(jr, jst[0]) and np.array_equal(jc, jst[1]) and np.array_equal(hr, hst[0]) and np.array_equal(hc, hst[1])
     nc, nv, nj, nh = ev.n_constraints, ev.n_vars, ev.nnz_jacobian, ev.nnz_hessian
+    assert ev.kernel_variant(0) == cell.fused[0].split("_")[1], (cell.id, ev.kernel_variant(0))  # bilinear_<family>_kernel
     seen = set()
     worst = {}
 
